@@ -297,6 +297,21 @@ def marl_groups(torch, E, V, dev):
 
 SARL_TRACE_NAMES = ("reward", "DataBuf", "data_t", "data_p", "over_power", "over_data", "rate")
 MARL_TRACE_NAMES = ("reward_user", "reward", "data_t", "data_p", "rate", "DataBuf")
+DUMP_BYTES = 60_000_000   # --dump-outputs budget for all traces together (the .npy headers add < 1 KB)
+
+
+def sample_traces(torch, out, E):
+    """{name: float32 ndarray} of the rollout traces `out` ([T, E, ...] each), restricted to a fixed, seeded sample of
+    env indices (the same sample for every trace; all E envs when they fit DUMP_BYTES)."""
+    import numpy as np
+
+    per_env = sum(v[:, 0].numel() * v.element_size() for v in out.values())
+    n = min(E, DUMP_BYTES // per_env)
+    if n < 1:
+        raise SystemExit(f"--dump-outputs: the traces of one env alone exceed {DUMP_BYTES} bytes")
+    idx = np.arange(E) if n == E else np.sort(np.random.default_rng(0).choice(E, n, replace=False))
+    sel = torch.as_tensor(idx, device=next(iter(out.values())).device)
+    return {k: v.index_select(1, sel).cpu().numpy() for k, v in out.items()}
 
 
 def make_rollout(torch, wl, E, V, M, T, local, rank, dev, sarl_path=None):
@@ -413,7 +428,16 @@ def main():
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true", help="skip the other configs' short measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the traces the last timed rollout returned (rank 0's shard) as DIR/<name>.npy, float32 "
+                         f"[T, n, ...] over a fixed, seeded sample of n env indices (all envs when they fit {DUMP_BYTES} "
+                         "bytes); the same arguments give the same inputs on every run, so two builds compare output "
+                         "for output (bench_outputs/ in the repository is git-ignored for this)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the CUDA rollout's traces: it does not apply to --impl reference")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -491,6 +515,9 @@ def main():
     # ---- timed region: K steps, device-timed, max over ranks
     sampler = ClockSampler(local)
     if rank == 0:
+        # the spin below runs for a wall-clock time, not a step count: restore the env afterwards so that the timed
+        # steps start from the state the warm-up left, the same on every run with the same arguments
+        warm_state = env.state_dict()
         sampler.start()
         t_spin = time.time()
         while True:  # keep the GPU under load until nvidia-smi delivers its first sample (<= 3 s)
@@ -500,6 +527,8 @@ def main():
             if sampler.lines or sampler.proc is None or time.time() - t_spin > 3.0:
                 break
         sampler.lines.clear()
+        env.load_state_dict(warm_state)
+        del warm_state
     if fold:
         env.collect_stats()  # discard what the warm-up rollouts accumulated
     stats_sum.zero_()
@@ -546,6 +575,7 @@ def main():
     clocks = sampler.stop() if rank == 0 else None
     value = world * E * T * args.steps / (ms_total * 1e-3)
     kernel_name = env.last_kernel()
+    dumped = sample_traces(torch, buf["out"], E) if args.dump_outputs and rank == 0 else None
 
     # ---- end to end through the public host-buffer API (pinned host in, pinned host out), same layout
     actions, arrivals, phases, out = buf["actions"], buf["arrivals"], buf["phases"], buf["out"]
@@ -676,6 +706,12 @@ def main():
             v, n, kind = cpu_throughput(wl, V, M, args.cpu_seconds, cores)
             line["cpu_baseline"] = {"value": v, "unit": UNIT, "cores": cores, "kind": kind,
                                     "sample": cpu_sample_text(kind, cores, args.cpu_seconds, n)}
+        if dumped is not None:
+            import numpy as np
+
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for k, a in dumped.items():
+                np.save(os.path.join(args.dump_outputs, f"{k}.npy"), a)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()

@@ -15,7 +15,7 @@ REPO_ROOT = os.path.dirname(PKG_DIR)
 CSRC = os.path.join(PKG_DIR, "csrc")
 LIB_PATH = os.environ.get("RISVEC_LIB") or os.path.join(PKG_DIR, "librisvec.so")  # override: A/B builds
 SOURCES = ["risvec.cu"]
-HEADERS = ["common.cuh", "geom.cuh", "ris.cuh", "step.cuh", "sarl_mma.cuh", "pairing.cuh", "replay.cuh"]
+HEADERS = sorted(f for f in os.listdir(CSRC) if f.endswith(".cuh"))  # every one is a rebuild dependency
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC",
               "-shared", "-split-compile", "0"]
 
