@@ -110,6 +110,9 @@ enum risvec_field {
     RISVEC_F_NOMA_NGROUPS,   /* i32 [E]    len(noma_groups); 0 = no groups yet           */
     RISVEC_F_NOMA_PAIRS,     /* i32 [E,V]  pairs (i0,j0,i1,j1,...) in list order, -1 pad */
     RISVEC_F_NOMA_NPAIRS,    /* i32 [E]    len(pairs)                                    */
+    /* per-env episode clock (risvec_episode_tick); both zero at creation */
+    RISVEC_F_EP_STEP,        /* i32 [E]    step of its episode the env's next driver step takes; 0 = starts */
+    RISVEC_F_EP_INDEX,       /* i32 [E]    the env's i_episode                           */
     RISVEC_F_COUNT
 };
 
@@ -330,6 +333,58 @@ int risvec_pair_noma(risvec_env_t* env, const risvec_pairing_t* cfg, const float
 int risvec_pair_reset(risvec_env_t* env, void* stream);
 /* ... for the envs with env_mask [E] u8 (device) != 0 only (NULL = all) */
 int risvec_pair_reset_masked(risvec_env_t* env, const uint8_t* env_mask, void* stream);
+
+/* ---- episode starts per env (marl_train_bcd.py:1268-1332): the device-side work at the start of an episode ----
+ * Stage bits; stages always run in this order.  The MARL driver runs all four (POSITIONS every
+ * env_refresh_every-th episode), the SARL driver POSITIONS only. */
+enum {
+    RISVEC_EP_RESET = 1,     /* make_new_game                                              */
+    RISVEC_EP_POSITIONS = 2, /* renew_positions + compute_parms                            */
+    RISVEC_EP_CHANNEL = 4,   /* optimize_phase_shift + update_channel_gains                */
+    RISVEC_EP_PAIRING = 8    /* pair_reset                                                 */
+};
+/* Every stage in `stages` for the envs whose stages_env [E] u8 (device) entry has its bit, in one call.
+ * stages_env NULL = every env runs `stages`.  The host cannot read stages_env without a synchronisation, so the
+ * kernel ANDs each entry with `stages` (bits outside `stages` are ignored); an env whose resulting bits are 0 keeps
+ * every field bit for bit.  uniforms [E, n_uni] f64 / used_out [E] i32 as in risvec_renew_positions (rows of envs
+ * that do not renew are ignored; their used_out is 0).  The draws are keyed like the separate calls and the host
+ * call counter of every stage in `stages` advances as the separate calls would, so each env ends bit-identical to
+ * running its stages as separate calls.  V <= 8, ncand <= 8, M <= 256 with the free channel runs as ONE launch
+ * (k_begin_episode); other shapes run the separate kernels back to back, restricted to the selected envs.
+ * RISVEC_ERR_INVALID for bits outside RISVEC_EP_*. */
+int risvec_begin_episode(risvec_env_t* env, const uint8_t* stages_env, int stages, const double* uniforms, int n_uni,
+                         int32_t* used_out, void* stream);
+
+/* Fixed-length episodes of the reference driver; positions_every = env_refresh_every (marl_train_bcd.py:1268). */
+typedef struct risvec_episode_schedule {
+    int32_t steps_per_episode, positions_every, stages, _pad;
+} risvec_episode_schedule_t;
+/* The episode clock: call once per driver step, before the step.  For every env:
+ *   start = (ep_step == 0); on start run `stages` (without POSITIONS unless ep_index % positions_every == 0);
+ *   done = (ep_step == steps_per_episode - 1), the terminal flag of the transition this step stores;
+ *   then ep_step += 1, and on wrap ep_step = 0, ep_index += 1.
+ * start_out / done_out [E] u8 (device) may be NULL.  Nothing is decided on the host, so the call can be captured in
+ * a CUDA graph.  Its draws are therefore keyed from device state, not from the host call counters (a graph freezes
+ * kernel arguments): RNG kinds reset / mobility / channel of the tick, call = the env's ep_index.  They stay seeded
+ * and independent of the sharding (global env index), differ per episode, and deliberately differ from the draws
+ * of risvec_begin_episode; the host call counters do not move.  Injected uniforms do not apply.  Staggered
+ * episodes: after make_new_game and one risvec_begin_episode for all envs, write per-env offsets into
+ * RISVEC_F_EP_STEP (for example e % steps_per_episode). */
+int risvec_episode_tick(risvec_env_t* env, const risvec_episode_schedule_t* schedule, uint8_t* start_out,
+                        uint8_t* done_out, void* stream);
+
+/* The driver's mask curriculum (batched.mask_schedule, marl_train_bcd.py:128-132,1323-1332); -1 selects the
+ * driver defaults topk_start = V - 1, topk_end = max(4, V / 2). */
+typedef struct risvec_pair_schedule {
+    int32_t topk_start, topk_end, warmup_episodes, _pad;
+    double tau_q_start, tau_q_end;
+} risvec_pair_schedule_t;
+/* risvec_pair_noma with per-env episode state: recalc_mask = new_episode = start[e] (start [E] u8, device), K_now /
+ * q_now from the env's RISVEC_F_EP_INDEX and `schedule`; envs with start[e] == 0 run as the call with
+ * recalc_mask = 0 and `reuse`.  Feed it the start_out of risvec_episode_tick. */
+int risvec_pair_noma_episodes(risvec_env_t* env, const risvec_pairing_t* cfg, const float* p01, int64_t p01_env_stride,
+                              const risvec_pair_schedule_t* schedule, const uint8_t* start, const int32_t* reuse,
+                              int decay, void* stream);
 
 /* ---- replay memory (SURVEY 8f row 4): Simulation-MARL-BCD/buffer.py, device resident ----
  * Same seven arrays as ReplayBuffer.__init__ (buffer.py:4-14): state / new_state [mem_size,

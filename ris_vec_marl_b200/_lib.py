@@ -43,8 +43,10 @@ FIELDS = ("pos_x", "pos_y", "dir", "vel", "dist", "angle", "amp", "theta_re", "t
           "DataBuf", "data_t", "data_p", "over_data", "over_power", "vehicle_rate", "data_r", "reward_user",
           "reward", "mec_queue_cycles", "stats", "last_power_W", "step_ctr",
           "V2I_Shadowing", "pair_hist", "unpaired_streak", "pair_tau", "pair_k", "pair_mask", "pair_rounds",
-          "noma_partner", "noma_ngroups", "noma_pairs", "noma_npairs")
+          "noma_partner", "noma_ngroups", "noma_pairs", "noma_npairs", "ep_step", "ep_index")
 PAIR_MAX_V = 12
+# stage bits of risvec_begin_episode / risvec_episode_tick (RISVEC_EP_*), in the order the stages run
+EP_STAGES = {"reset": 1, "positions": 2, "channel": 4, "pairing": 8}
 REPLAY_FIELDS = ("state_memory", "action_memory", "reward_global_memory", "reward_local_memory", "new_state_memory",
                  "terminal_memory", "mask_memory")
 
@@ -94,6 +96,20 @@ class Pairing(C.Structure):
         ("score_w_delta_db", C.c_double), ("score_w_history", C.c_double), ("abs_gain_min_db", C.c_double),
         ("qos_soft_penalty_dbscore", C.c_double), ("pair_hist_decay", C.c_double),
     ]
+
+
+class EpisodeSchedule(C.Structure):
+    """Mirror of `risvec_episode_schedule_t`."""
+
+    _fields_ = [("steps_per_episode", C.c_int32), ("positions_every", C.c_int32), ("stages", C.c_int32),
+                ("_pad", C.c_int32)]
+
+
+class PairSchedule(C.Structure):
+    """Mirror of `risvec_pair_schedule_t` (the mask curriculum of `batched.mask_schedule`; -1 = driver default)."""
+
+    _fields_ = [("topk_start", C.c_int32), ("topk_end", C.c_int32), ("warmup_episodes", C.c_int32), ("_pad", C.c_int32),
+                ("tau_q_start", C.c_double), ("tau_q_end", C.c_double)]
 
 
 class MarlOut(C.Structure):
@@ -148,6 +164,10 @@ EXPORTS = {
     "risvec_pair_noma": (C.c_int, [C.c_void_p, C.POINTER(Pairing), C.c_void_p, C.c_int64, C.c_int, C.c_double, C.c_int,
                                    C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
     "risvec_pair_reset": (C.c_int, [C.c_void_p, C.c_void_p]),
+    "risvec_begin_episode": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
+    "risvec_episode_tick": (C.c_int, [C.c_void_p, C.POINTER(EpisodeSchedule), C.c_void_p, C.c_void_p, C.c_void_p]),
+    "risvec_pair_noma_episodes": (C.c_int, [C.c_void_p, C.POINTER(Pairing), C.c_void_p, C.c_int64,
+                                            C.POINTER(PairSchedule), C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     "risvec_replay_create": (C.c_int, [C.c_int, C.c_int64, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
     "risvec_replay_destroy": (C.c_int, [C.c_void_p]),
     "risvec_replay_field": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_int64),

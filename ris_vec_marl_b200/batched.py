@@ -13,7 +13,8 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import CHANNEL, FIELDS, NSTAT, STAT_COLUMNS, VARIANT, MarlOut, Pairing, Params, SarlOut, check
+from ._lib import (CHANNEL, EP_STAGES, FIELDS, NSTAT, STAT_COLUMNS, VARIANT, EpisodeSchedule, MarlOut, Pairing,
+                   PairSchedule, Params, SarlOut, check)
 
 _PARAM_NAMES = {n for n, _ in Params._fields_} - {"_pad0"}
 _PAIRING_NAMES = {n for n, _ in Pairing._fields_}
@@ -105,7 +106,7 @@ class BatchedEnviron:
                                          C.byref(fl)))
             typestr = "|u1" if eb.value == 1 else ("<f" if fl.value else "<i") + str(eb.value)
             per_env_scalar = name in ("reward", "mec_queue_cycles", "step_ctr", "pair_tau", "pair_k", "pair_rounds",
-                                      "noma_ngroups", "noma_npairs")
+                                      "noma_ngroups", "noma_npairs", "ep_step", "ep_index")
             shape = (rows.value,) if per_env_scalar else (rows.value, cols.value)
             self._views[name] = torch.as_tensor(_DevView(ptr.value, shape, typestr), device=self.device)
         self._views["last_power_W"] = self._views["last_power_W"].view(self.E, 2, self.V)
@@ -491,6 +492,75 @@ class BatchedEnviron:
         check(self._lib.risvec_pair_noma(self._h, C.byref(self.pairing), self._p(t), stride, int(topk), float(tau_q),
                                          int(bool(recalc_mask)), self._p(ru), int(bool(decay)), int(bool(new_episode)),
                                          self.stream))
+        return self._views["noma_partner"], self._views["noma_ngroups"]
+
+    # ------------------------------------------------------------------ episodes per env
+    @staticmethod
+    def _stage_bits(stages):
+        if isinstance(stages, int):
+            return stages
+        bits = 0
+        for st in stages:
+            if st not in EP_STAGES:
+                raise ValueError(f"unknown episode stage {st!r} (one of {tuple(EP_STAGES)})")
+            bits |= EP_STAGES[st]
+        return bits
+
+    def begin_episode(self, stages=("positions", "channel", "pairing"), per_env=None, uniforms=None):
+        """The device-side work at the start of an episode (marl_train_bcd.py:1268-1309), for every env or -- `per_env`
+        [E] u8 of `EP_STAGES` bits -- for each env the stages its entry selects (AND-ed with `stages`).  Stages run in
+        the order reset, positions, channel, pairing; each env ends bit-identical to running its stages as the separate
+        calls (`make_new_game`, `renew_positions` + `compute_parms`, `optimize_phase_shift` + `update_channel_gains`,
+        `pair_reset`).  One launch for V <= 8 with the free channel.  `uniforms` [E, n] as in `renew_positions`.
+        Returns `used` [E] int32 when positions are renewed, else None.
+
+        Staggered episodes: `make_new_game()`, then one `begin_episode()` for all envs, then write per-env offsets into
+        `env.ep_step` (for example `torch.arange(E) % 100`); from then on `episode_tick` runs the starts."""
+        bits = self._stage_bits(stages)
+        pe = None if per_env is None else self._dev(torch.as_tensor(per_env).to(torch.uint8), torch.uint8, (self.E,))
+        u = self._dev(uniforms, torch.float64)
+        n = 0 if u is None else u.shape[1]
+        used = torch.empty(self.E, dtype=torch.int32, device=self.device) if bits & EP_STAGES["positions"] else None
+        check(self._lib.risvec_begin_episode(self._h, self._p(pe), bits, self._p(u), n, self._p(used), self.stream))
+        return used
+
+    def episode_tick(self, steps_per_episode=100, positions_every=5, stages=("positions", "channel", "pairing"),
+                     out=None):
+        """The per-env episode clock; call once per driver step, before the step.  Envs with `ep_step == 0` start an
+        episode and run `stages` (positions only when `ep_index % positions_every == 0`, the driver's
+        env_refresh_every); `done` flags the last step of an episode (the terminal of the transition stored this
+        step); then the clock advances.  Returns `(start, done)` u8 [E]; pass the previous result as `out` to reuse its
+        buffers (a CUDA graph capture needs fixed buffers).  The draws are keyed by the env's episode index, not by
+        host counters, so a captured graph draws fresh numbers every episode (they differ from `begin_episode`'s)."""
+        sch = EpisodeSchedule(int(steps_per_episode), int(positions_every), self._stage_bits(stages), 0)
+        if out is None:
+            out = (torch.empty(self.E, dtype=torch.uint8, device=self.device),
+                   torch.empty(self.E, dtype=torch.uint8, device=self.device))
+        start, done = out
+        for t in (start, done):
+            if t.dtype != torch.uint8 or tuple(t.shape) != (self.E,) or t.device != self.device or not t.is_contiguous():
+                raise ValueError(f"out must hold two contiguous uint8 [{self.E}] tensors on {self.device}")
+        check(self._lib.risvec_episode_tick(self._h, C.byref(sch), self._p(start), self._p(done), self.stream))
+        return start, done
+
+    def pair_noma_episodes(self, p01, start, schedule=(None, None, 0.2, 0.4, 200), reuse=None, decay=True):
+        """`pair_noma` with per-env episode state: envs with `start` [E] != 0 build the mask and solve as the first step
+        of an episode, with K_now / q_now of `mask_schedule(env.ep_index[e], ...)`; the others run the non-recalc step
+        with `reuse`.  `schedule` = (topk_start, topk_end, tau_q_start, tau_q_end, warmup_episodes), None = driver
+        default (config.yaml: 7, 7, 0.10, 0.25, 200).  Returns the views `(noma_partner, noma_ngroups)`."""
+        t = self._dev(p01, torch.float32)
+        if tuple(t.shape) == (self.E, 2, self.V):
+            stride = 2 * self.V
+        elif tuple(t.shape) == (self.E, self.V):
+            stride = self.V
+        else:
+            raise ValueError(f"p01 must be [E,V] or [E,2,V], got {tuple(t.shape)}")
+        st = self._dev(start, torch.uint8, (self.E,))
+        ru = self._dev(reuse, torch.int32, (self.E,))
+        k0, k1, q0, q1, warm = schedule
+        sch = PairSchedule(-1 if k0 is None else int(k0), -1 if k1 is None else int(k1), int(warm), 0, float(q0), float(q1))
+        check(self._lib.risvec_pair_noma_episodes(self._h, C.byref(self.pairing), self._p(t), stride, C.byref(sch),
+                                                  self._p(st), self._p(ru), int(bool(decay)), self.stream))
         return self._views["noma_partner"], self._views["noma_ngroups"]
 
     def shard_stats(self, out=None, accumulate=False):

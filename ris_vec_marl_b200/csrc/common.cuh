@@ -38,7 +38,26 @@ struct State {
 // by (global env index, per-call counter, slot, stream kind): draws do not depend on how
 // envs are sharded over GPUs or on launch geometry.
 // ---------------------------------------------------------------------------------------
-enum RngKind : unsigned { kRngReset = 1, kRngMobility = 2, kRngArrival = 3, kRngChannel = 4 };
+// kinds 5-7: the draws of risvec_episode_tick, keyed by the env's episode index instead of a host call counter
+enum RngKind : unsigned {
+    kRngReset = 1, kRngMobility = 2, kRngArrival = 3, kRngChannel = 4,
+    kRngEpReset = 5, kRngEpMobility = 6, kRngEpChannel = 7
+};
+
+// Per-env selection of the episode-start kernels (risvec_begin_episode / risvec_episode_tick on the shapes the
+// fused kernel does not take).  Zero-initialised = every env, host-keyed draws: exactly the plain entry points.
+struct EnvGate {
+    const unsigned char* bits;  // [E] per-env RISVEC_EP_* bits, or null (every env runs this launch)
+    unsigned bit;               // the stage this launch runs
+    const int* call;            // [E] per-env RNG call = episode index (device-keyed draws), or null (host counter)
+    __device__ bool on(long long e) const { return bits == nullptr || (bits[e] & bit) != 0; }
+    __device__ unsigned long long key(long long e, unsigned long long host_call) const {
+        return call != nullptr ? (unsigned long long)(unsigned)call[e] : host_call;
+    }
+    __device__ unsigned kind(unsigned host_kind, unsigned device_kind) const {
+        return call != nullptr ? device_kind : host_kind;
+    }
+};
 
 __host__ __device__ inline uint4 philox4x32_10(uint4 c, uint2 k) {
     const uint32_t M0 = 0xD2511F53u, M1 = 0xCD9E8D57u, W0 = 0x9E3779B9u, W1 = 0xBB67AE85u;

@@ -6,13 +6,11 @@
 
 namespace risvec {
 
-// make_new_game: one thread per env (the draws of one env are consumed sequentially).
-__global__ void k_make_new_game(Dims d, State s, risvec_params_t p, const int* __restrict__ ints, int n_ints,
-                                const int* __restrict__ dirs, int n_dirs, unsigned long long call,
-                                const unsigned char* __restrict__ env_mask) {
-    const int e = blockIdx.x * blockDim.x + threadIdx.x;
-    if (e >= d.E) return;
-    if (env_mask != nullptr && env_mask[e] == 0) return;  // per-env reset: this env keeps its state
+// make_new_game of env e by one thread (the draws of one env are consumed sequentially); `kind` / `call` key the
+// Philox draws.  Shared by k_make_new_game and the fused episode start (episode.cuh).
+__device__ __forceinline__ void make_new_game_env(const Dims& d, const State& s, const risvec_params_t& p, int e,
+                                                  const int* __restrict__ ints, int n_ints, const int* __restrict__ dirs,
+                                                  int n_dirs, unsigned long long call, unsigned kind) {
     const int V = d.V;
     int cur = 0, curd = 0;
     auto randint = [&](int lo, int hi) -> int {
@@ -20,7 +18,7 @@ __global__ void k_make_new_game(Dims d, State s, risvec_params_t p, const int* _
         if (ints != nullptr) {
             v = cur < n_ints ? ints[(size_t)e * n_ints + cur] : lo;
         } else {
-            uint4 r = rng_draw(d, e, call, (unsigned)cur, kRngReset);
+            uint4 r = rng_draw(d, e, call, (unsigned)cur, kind);
             v = lo + (int)__umulhi(r.x, (unsigned)(hi - lo));
         }
         ++cur;
@@ -52,7 +50,7 @@ __global__ void k_make_new_game(Dims d, State s, risvec_params_t p, const int* _
         if (dirs != nullptr) {
             heading = curd < n_dirs ? dirs[(size_t)e * n_dirs + curd] : RISVEC_DIR_DOWN;
         } else {
-            uint4 q = rng_draw(d, e, call, 1024u + (unsigned)curd, kRngReset);
+            uint4 q = rng_draw(d, e, call, 1024u + (unsigned)curd, kind);
             heading = (int)(q.x & 3u);
         }
         ++curd;
@@ -64,12 +62,23 @@ __global__ void k_make_new_game(Dims d, State s, risvec_params_t p, const int* _
     for (int v = 0; v < V; ++v) s.databuf[(size_t)e * V + v] = buf;
 }
 
-// renew_positions: one thread per env, vehicles in index order; arithmetic uses the
-// round-to-nearest intrinsics so no FMA contraction can change a bit w.r.t. the reference.
-__global__ void k_renew_positions(Dims d, State s, risvec_params_t p, const double* __restrict__ uniforms, int n_uni,
-                                  int* __restrict__ used_out, unsigned long long call) {
+// make_new_game: one thread per env.  env_mask (risvec_make_new_game_masked) and the gate select envs.
+__global__ void k_make_new_game(Dims d, State s, risvec_params_t p, const int* __restrict__ ints, int n_ints,
+                                const int* __restrict__ dirs, int n_dirs, unsigned long long call,
+                                const unsigned char* __restrict__ env_mask, EnvGate g) {
     const int e = blockIdx.x * blockDim.x + threadIdx.x;
     if (e >= d.E) return;
+    if (env_mask != nullptr && env_mask[e] == 0) return;  // per-env reset: this env keeps its state
+    if (!g.on(e)) return;
+    make_new_game_env(d, s, p, e, ints, n_ints, dirs, n_dirs, g.key(e, call), g.kind(kRngReset, kRngEpReset));
+}
+
+// renew_positions of env e by one thread, vehicles in index order; arithmetic uses the
+// round-to-nearest intrinsics so no FMA contraction can change a bit w.r.t. the reference.
+// Returns the number of uniforms consumed.
+__device__ __forceinline__ int renew_positions_env(const Dims& d, const State& s, const risvec_params_t& p, int e,
+                                                   const double* __restrict__ uniforms, int n_uni,
+                                                   unsigned long long call, unsigned kind) {
     const int V = d.V;
     int cur = 0;
     for (int i = 0; i < V; ++i) {
@@ -102,7 +111,7 @@ __global__ void k_renew_positions(Dims d, State s, risvec_params_t p, const doub
                 if (uniforms != nullptr) {
                     u = cur < n_uni ? uniforms[(size_t)e * n_uni + cur] : 1.0;
                 } else {
-                    uint4 r = rng_draw(d, e, call, (unsigned)(i * 16 + which * 8 + j), kRngMobility);
+                    uint4 r = rng_draw(d, e, call, (unsigned)(i * 16 + which * 8 + j), kind);
                     u = u01d(r.x, r.y);
                 }
                 ++cur;
@@ -141,22 +150,46 @@ __global__ void k_renew_positions(Dims d, State s, risvec_params_t p, const doub
         s.pos_y[ix] = y;
         s.dir[ix] = heading;
     }
+    return cur;
+}
+
+// renew_positions: one thread per env.  Envs the gate leaves out keep their state and report 0 draws used.
+__global__ void k_renew_positions(Dims d, State s, risvec_params_t p, const double* __restrict__ uniforms, int n_uni,
+                                  int* __restrict__ used_out, unsigned long long call, EnvGate g) {
+    const int e = blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= d.E) return;
+    int cur = 0;
+    if (g.on(e))
+        cur = renew_positions_env(d, s, p, e, uniforms, n_uni, g.key(e, call), g.kind(kRngMobility, kRngEpMobility));
     if (used_out != nullptr) used_out[e] = cur;
 }
 
 // compute_parms: one thread per (env, vehicle).  Distances and angles follow the reference's
 // operation order exactly; the V x M phasor table `phases_R_i` is NOT materialised in HBM --
 // the channel kernels regenerate exp(j*pi*m*(angle_BR - angle_v)) from `angle` in float64.
-__global__ void k_compute_parms(Dims d, State s) {
-    const size_t ix = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (ix >= (size_t)d.E * d.V) return;
-    const double dx = __dsub_rn(s.pos_x[ix], kRisX);
-    const double dy = __dsub_rn(s.pos_y[ix], kRisY);
+struct Parms {
+    double dist, angle, amp;
+};
+__device__ __forceinline__ Parms compute_parms_of(const Dims& d, double x, double y) {
+    const double dx = __dsub_rn(x, kRisX);
+    const double dy = __dsub_rn(y, kRisY);
     const double dz = kVehZ - kRisZ;
     const double dist = __dsqrt_rn(__dadd_rn(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)), dz * dz));
-    s.dist[ix] = dist;
-    s.angle[ix] = __ddiv_rn(dx, dist);
-    s.amp[ix] = (kRo * kRo) / (pow(dist, kAlpha1) * pow(d.dist_BR, kAlpha2));
+    Parms r;
+    r.dist = dist;
+    r.angle = __ddiv_rn(dx, dist);
+    r.amp = (kRo * kRo) / (pow(dist, kAlpha1) * pow(d.dist_BR, kAlpha2));
+    return r;
+}
+
+__global__ void k_compute_parms(Dims d, State s, EnvGate g) {
+    const size_t ix = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (ix >= (size_t)d.E * d.V) return;
+    if (!g.on((long long)(ix / d.V))) return;
+    const Parms r = compute_parms_of(d, s.pos_x[ix], s.pos_y[ix]);
+    s.dist[ix] = r.dist;
+    s.angle[ix] = r.angle;
+    s.amp[ix] = r.amp;
 }
 
 }  // namespace risvec

@@ -38,7 +38,27 @@ struct PairArgs {
     int* npairs;
     int* rounds;
     unsigned char* mask;
+    // per-env episode state (risvec_pair_noma_episodes); null = the scalar recalc / fresh / topk / tau_q above
+    const unsigned char* start;  // [E] != 0: first step of the env's episode (recalc_mask = new_episode = 1)
+    const int* ep_index;         // [E] i_episode: K_now / q_now of the mask curriculum, computed per env
+    int sched_topk_start, sched_topk_end, sched_warmup;
+    double sched_tau_q_start, sched_tau_q_end;
 };
+
+// batched.mask_schedule (`_anneal_topk` marl_train_bcd.py:128-132 and :1323-1332) for one env: python's round is
+// half-to-even (rint), and the explicit round-to-nearest intrinsics keep every operation as python evaluates it
+__device__ __forceinline__ void mask_schedule_dev(const PairArgs& a, int N, int ep, int* K, double* q) {
+    const int k_start = a.sched_topk_start < 0 ? N - 1 : a.sched_topk_start;
+    const int k_end = a.sched_topk_end < 0 ? max(4, N / 2) : a.sched_topk_end;
+    const int warm = a.sched_warmup;
+    const double w = (double)max(1, warm);
+    const int i = max(0, min(ep, warm));
+    const double kf = __dadd_rn((double)k_end, __dmul_rn((double)(k_start - k_end), __dsub_rn(1.0, __ddiv_rn((double)i, w))));
+    const int k = (int)rint(kf);
+    const double prog = fmin(1.0, __ddiv_rn((double)ep, w));
+    *K = min(max(k, 1), N - 1);
+    *q = __dadd_rn(a.sched_tau_q_start, __dmul_rn(__dsub_rn(a.sched_tau_q_end, a.sched_tau_q_start), prog));
+}
 
 __host__ __device__ inline size_t pair_smem_bytes(int N) {
     const size_t NN = (size_t)N * N, NS = (size_t)1 << N;
@@ -405,10 +425,16 @@ __global__ void k_pair_noma(Dims d, State s, PairArgs a) {
     if (e >= d.E) return;    // whole warps leave together; only __syncwarp is used below
     PairCtx<N> c;
     c.carve(pair_smem + pair_smem_bytes(N) * wib, lane);
+    int recalc = a.recalc, fresh = a.fresh, topk = a.topk;
+    double tau_q = a.tau_q;
+    if (a.start != nullptr) {                                 // per-env episode state
+        recalc = fresh = a.start[e] != 0;
+        if (recalc) mask_schedule_dev(a, N, a.ep_index[e], &topk, &tau_q);
+    }
 
     float* H = a.hist + e * NN;
     for (int x = lane; x < NN; x += 32) {
-        const float h = a.fresh ? 0.f : H[x];
+        const float h = fresh ? 0.f : H[x];
         c.Hs[x] = a.decay ? __fmul_rn(h, a.decay_f) : h;     // :1406 (float32 array *= python float)
     }
     if (lane < N) {
@@ -422,9 +448,9 @@ __global__ void k_pair_noma(Dims d, State s, PairArgs a) {
 
     double tau;
     int K;
-    if (a.recalc) {                                           // :1319-1343
-        tau = c.adaptive_tau(a.tau_q);
-        K = a.topk;
+    if (recalc) {                                             // :1319-1343
+        tau = c.adaptive_tau(tau_q);
+        K = topk;
         c.build_mask(tau, K);
         for (int x = lane; x < NN; x += 32) a.mask[e * NN + x] = c.feas[x];
         if (lane == 0) { a.tau[e] = tau; a.lastk[e] = K; }
@@ -436,7 +462,7 @@ __global__ void k_pair_noma(Dims d, State s, PairArgs a) {
     }
 
     int np = 0, rounds = 0;
-    const bool frozen = !a.fresh && a.reuse != nullptr && a.reuse[e] != 0 && a.ngroups[e] > 0;
+    const bool frozen = !fresh && a.reuse != nullptr && a.reuse[e] != 0 && a.ngroups[e] > 0;
     if (frozen) {                                             // :1542-1547
         np = a.npairs[e];
         if (lane < 2 * np) c.pr[lane] = a.pairs[e * N + lane];
@@ -491,16 +517,31 @@ __global__ void k_pair_noma(Dims d, State s, PairArgs a) {
     for (int x = lane; x < NN; x += 32) H[x] = c.Hs[x];
     if (lane < N) {
         int* sk = a.streak + e * N + lane;
-        *sk = (used >> lane & 1u) ? 0 : (a.fresh ? 0 : *sk) + 1;
+        *sk = (used >> lane & 1u) ? 0 : (fresh ? 0 : *sk) + 1;
     }
 }
 
-// new episode (:1282-1297): history, streak, thresholds and frozen groups cleared
-__global__ void k_pair_reset(Dims d, PairArgs a, const unsigned char* __restrict__ env_mask) {
+// new episode (:1282-1297) of env e by the threads x0, x0 + step, ... (x0 < step): history, streak, thresholds and
+// frozen groups cleared.  The fused episode start (episode.cuh) runs it with the env's 8 lanes.
+__device__ __forceinline__ void pair_reset_env(const PairArgs& a, int N, long long e, int x0, int step) {
+    const int NN = N * N;
+    for (int x = x0; x < NN; x += step) {
+        a.hist[e * NN + x] = 0.f;
+        a.mask[e * NN + x] = 0;
+    }
+    for (int x = x0; x < N; x += step) {
+        a.streak[e * N + x] = 0;
+        a.partner[e * N + x] = RISVEC_PARTNER_NONE;
+        a.pairs[e * N + x] = -1;
+    }
+    if (x0 == 0) { a.tau[e] = 0.0; a.lastk[e] = 0; a.ngroups[e] = 0; a.npairs[e] = 0; a.rounds[e] = 0; }
+}
+
+__global__ void k_pair_reset(Dims d, PairArgs a, const unsigned char* __restrict__ env_mask, EnvGate g) {
     const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     const int N = d.V, NN = N * N;
     if (t >= (long long)d.E * NN) return;
-    auto on = [&](long long e) { return env_mask == nullptr || env_mask[e] != 0; };  // per-env reset
+    auto on = [&](long long e) { return (env_mask == nullptr || env_mask[e] != 0) && g.on(e); };  // per-env reset
     if (on(t / NN)) {
         a.hist[t] = 0.f;
         a.mask[t] = 0;

@@ -81,12 +81,12 @@ __device__ inline void geom_phasor(double delta, int m, double* re, double* im) 
 // K > 0 independent of theta.  The coordinate search therefore keeps S incrementally:
 // for each m the candidate maximising |S - theta_m c_m + e_k c_m|^2 wins, first maximum on
 // ties, accepted only if strictly positive (best starts at 0, MARL:210-218).
-__global__ void k_bcd(Dims d, State s) {
+__global__ void k_bcd(Dims d, State s, EnvGate g) {
     extern __shared__ double2 bcd_smem[];
     const int wpb = blockDim.x >> 5;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int e = blockIdx.x * wpb + warp;
-    if (e >= d.E) return;  // whole warp leaves together
+    if (e >= d.E || !g.on(e)) return;  // whole warp leaves together
     const int V = d.V, M = d.M;
     double2* c = bcd_smem + (size_t)warp * 2 * M;
     double2* th = c + M;
@@ -172,17 +172,14 @@ __global__ void k_bcd(Dims d, State s) {
 // (z_v = exp(j pi (angle_BR - angle_v)) of vehicle v = k, shuffled to the env's lanes) and float64
 // complex powers: lane k owns the elements m = k + 8 i, w = z^k * (z^8)^i.  Same search, same
 // tie rule (first maximum), same acceptance test as k_bcd.
-__global__ void k_bcd_v8(Dims d, State s) {
-    extern __shared__ double2 bcd_smem[];
-    const int wpb = blockDim.x >> 5;
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, el = lane >> 3, k = lane & 7;
-    const int e_raw = (blockIdx.x * wpb + warp) * 4 + el;
-    const bool env_ok = e_raw < d.E;
-    const int e = min(e_raw, d.E - 1);
+// bcd_v8_warp is the body for the env e of this lane's group: `angle` = angle of vehicle min(k, V - 1) of env e,
+// c / th = the env's 2 M double2 of shared memory (th holds the result afterwards).  All 32 lanes must call it
+// (full-warp shuffles); only `write` envs store theta.  Shared by k_bcd_v8 and the fused episode start.
+__device__ __forceinline__ void bcd_v8_warp(const Dims& d, const State& s, int e, bool write, double angle,
+                                            double2* c, double2* th) {
+    const int lane = threadIdx.x & 31, k = lane & 7;
     const int V = d.V, M = d.M, base = lane & ~7;
-    double2* c = bcd_smem + (size_t)(warp * 4 + el) * 2 * M;
-    double2* th = c + M;
-    const double2 my_z = unit_phasor64(d.angle_BR - s.angle[(size_t)e * V + min(k, V - 1)]);
+    const double2 my_z = unit_phasor64(d.angle_BR - angle);
     for (int m = k; m < M; m += 8) c[m] = make_double2(0.0, 0.0);
     for (int v = 0; v < V; ++v) {
         const double2 z = make_double2(__shfl_sync(kFull, my_z.x, base + v), __shfl_sync(kFull, my_z.y, base + v));
@@ -241,47 +238,66 @@ __global__ void k_bcd_v8(Dims d, State s) {
         }
         __syncwarp();
     }
-    if (env_ok)
+    if (write)
         for (int m = k; m < M; m += 8) {
             s.theta_re[(size_t)e * M + m] = th[m].x;
             s.theta_im[(size_t)e * M + m] = th[m].y;
         }
 }
 
+__global__ void k_bcd_v8(Dims d, State s, EnvGate g) {
+    extern __shared__ double2 bcd_smem[];
+    const int wpb = blockDim.x >> 5;
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, el = lane >> 3, k = lane & 7;
+    const int e_raw = (blockIdx.x * wpb + warp) * 4 + el;
+    const int e = min(e_raw, d.E - 1);
+    const bool env_ok = e_raw < d.E && g.on(e);
+    double2* c = bcd_smem + (size_t)(warp * 4 + el) * 2 * d.M;
+    bcd_v8_warp(d, s, e, env_ok, s.angle[(size_t)e * d.V + min(k, d.V - 1)], c, c + d.M);
+}
+
 // update_channel_gains, "free" model, lane = (env, vehicle): the vehicle's phasor z_v^m is stepped
 // by one float64 complex multiplication per element (re-anchored by an exact sincospi every 32
 // elements), the M products theta_m z_v^m are summed in order -- no shuffles at all.
-template <int VP>
-__global__ void k_gains_free_v(Dims d, State s) {
-    const long long gtid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    const int e_raw = (int)(gtid / VP), v = (int)(gtid % VP);
-    const bool act = e_raw < d.E && v < d.V;
-    const int e = min(e_raw, d.E - 1), M = d.M;
-    const size_t ev = (size_t)e * d.V + min(v, d.V - 1);
-    const double delta = d.angle_BR - s.angle[ev];
+// gains_free_lane is the per-vehicle body: theta_m = (tr[m * ts], ti[m * ts]) (ts = 1: the state arrays; ts = 2: an
+// interleaved double2 copy in shared memory).  Shared by k_gains_free_v and the fused episode start.
+__device__ __forceinline__ double gains_free_lane(const Dims& d, double angle, double amp, const double* tr,
+                                                  const double* ti, int ts) {
+    const int M = d.M;
+    const double delta = d.angle_BR - angle;
     const double2 z = unit_phasor64(delta);
-    const double* tr = s.theta_re + (size_t)e * M;
-    const double* ti = s.theta_im + (size_t)e * M;
     double sr = 0.0, si = 0.0;
     double2 w = make_double2(1.0, 0.0);
     for (int m = 0; m < M; ++m) {
         if ((m & 31) == 0 && m) w = unit_phasor64((double)m * delta);
-        const double a = tr[m], b = ti[m];
+        const double a = tr[(size_t)m * ts], b = ti[(size_t)m * ts];
         sr += a * w.x - b * w.y;
         si += a * w.y + b * w.x;
         w = cmul64(w, z);
     }
-    if (act) s.gains[ev] = s.amp[ev] * (sr * sr + si * si);
+    return amp * (sr * sr + si * si);
+}
+
+template <int VP>
+__global__ void k_gains_free_v(Dims d, State s, EnvGate g) {
+    const long long gtid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    const int e_raw = (int)(gtid / VP), v = (int)(gtid % VP);
+    const int e = min(e_raw, d.E - 1), M = d.M;
+    const bool act = e_raw < d.E && v < d.V && g.on(e);
+    const size_t ev = (size_t)e * d.V + min(v, d.V - 1);
+    const double gain = gains_free_lane(d, s.angle[ev], s.amp[ev], s.theta_re + (size_t)e * M,
+                                        s.theta_im + (size_t)e * M, 1);
+    if (act) s.gains[ev] = gain;
 }
 
 // update_channel_gains, "free" model (MARL:263-273): the cascaded RIS reduction
 //   gain_v = amp_v * | sum_m theta_m * phasor(v, m) |^2
 // one warp per env, lanes stride over the M elements, complex warp-shuffle reduction.
-__global__ void k_gains_free(Dims d, State s) {
+__global__ void k_gains_free(Dims d, State s, EnvGate g) {
     const int wpb = blockDim.x >> 5;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int e = blockIdx.x * wpb + warp;
-    if (e >= d.E) return;
+    if (e >= d.E || !g.on(e)) return;
     const int V = d.V, M = d.M;
     for (int v = 0; v < V; ++v) {
         const double delta = d.angle_BR - s.angle[(size_t)e * V + v];
@@ -305,19 +321,22 @@ __global__ void k_gains_free(Dims d, State s) {
 // then exponential (K = 0) or two normals.
 __global__ void k_gains_3gpp(Dims d, State s, risvec_params_t p, const double* __restrict__ c_rand,
                              const double* __restrict__ c_normal, const double* __restrict__ c_exp,
-                             unsigned long long call) {
+                             unsigned long long call_host, EnvGate g) {
     const size_t ix = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (ix >= (size_t)d.E * d.V) return;
     const int e = (int)(ix / d.V), v = (int)(ix % d.V);
+    if (!g.on(e)) return;
+    const unsigned long long call = g.key(e, call_host);
+    const unsigned kind = g.kind(kRngChannel, kRngEpChannel);
     double u, z0, z1, z2, ex;
     if (c_rand != nullptr) {
         u = c_rand[ix];
         z0 = c_normal[ix * 3 + 0]; z1 = c_normal[ix * 3 + 1]; z2 = c_normal[ix * 3 + 2];
         ex = c_exp[ix];
     } else {
-        const uint4 a = rng_draw(d, e, call, (unsigned)(v * 4 + 0), kRngChannel);
-        const uint4 b = rng_draw(d, e, call, (unsigned)(v * 4 + 1), kRngChannel);
-        const uint4 c = rng_draw(d, e, call, (unsigned)(v * 4 + 2), kRngChannel);
+        const uint4 a = rng_draw(d, e, call, (unsigned)(v * 4 + 0), kind);
+        const uint4 b = rng_draw(d, e, call, (unsigned)(v * 4 + 1), kind);
+        const uint4 c = rng_draw(d, e, call, (unsigned)(v * 4 + 2), kind);
         u = u01d(a.x, a.y);
         ex = -log1p(-u01d(a.z, a.w));
         // Box-Muller pairs

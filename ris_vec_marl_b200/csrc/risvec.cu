@@ -15,6 +15,7 @@
 #include "sarl_umma.cuh"
 #include "marl_tma.cuh"
 #include "pairing.cuh"
+#include "episode.cuh"
 #include "replay.cuh"
 
 using namespace risvec;
@@ -96,6 +97,8 @@ struct risvec_env {
     const char* step_kernel;  // name of the kernel(s) the latest rollout launched (risvec_last_step_kernel)
     double* stats_slots;      // attached statistics accumulator (risvec_attach_stats_accumulator) or null
     int stats_folded;         // the latest rollout kernel added its statistics itself
+    unsigned char* ep_bits;   // [E] in the arena: stage bits of the current tick (episode clock, unfused shapes)
+    int* ep_keys;             // [E] in the arena: episode index that keys the tick's draws (same)
 };
 
 struct risvec_replay {
@@ -446,6 +449,15 @@ __global__ void __launch_bounds__(1024) k_shard_stats(Dims d, State s, double* o
     if (threadIdx.x <= RISVEC_NSTAT) atomicAdd(out + threadIdx.x, red[0][threadIdx.x]);
 }
 
+int launch_make_new_game(risvec_env* env, const uint8_t* env_mask, const int32_t* reset_ints, int n_ints,
+                         const int32_t* reset_dirs, int n_dirs, EnvGate g, void* stream);
+int launch_renew_positions(risvec_env* env, const double* uniforms, int n, int32_t* used_out, EnvGate g, void* stream);
+int launch_compute_parms(risvec_env* env, EnvGate g, void* stream);
+int launch_bcd(risvec_env* env, EnvGate g, void* stream);
+int launch_gains(risvec_env* env, const double* chan_rand, const double* chan_normal, const double* chan_exp, EnvGate g,
+                 void* stream);
+int launch_pair_reset(risvec_env* env, const uint8_t* env_mask, EnvGate g, void* stream);
+
 }  // namespace
 
 // ======================================================================================
@@ -555,13 +567,18 @@ int risvec_create(const risvec_params_t* params, int variant, int E, int V, int 
         {RISVEC_F_PAIR_HIST, E, V * V, 4, 1}, {RISVEC_F_PAIR_STREAK, E, V, 4, 0}, {RISVEC_F_PAIR_TAU, E, 1, 8, 1},
         {RISVEC_F_PAIR_K, E, 1, 4, 0}, {RISVEC_F_PAIR_MASK, E, V * V, 1, 0}, {RISVEC_F_PAIR_ROUNDS, E, 1, 4, 0},
         {RISVEC_F_NOMA_PARTNER, E, V, 4, 0}, {RISVEC_F_NOMA_NGROUPS, E, 1, 4, 0}, {RISVEC_F_NOMA_PAIRS, E, V, 4, 0},
-        {RISVEC_F_NOMA_NPAIRS, E, 1, 4, 0}};
+        {RISVEC_F_NOMA_NPAIRS, E, 1, 4, 0},
+        {RISVEC_F_EP_STEP, E, 1, 4, 0}, {RISVEC_F_EP_INDEX, E, 1, 4, 0}};
     size_t off = 0;
     for (int i = 0; i < RISVEC_F_COUNT; ++i) {
         const Spec& sp = specs[i];
         env->fields[sp.f] = {off, sp.rows, sp.cols, sp.eb, sp.fl};
         off = align_up(off + (size_t)sp.rows * sp.cols * sp.eb, 256);
     }
+    const size_t ep_bits_off = off;  // hand-over of the episode clock to the per-stage kernels (not a field)
+    off = align_up(off + (size_t)E, 256);
+    const size_t ep_keys_off = off;
+    off = align_up(off + (size_t)E * 4, 256);
     env->arena_bytes = off;
     cudaError_t ce = cudaMalloc((void**)&env->arena, env->arena_bytes);
     if (ce != cudaSuccess) {
@@ -575,6 +592,8 @@ int risvec_create(const risvec_params_t* params, int variant, int E, int V, int 
         return fail(RISVEC_ERR_CUDA, "cudaMemset: %s", cudaGetErrorString(ce));
     }
     bind_state(env);
+    env->ep_bits = (unsigned char*)(env->arena + ep_bits_off);
+    env->ep_keys = (int*)(env->arena + ep_keys_off);
     *out = env;
     return RISVEC_OK;
 }
@@ -637,29 +656,20 @@ int risvec_make_new_game_masked(risvec_env_t* env, const uint8_t* env_mask, cons
     if (reset_ints == nullptr && reset_dirs != nullptr)
         return fail(RISVEC_ERR_INVALID, "reset_dirs given without reset_ints");
     ENTER_DEVICE(env->device);
-    const int threads = 128, blocks = (env->dims.E + threads - 1) / threads;
-    k_make_new_game<<<blocks, threads, 0, (cudaStream_t)stream>>>(env->dims, env->st, env->params, reset_ints, n_ints,
-                                                                  reset_dirs, n_dirs, env->reset_calls++, env_mask);
-    return check_launch(env, "k_make_new_game");
+    return launch_make_new_game(env, env_mask, reset_ints, n_ints, reset_dirs, n_dirs, EnvGate{}, stream);
 }
 
 int risvec_renew_positions(risvec_env_t* env, const double* uniforms, int n, int32_t* used_out, void* stream) {
     if (!env) return fail(RISVEC_ERR_INVALID, "NULL handle");
     if (uniforms != nullptr && n < 1) return fail(RISVEC_ERR_INVALID, "uniforms given with n = %d", n);
     ENTER_DEVICE(env->device);
-    const int threads = 128, blocks = (env->dims.E + threads - 1) / threads;
-    k_renew_positions<<<blocks, threads, 0, (cudaStream_t)stream>>>(env->dims, env->st, env->params, uniforms, n,
-                                                                    used_out, env->mob_calls++);
-    return check_launch(env, "k_renew_positions");
+    return launch_renew_positions(env, uniforms, n, used_out, EnvGate{}, stream);
 }
 
 int risvec_compute_parms(risvec_env_t* env, void* stream) {
     if (!env) return fail(RISVEC_ERR_INVALID, "NULL handle");
     ENTER_DEVICE(env->device);
-    const long long n = (long long)env->dims.E * env->dims.V;
-    const int threads = 256, blocks = (int)((n + threads - 1) / threads);
-    k_compute_parms<<<blocks, threads, 0, (cudaStream_t)stream>>>(env->dims, env->st);
-    return check_launch(env, "k_compute_parms");
+    return launch_compute_parms(env, EnvGate{}, stream);
 }
 
 int risvec_set_phase(risvec_env_t* env, const float* phase, void* stream) {
@@ -674,6 +684,46 @@ int risvec_set_phase(risvec_env_t* env, const float* phase, void* stream) {
 int risvec_optimize_phase_shift(risvec_env_t* env, void* stream) {
     if (!env) return fail(RISVEC_ERR_INVALID, "NULL handle");
     ENTER_DEVICE(env->device);
+    return launch_bcd(env, EnvGate{}, stream);
+}
+
+int risvec_update_channel_gains(risvec_env_t* env, const double* chan_rand, const double* chan_normal,
+                                const double* chan_exp, void* stream) {
+    if (!env) return fail(RISVEC_ERR_INVALID, "NULL handle");
+    const bool any = chan_rand || chan_normal || chan_exp;
+    if (env->params.channel_model != RISVEC_CHANNEL_FREE && any && !(chan_rand && chan_normal && chan_exp))
+        return fail(RISVEC_ERR_INVALID, "chan_rand, chan_normal and chan_exp must be given together");
+    ENTER_DEVICE(env->device);
+    return launch_gains(env, chan_rand, chan_normal, chan_exp, EnvGate{}, stream);
+}
+
+}  // extern "C"
+
+namespace {
+// The per-stage launches behind the plain entry points; `g` restricts them to some envs (the episode-start calls
+// on the shapes k_begin_episode does not take).  A zero gate is exactly the plain entry point.
+int launch_make_new_game(risvec_env* env, const uint8_t* env_mask, const int32_t* reset_ints, int n_ints,
+                         const int32_t* reset_dirs, int n_dirs, EnvGate g, void* stream) {
+    const int threads = 128, blocks = (env->dims.E + threads - 1) / threads;
+    const unsigned long long call = g.call ? 0 : env->reset_calls++;
+    k_make_new_game<<<blocks, threads, 0, (cudaStream_t)stream>>>(env->dims, env->st, env->params, reset_ints, n_ints,
+                                                                  reset_dirs, n_dirs, call, env_mask, g);
+    return check_launch(env, "k_make_new_game");
+}
+int launch_renew_positions(risvec_env* env, const double* uniforms, int n, int32_t* used_out, EnvGate g, void* stream) {
+    const int threads = 128, blocks = (env->dims.E + threads - 1) / threads;
+    const unsigned long long call = g.call ? 0 : env->mob_calls++;
+    k_renew_positions<<<blocks, threads, 0, (cudaStream_t)stream>>>(env->dims, env->st, env->params, uniforms, n,
+                                                                    used_out, call, g);
+    return check_launch(env, "k_renew_positions");
+}
+int launch_compute_parms(risvec_env* env, EnvGate g, void* stream) {
+    const long long n = (long long)env->dims.E * env->dims.V;
+    const int threads = 256, blocks = (int)((n + threads - 1) / threads);
+    k_compute_parms<<<blocks, threads, 0, (cudaStream_t)stream>>>(env->dims, env->st, g);
+    return check_launch(env, "k_compute_parms");
+}
+int launch_bcd(risvec_env* env, EnvGate g, void* stream) {
     if (env->dims.ncand <= 8 && env->dims.V <= 8 && env->dims.M <= 256 && !env->force_generic) {
         // 4 envs per warp, lane = (env, candidate)
         const int wpb = env->dims.M <= 64 ? 4 : 1;
@@ -681,21 +731,18 @@ int risvec_optimize_phase_shift(risvec_env_t* env, void* stream) {
         const size_t smem = (size_t)wpb * 4 * 2 * env->dims.M * sizeof(double2);
         if (smem > 48 * 1024)
             CUDA_TRY(cudaFuncSetAttribute(k_bcd_v8, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        k_bcd_v8<<<blocks, 32 * wpb, smem, (cudaStream_t)stream>>>(env->dims, env->st);
+        k_bcd_v8<<<blocks, 32 * wpb, smem, (cudaStream_t)stream>>>(env->dims, env->st, g);
         return check_launch(env, "k_bcd_v8");
     }
     const int wpb = 4, threads = 32 * wpb, blocks = (env->dims.E + wpb - 1) / wpb;
     const size_t smem = (size_t)wpb * 2 * env->dims.M * sizeof(double2);
     if (smem > 48 * 1024)
         CUDA_TRY(cudaFuncSetAttribute(k_bcd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    k_bcd<<<blocks, threads, smem, (cudaStream_t)stream>>>(env->dims, env->st);
+    k_bcd<<<blocks, threads, smem, (cudaStream_t)stream>>>(env->dims, env->st, g);
     return check_launch(env, "k_bcd");
 }
-
-int risvec_update_channel_gains(risvec_env_t* env, const double* chan_rand, const double* chan_normal,
-                                const double* chan_exp, void* stream) {
-    if (!env) return fail(RISVEC_ERR_INVALID, "NULL handle");
-    ENTER_DEVICE(env->device);
+int launch_gains(risvec_env* env, const double* chan_rand, const double* chan_normal, const double* chan_exp, EnvGate g,
+                 void* stream) {
     if (env->params.channel_model == RISVEC_CHANNEL_FREE) {
         if (!env->force_generic) {  // lane = (env, vehicle), sequential over the elements
             const int VP = pow2ceil(env->dims.V);
@@ -703,28 +750,29 @@ int risvec_update_channel_gains(risvec_env_t* env, const double* chan_rand, cons
             const int threads = 128, blocks = (int)((n + threads - 1) / threads);
             cudaStream_t st = (cudaStream_t)stream;
             switch (VP) {
-                case 1: k_gains_free_v<1><<<blocks, threads, 0, st>>>(env->dims, env->st); break;
-                case 2: k_gains_free_v<2><<<blocks, threads, 0, st>>>(env->dims, env->st); break;
-                case 4: k_gains_free_v<4><<<blocks, threads, 0, st>>>(env->dims, env->st); break;
-                case 8: k_gains_free_v<8><<<blocks, threads, 0, st>>>(env->dims, env->st); break;
-                case 16: k_gains_free_v<16><<<blocks, threads, 0, st>>>(env->dims, env->st); break;
-                default: k_gains_free_v<32><<<blocks, threads, 0, st>>>(env->dims, env->st); break;
+                case 1: k_gains_free_v<1><<<blocks, threads, 0, st>>>(env->dims, env->st, g); break;
+                case 2: k_gains_free_v<2><<<blocks, threads, 0, st>>>(env->dims, env->st, g); break;
+                case 4: k_gains_free_v<4><<<blocks, threads, 0, st>>>(env->dims, env->st, g); break;
+                case 8: k_gains_free_v<8><<<blocks, threads, 0, st>>>(env->dims, env->st, g); break;
+                case 16: k_gains_free_v<16><<<blocks, threads, 0, st>>>(env->dims, env->st, g); break;
+                default: k_gains_free_v<32><<<blocks, threads, 0, st>>>(env->dims, env->st, g); break;
             }
             return check_launch(env, "k_gains_free_v");
         }
         const int wpb = 4, threads = 32 * wpb, blocks = (env->dims.E + wpb - 1) / wpb;
-        k_gains_free<<<blocks, threads, 0, (cudaStream_t)stream>>>(env->dims, env->st);
+        k_gains_free<<<blocks, threads, 0, (cudaStream_t)stream>>>(env->dims, env->st, g);
         return check_launch(env, "k_gains_free");
     }
-    const bool any = chan_rand || chan_normal || chan_exp;
-    if (any && !(chan_rand && chan_normal && chan_exp))
-        return fail(RISVEC_ERR_INVALID, "chan_rand, chan_normal and chan_exp must be given together");
     const long long n = (long long)env->dims.E * env->dims.V;
     const int threads = 128, blocks = (int)((n + threads - 1) / threads);
+    const unsigned long long call = g.call ? 0 : env->chan_calls++;
     k_gains_3gpp<<<blocks, threads, 0, (cudaStream_t)stream>>>(env->dims, env->st, env->params, chan_rand, chan_normal,
-                                                               chan_exp, env->chan_calls++);
+                                                               chan_exp, call, g);
     return check_launch(env, "k_gains_3gpp");
 }
+}  // namespace
+
+extern "C" {
 
 // statistics accumulator attached: kernels that fold the statistics pass set env->stats_folded, every other kernel
 // is followed by k_shard_stats into slot 0
@@ -1288,22 +1336,10 @@ static PairArgs pair_state_args(risvec_env* env) {
     return a;
 }
 
-int risvec_pair_noma(risvec_env_t* env, const risvec_pairing_t* cfg, const float* p01, int64_t p01_env_stride,
-                     int topk, double tau_q, int recalc_mask, const int32_t* reuse, int decay, int new_episode,
-                     void* stream) {
-    if (!env || !cfg || !p01) return fail(RISVEC_ERR_INVALID, "NULL argument");
-    if (new_episode && !recalc_mask)
-        return fail(RISVEC_ERR_INVALID, "new_episode needs recalc_mask (the first step of an episode builds the mask)");
+// the launch shared by risvec_pair_noma and risvec_pair_noma_episodes: `a` carries the state pointers and the
+// per-call episode arguments, the knobs of `cfg` are added here
+static int pair_noma_launch(risvec_env* env, const risvec_pairing_t* cfg, PairArgs a, void* stream) {
     const int V = env->dims.V;
-    if (V > RISVEC_PAIR_MAX_V)
-        return fail(RISVEC_ERR_UNSUPPORTED, "pairing is an exact matching over 2^V subsets: V = %d > %d", V,
-                    RISVEC_PAIR_MAX_V);
-    if (p01_env_stride < V) return fail(RISVEC_ERR_INVALID, "p01_env_stride %lld < V", (long long)p01_env_stride);
-    if (!(tau_q >= 0.0 && tau_q <= 1.0)) return fail(RISVEC_ERR_INVALID, "tau_q must be in [0, 1]");
-    ENTER_DEVICE(env->device);
-    PairArgs a = pair_state_args(env);
-    a.p01 = p01; a.p01_stride = p01_env_stride; a.reuse = reuse;
-    a.topk = topk; a.tau_q = tau_q; a.recalc = recalc_mask != 0; a.decay = decay != 0; a.fresh = new_episode != 0;
     a.min_pairs = cfg->min_pair_target > 1 ? cfg->min_pair_target : 1;
     a.backoff_rounds = cfg->mwm_backoff_rounds;
     a.accept_q = cfg->mwm_accept_quantile; a.accept_q_step = cfg->mwm_accept_q_step;
@@ -1329,16 +1365,161 @@ int risvec_pair_noma(risvec_env_t* env, const risvec_pairing_t* cfg, const float
     return check_launch(env, "k_pair_noma");
 }
 
+int risvec_pair_noma(risvec_env_t* env, const risvec_pairing_t* cfg, const float* p01, int64_t p01_env_stride,
+                     int topk, double tau_q, int recalc_mask, const int32_t* reuse, int decay, int new_episode,
+                     void* stream) {
+    if (!env || !cfg || !p01) return fail(RISVEC_ERR_INVALID, "NULL argument");
+    if (new_episode && !recalc_mask)
+        return fail(RISVEC_ERR_INVALID, "new_episode needs recalc_mask (the first step of an episode builds the mask)");
+    const int V = env->dims.V;
+    if (V > RISVEC_PAIR_MAX_V)
+        return fail(RISVEC_ERR_UNSUPPORTED, "pairing is an exact matching over 2^V subsets: V = %d > %d", V,
+                    RISVEC_PAIR_MAX_V);
+    if (p01_env_stride < V) return fail(RISVEC_ERR_INVALID, "p01_env_stride %lld < V", (long long)p01_env_stride);
+    if (!(tau_q >= 0.0 && tau_q <= 1.0)) return fail(RISVEC_ERR_INVALID, "tau_q must be in [0, 1]");
+    ENTER_DEVICE(env->device);
+    PairArgs a = pair_state_args(env);
+    a.p01 = p01; a.p01_stride = p01_env_stride; a.reuse = reuse;
+    a.topk = topk; a.tau_q = tau_q; a.recalc = recalc_mask != 0; a.decay = decay != 0; a.fresh = new_episode != 0;
+    return pair_noma_launch(env, cfg, a, stream);
+}
+
+int risvec_pair_noma_episodes(risvec_env_t* env, const risvec_pairing_t* cfg, const float* p01, int64_t p01_env_stride,
+                              const risvec_pair_schedule_t* schedule, const uint8_t* start, const int32_t* reuse,
+                              int decay, void* stream) {
+    if (!env || !cfg || !p01 || !schedule || !start) return fail(RISVEC_ERR_INVALID, "NULL argument");
+    const int V = env->dims.V;
+    if (V > RISVEC_PAIR_MAX_V)
+        return fail(RISVEC_ERR_UNSUPPORTED, "pairing is an exact matching over 2^V subsets: V = %d > %d", V,
+                    RISVEC_PAIR_MAX_V);
+    if (p01_env_stride < V) return fail(RISVEC_ERR_INVALID, "p01_env_stride %lld < V", (long long)p01_env_stride);
+    const double q0 = schedule->tau_q_start, q1 = schedule->tau_q_end;
+    if (!(q0 >= 0.0 && q0 <= 1.0 && q1 >= 0.0 && q1 <= 1.0))
+        return fail(RISVEC_ERR_INVALID, "schedule tau_q_start / tau_q_end must be in [0, 1]");
+    ENTER_DEVICE(env->device);
+    PairArgs a = pair_state_args(env);
+    a.p01 = p01; a.p01_stride = p01_env_stride; a.reuse = reuse; a.decay = decay != 0;
+    a.start = start;
+    a.ep_index = (const int*)(env->arena + env->fields[RISVEC_F_EP_INDEX].offset);
+    a.sched_topk_start = schedule->topk_start; a.sched_topk_end = schedule->topk_end;
+    a.sched_warmup = schedule->warmup_episodes;
+    a.sched_tau_q_start = q0; a.sched_tau_q_end = q1;
+    return pair_noma_launch(env, cfg, a, stream);
+}
+
 int risvec_pair_reset(risvec_env_t* env, void* stream) { return risvec_pair_reset_masked(env, nullptr, stream); }
 
 int risvec_pair_reset_masked(risvec_env_t* env, const uint8_t* env_mask, void* stream) {
     if (!env) return fail(RISVEC_ERR_INVALID, "NULL handle");
     ENTER_DEVICE(env->device);
+    return launch_pair_reset(env, env_mask, EnvGate{}, stream);
+}
+
+}  // extern "C"
+
+namespace {
+int launch_pair_reset(risvec_env* env, const uint8_t* env_mask, EnvGate g, void* stream) {
     PairArgs a = pair_state_args(env);
     const long long n = (long long)env->dims.E * env->dims.V * env->dims.V;
     const int threads = 256, blocks = (int)((n + threads - 1) / threads);
-    k_pair_reset<<<blocks, threads, 0, (cudaStream_t)stream>>>(env->dims, a, env_mask);
+    k_pair_reset<<<blocks, threads, 0, (cudaStream_t)stream>>>(env->dims, a, env_mask, g);
     return check_launch(env, "k_pair_reset");
+}
+
+constexpr int kEpAll = RISVEC_EP_RESET | RISVEC_EP_POSITIONS | RISVEC_EP_CHANNEL | RISVEC_EP_PAIRING;
+
+// k_begin_episode takes the shapes of k_bcd_v8 with the free channel
+bool episode_fused(const risvec_env* env) {
+    const Dims& d = env->dims;
+    return d.V <= 8 && d.ncand <= 8 && d.M <= 256 && env->params.channel_model == RISVEC_CHANNEL_FREE &&
+           !env->force_generic;
+}
+
+template <bool CLOCK>
+int launch_begin_episode(risvec_env* env, const EpisodeArgs& a, void* stream) {
+    const int wpb = env->dims.M <= 64 ? 4 : 1;  // as k_bcd_v8: 4 envs per warp, 2 M double2 of shared memory per env
+    const int blocks = (env->dims.E + 4 * wpb - 1) / (4 * wpb);
+    const size_t smem = (size_t)wpb * 4 * 2 * env->dims.M * sizeof(double2);
+    if (smem > 48 * 1024)
+        CUDA_TRY(cudaFuncSetAttribute(k_begin_episode<CLOCK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    k_begin_episode<CLOCK><<<blocks, 32 * wpb, smem, (cudaStream_t)stream>>>(env->dims, env->st, env->params,
+                                                                              pair_state_args(env), a);
+    return check_launch(env, "k_begin_episode");
+}
+
+// the stages `stages` as separate kernels restricted by `g` (g.bits null = every env), in the fixed order
+int episode_stages_separate(risvec_env* env, int stages, EnvGate g, const double* uniforms, int n_uni, int32_t* used_out,
+                            void* stream) {
+    auto gate = [&](unsigned bit) { EnvGate h = g; h.bit = bit; return h; };
+    if (stages & RISVEC_EP_RESET)
+        if (int rc = launch_make_new_game(env, nullptr, nullptr, 0, nullptr, 0, gate(RISVEC_EP_RESET), stream)) return rc;
+    if (stages & RISVEC_EP_POSITIONS) {
+        if (int rc = launch_renew_positions(env, uniforms, n_uni, used_out, gate(RISVEC_EP_POSITIONS), stream)) return rc;
+        if (int rc = launch_compute_parms(env, gate(RISVEC_EP_POSITIONS), stream)) return rc;
+    }
+    if (stages & RISVEC_EP_CHANNEL) {
+        if (int rc = launch_bcd(env, gate(RISVEC_EP_CHANNEL), stream)) return rc;
+        if (int rc = launch_gains(env, nullptr, nullptr, nullptr, gate(RISVEC_EP_CHANNEL), stream)) return rc;
+    }
+    if (stages & RISVEC_EP_PAIRING)
+        if (int rc = launch_pair_reset(env, nullptr, gate(RISVEC_EP_PAIRING), stream)) return rc;
+    return RISVEC_OK;
+}
+}  // namespace
+
+extern "C" {
+
+int risvec_begin_episode(risvec_env_t* env, const uint8_t* stages_env, int stages, const double* uniforms, int n_uni,
+                         int32_t* used_out, void* stream) {
+    if (!env) return fail(RISVEC_ERR_INVALID, "NULL handle");
+    if (stages & ~kEpAll) return fail(RISVEC_ERR_INVALID, "unknown stage bits 0x%x", stages & ~kEpAll);
+    if (uniforms != nullptr && n_uni < 1) return fail(RISVEC_ERR_INVALID, "uniforms given with n_uni = %d", n_uni);
+    if (stages == 0) return RISVEC_OK;
+    if (!(stages & RISVEC_EP_POSITIONS)) {  // nothing renews: the uniforms and used_out are not touched
+        uniforms = nullptr;
+        used_out = nullptr;
+    }
+    ENTER_DEVICE(env->device);
+    if (!episode_fused(env)) {
+        EnvGate g{};
+        g.bits = stages_env;
+        return episode_stages_separate(env, stages, g, uniforms, n_uni, used_out, stream);
+    }
+    EpisodeArgs a;
+    memset(&a, 0, sizeof(a));
+    a.stages = (unsigned)stages; a.stages_env = stages_env;
+    a.uniforms = uniforms; a.n_uni = n_uni; a.used_out = used_out;
+    a.reset_call = env->reset_calls; a.mob_call = env->mob_calls;
+    if (int rc = launch_begin_episode<false>(env, a, stream)) return rc;
+    // the counters advance as the separate calls advance them (the free channel draws nothing)
+    if (stages & RISVEC_EP_RESET) env->reset_calls++;
+    if (stages & RISVEC_EP_POSITIONS) env->mob_calls++;
+    return RISVEC_OK;
+}
+
+int risvec_episode_tick(risvec_env_t* env, const risvec_episode_schedule_t* schedule, uint8_t* start_out,
+                        uint8_t* done_out, void* stream) {
+    if (!env || !schedule) return fail(RISVEC_ERR_INVALID, "NULL argument");
+    if (schedule->steps_per_episode < 1 || schedule->positions_every < 1)
+        return fail(RISVEC_ERR_INVALID, "steps_per_episode and positions_every must be >= 1");
+    if (schedule->stages & ~kEpAll) return fail(RISVEC_ERR_INVALID, "unknown stage bits 0x%x", schedule->stages & ~kEpAll);
+    ENTER_DEVICE(env->device);
+    EpisodeArgs a;
+    memset(&a, 0, sizeof(a));
+    a.stages = (unsigned)schedule->stages;
+    a.ep_step = (int*)(env->arena + env->fields[RISVEC_F_EP_STEP].offset);
+    a.ep_index = (int*)(env->arena + env->fields[RISVEC_F_EP_INDEX].offset);
+    a.steps_per_episode = schedule->steps_per_episode; a.positions_every = schedule->positions_every;
+    a.start_out = start_out; a.done_out = done_out;
+    if (episode_fused(env)) return launch_begin_episode<true>(env, a, stream);
+    // other shapes: the clock writes each env's bits and draw key, then the stage kernels run for those envs
+    a.bits_out = env->ep_bits; a.key_out = env->ep_keys;
+    k_episode_clock<<<(env->dims.E + 127) / 128, 128, 0, (cudaStream_t)stream>>>(env->dims, a);
+    if (int rc = check_launch(env, "k_episode_clock")) return rc;
+    EnvGate g{};
+    g.bits = env->ep_bits;
+    g.call = env->ep_keys;
+    return episode_stages_separate(env, schedule->stages, g, nullptr, 0, nullptr, stream);
 }
 
 int risvec_replay_create(int device, int64_t mem_size, int input_shape, int n_actions, int n_agents,
