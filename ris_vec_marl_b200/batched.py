@@ -250,27 +250,34 @@ class BatchedEnviron:
         return self._views["gains"]
 
     # ------------------------------------------------------------------ steps / rollouts
-    def _alloc_traces(self, names, T, all_names):
+    def _trace_shape(self, name, T):
         E, V = self.E, self.V
-        shapes = {"reward": (T, E), "stats": (T, E, NSTAT), "last_power": (T, E, 2, V)}
+        return {"reward": (T, E), "stats": (T, E, NSTAT), "last_power": (T, E, 2, V)}.get(name, (T, E, V))
+
+    def _alloc_traces(self, names, T, all_names):
         out = {}
         for n in names:
             if n not in all_names:
                 raise ValueError(f"unknown trace {n!r}")
-            out[n] = torch.empty(shapes.get(n, (T, E, V)), dtype=torch.float32, device=self.device)
+            out[n] = torch.empty(self._trace_shape(n, T), dtype=torch.float32, device=self.device)
         return out
 
-    def _check_out(self, out, T, all_names):
-        """Preallocated traces go to the kernels as raw pointers: refuse anything that is not exactly the
-        buffer `_alloc_traces` would make (name, shape, float32, this device, contiguous)."""
-        shapes = {"reward": (T, self.E), "stats": (T, self.E, NSTAT), "last_power": (T, self.E, 2, self.V)}
+    @staticmethod
+    def _check(name, t, dtype, shape, device):
+        """A caller's tensor goes to the library as a raw pointer, and the library derives every extent it reads or
+        writes from the handle's shape: refuse anything but a contiguous `dtype` tensor of exactly `shape` on
+        `device`.  Never convert: a converted copy is not the buffer the caller reads the results from."""
+        if (not isinstance(t, torch.Tensor) or tuple(t.shape) != tuple(shape) or t.dtype != dtype or t.device != device
+                or not t.is_contiguous()):
+            raise ValueError(f"{name} must be a contiguous {dtype} tensor of shape {tuple(shape)} on {device}")
+
+    def _check_out(self, out, T, all_names, device):
+        """Preallocated traces: the names in `all_names`, each exactly the buffer `_alloc_traces` would make, but on
+        `device`."""
         for k, v in out.items():
             if k not in all_names:
                 raise ValueError(f"unknown trace {k!r}")
-            want = shapes.get(k, (T, self.E, self.V))
-            if (not isinstance(v, torch.Tensor) or tuple(v.shape) != want or v.dtype != torch.float32
-                    or v.device != self.device or not v.is_contiguous()):
-                raise ValueError(f"out[{k!r}] must be a contiguous float32 tensor of shape {want} on {self.device}")
+            self._check(f"out[{k!r}]", v, torch.float32, self._trace_shape(k, T), device)
 
     def rollout_marl(self, actions, partner, ngroups, arrivals=None, traces=MARL_TRACES, out=None):
         """T fused Environ.step calls; actions [T,E,2,V]; returns {trace: tensor [T,...]}.
@@ -285,7 +292,7 @@ class BatchedEnviron:
         if out is None:
             out = self._alloc_traces(traces, T, MARL_TRACES)
         else:
-            self._check_out(out, T, MARL_TRACES)
+            self._check_out(out, T, MARL_TRACES, self.device)
         o = MarlOut(**{k: v.data_ptr() for k, v in out.items()})
         check(self._lib.risvec_rollout_marl(self._h, T, self._p(a), self._p(pt), self._p(ng), self._p(ar), C.byref(o),
                                             self.stream))
@@ -301,7 +308,7 @@ class BatchedEnviron:
         if out is None:
             out = self._alloc_traces(traces, T, SARL_TRACES)
         else:
-            self._check_out(out, T, SARL_TRACES)
+            self._check_out(out, T, SARL_TRACES, self.device)
         o = SarlOut(**{k: v.data_ptr() for k, v in out.items()})
         check(self._lib.risvec_rollout_sarl(self._h, T, self._p(a), self._p(ph), self._p(ar), C.byref(o), self.stream))
         return out
@@ -355,21 +362,37 @@ class BatchedEnviron:
 
     # ---- host-buffer entry points (the end-to-end path: H2D + rollout + D2H on one stream)
     @staticmethod
-    def _hp(t):
-        return C.c_void_p(t.data_ptr()) if t is not None else C.c_void_p(None)
+    def _steps(t):
+        """T of a [T, ...] host argument (None when `t` is no tensor: `_check` then refuses it)."""
+        return t.shape[0] if isinstance(t, torch.Tensor) and t.dim() > 0 else None
 
     def rollout_sarl_host(self, actions, phases, arrivals, out):
-        """`actions/phases/arrivals` and the tensors in `out` are (pinned) HOST tensors."""
-        T = actions.shape[0]
+        """`rollout_sarl` with CPU tensors (pinned for full copy speed): `actions` [T,E,2,V] f32, `phases` [T,E,M]
+        f32, `arrivals` [T,E,V] i32 or None, and the `out` traces, all contiguous.  Other input is refused."""
+        cpu, T = torch.device("cpu"), self._steps(actions)
+        self._check("actions", actions, torch.float32, (T, self.E, 2, self.V), cpu)
+        self._check("phases", phases, torch.float32, (T, self.E, self.M), cpu)
+        if arrivals is not None:
+            self._check("arrivals", arrivals, torch.int32, (T, self.E, self.V), cpu)
+        self._check_out(out, T, SARL_TRACES, cpu)
         o = SarlOut(**{k: v.data_ptr() for k, v in out.items()})
-        check(self._lib.risvec_rollout_sarl_host(self._h, T, self._hp(actions), self._hp(phases), self._hp(arrivals),
+        check(self._lib.risvec_rollout_sarl_host(self._h, T, self._p(actions), self._p(phases), self._p(arrivals),
                                                  C.byref(o), self.stream))
 
     def rollout_marl_host(self, actions, partner, ngroups, arrivals, out):
-        T = actions.shape[0]
+        """`rollout_marl` with CPU tensors (pinned for full copy speed): `actions` [T,E,2,V] f32, `partner` [E,V] i32,
+        `ngroups` [E] i32, `arrivals` [T,E,V] i32 or None, and the `out` traces, all contiguous.  Other input is
+        refused."""
+        cpu, T = torch.device("cpu"), self._steps(actions)
+        self._check("actions", actions, torch.float32, (T, self.E, 2, self.V), cpu)
+        self._check("partner", partner, torch.int32, (self.E, self.V), cpu)
+        self._check("ngroups", ngroups, torch.int32, (self.E,), cpu)
+        if arrivals is not None:
+            self._check("arrivals", arrivals, torch.int32, (T, self.E, self.V), cpu)
+        self._check_out(out, T, MARL_TRACES, cpu)
         o = MarlOut(**{k: v.data_ptr() for k, v in out.items()})
-        check(self._lib.risvec_rollout_marl_host(self._h, T, self._hp(actions), self._hp(partner), self._hp(ngroups),
-                                                 self._hp(arrivals), C.byref(o), self.stream))
+        check(self._lib.risvec_rollout_marl_host(self._h, T, self._p(actions), self._p(partner), self._p(ngroups),
+                                                 self._p(arrivals), C.byref(o), self.stream))
 
     # ---- packed record layout: the native streaming format for V == 8 (include/risvec.h)
     def pack_inputs(self, actions, arrivals, phases=None):
@@ -420,14 +443,22 @@ class BatchedEnviron:
         return out_rec, reward
 
     def rollout_packed_host(self, in_rec, out_rec, reward, partner=None, ngroups=None):
-        """Same with (pinned) HOST record tensors: chunked H2D -> rollout -> D2H pipeline."""
-        T = in_rec.shape[0]
+        """Same with CPU tensors (pinned for full copy speed), all contiguous f32 unless noted: `in_rec`
+        [T, E/4, 4*W_in], `out_rec` [T, E/4, 4*W_out], `reward` [T, E]; MARL also `partner` [E,V] i32 and `ngroups`
+        [E] i32.  Other input is refused.  Chunked H2D -> rollout -> D2H pipeline."""
+        cpu, T, G = torch.device("cpu"), self._steps(in_rec), self.E // 4
+        w_in = _lib.sarl_in_words(self.M) if self.variant == "sarl" else _lib.MARL_IN_WORDS
+        self._check("in_rec", in_rec, torch.float32, (T, G, 4 * w_in), cpu)
+        self._check("out_rec", out_rec, torch.float32, (T, G, 4 * self.packed_out_words()), cpu)
+        self._check("reward", reward, torch.float32, (T, self.E), cpu)
         if self.variant == "sarl":
-            check(self._lib.risvec_rollout_sarl_packed_host(self._h, T, self._hp(in_rec), self._hp(out_rec),
-                                                            self._hp(reward), self.stream))
+            check(self._lib.risvec_rollout_sarl_packed_host(self._h, T, self._p(in_rec), self._p(out_rec),
+                                                            self._p(reward), self.stream))
         else:
-            check(self._lib.risvec_rollout_marl_packed_host(self._h, T, self._hp(in_rec), self._hp(partner),
-                                                            self._hp(ngroups), self._hp(out_rec), self._hp(reward),
+            self._check("partner", partner, torch.int32, (self.E, self.V), cpu)
+            self._check("ngroups", ngroups, torch.int32, (self.E,), cpu)
+            check(self._lib.risvec_rollout_marl_packed_host(self._h, T, self._p(in_rec), self._p(partner),
+                                                            self._p(ngroups), self._p(out_rec), self._p(reward),
                                                             self.stream))
 
     # ---- driver-side glue on device (SURVEY.md 8f row 1)

@@ -1,4 +1,5 @@
 // C ABI of the risvec library (include/risvec.h): handle, state arena, launches.
+#include <algorithm>
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
@@ -88,7 +89,7 @@ struct risvec_env {
     size_t scratch_bytes;
     int pipe_ready;
     cudaStream_t s_in, s_out;
-    cudaEvent_t ev[2 * 64 + 2];  // 2 * kMaxChunks + 2
+    cudaEvent_t ev[2 * 64 + 3];  // 2 * kMaxChunks + 3: per chunk in / kernel, start, in done, done
     int force_generic;  // RISVEC_FORCE_GENERIC=1: always use the shape-generic kernels (tests)
     int sarl_umma;      // large shapes: k_sarl_umma (tcgen05) unless RISVEC_SARL_PATH=mma-sync (k_sarl_mma_big)
     int sarl_path;      // RISVEC_SARL_PATH = auto (0) | mma (1) | v8 (2) | generic (3): tests / A-B runs
@@ -607,7 +608,7 @@ int risvec_destroy(risvec_env_t* env) {
     if (env->pipe_ready) {
         cudaStreamDestroy(env->s_in);
         cudaStreamDestroy(env->s_out);
-        for (int i = 0; i < 2 * 64 + 2; ++i) cudaEventDestroy(env->ev[i]);
+        for (cudaEvent_t e : env->ev) cudaEventDestroy(e);
     }
     delete env;
     return RISVEC_OK;
@@ -770,6 +771,49 @@ int launch_gains(risvec_env* env, const double* chan_rand, const double* chan_no
                                                                chan_exp, call, g);
     return check_launch(env, "k_gains_3gpp");
 }
+
+// Argument checks shared by each rollout entry point and its `_host` form: both refuse the same input with the same
+// message, and the `_host` form does so before it enqueues a copy.
+int check_marl_args(const risvec_env* env, int T, const void* action, const void* partner, const void* ngroups) {
+    if (!env) return fail(RISVEC_ERR_INVALID, "NULL handle");
+    if (env->dims.variant != RISVEC_VARIANT_MARL) return fail(RISVEC_ERR_INVALID, "handle is not a MARL env");
+    if (T < 1) return fail(RISVEC_ERR_INVALID, "T must be >= 1 (got %d)", T);
+    if (!action || !partner || !ngroups) return fail(RISVEC_ERR_INVALID, "action, partner and ngroups are required");
+    return RISVEC_OK;
+}
+int check_sarl_args(const risvec_env* env, int T, const void* action, const void* phase) {
+    if (!env) return fail(RISVEC_ERR_INVALID, "NULL handle");
+    if (env->dims.variant != RISVEC_VARIANT_SARL) return fail(RISVEC_ERR_INVALID, "handle is not a SARL env");
+    if (T < 1) return fail(RISVEC_ERR_INVALID, "T must be >= 1 (got %d)", T);
+    if (!action || !phase) return fail(RISVEC_ERR_INVALID, "action and phase are required");
+    return RISVEC_OK;
+}
+// ---- packed record layout (include/risvec.h): one input / one output stream per rollout
+int packed_sarl_mpi(const risvec_env* env) {  // 0 = shape not covered by the packed kernels
+    const int V = env->dims.V, M = env->dims.M;
+    if (V != 8 || env->dims.E % 4 != 0) return 0;
+    return M == 16 ? 2 : (M == 40 ? 5 : 0);
+}
+int check_sarl_packed_args(const risvec_env* env, int T, const void* in_rec, const void* out_rec, const void* reward) {
+    if (!env) return fail(RISVEC_ERR_INVALID, "NULL handle");
+    if (env->dims.variant != RISVEC_VARIANT_SARL) return fail(RISVEC_ERR_INVALID, "handle is not a SARL env");
+    if (T < 1 || !in_rec || !out_rec || !reward) return fail(RISVEC_ERR_INVALID, "T >= 1 and all three buffers are required");
+    if (!packed_sarl_mpi(env))
+        return fail(RISVEC_ERR_UNSUPPORTED, "packed SARL records need V == 8, E %% 4 == 0 and M in {16, 40} "
+                    "(got V = %d, E = %d, M = %d)", env->dims.V, env->dims.E, env->dims.M);
+    return RISVEC_OK;
+}
+int check_marl_packed_args(const risvec_env* env, int T, const void* in_rec, const void* partner, const void* ngroups,
+                           const void* out_rec, const void* reward) {
+    if (!env) return fail(RISVEC_ERR_INVALID, "NULL handle");
+    if (env->dims.variant != RISVEC_VARIANT_MARL) return fail(RISVEC_ERR_INVALID, "handle is not a MARL env");
+    if (T < 1 || !in_rec || !partner || !ngroups || !out_rec || !reward)
+        return fail(RISVEC_ERR_INVALID, "T >= 1 and all buffers are required");
+    if (env->dims.V != 8 || env->dims.E % 4 != 0)
+        return fail(RISVEC_ERR_UNSUPPORTED, "packed MARL records need V == 8 and E %% 4 == 0 (got V = %d, E = %d)",
+                    env->dims.V, env->dims.E);
+    return RISVEC_OK;
+}
 }  // namespace
 
 extern "C" {
@@ -799,10 +843,7 @@ int risvec_rollout_sarl(risvec_env_t* env, int T, const float* action, const flo
 
 static int rollout_marl_impl(risvec_env_t* env, int T, const float* action, const int32_t* partner, const int32_t* ngroups,
                              const int32_t* arrivals, const risvec_marl_out_t* out, void* stream) {
-    if (!env) return fail(RISVEC_ERR_INVALID, "NULL handle");
-    if (env->dims.variant != RISVEC_VARIANT_MARL) return fail(RISVEC_ERR_INVALID, "handle is not a MARL env");
-    if (T < 1) return fail(RISVEC_ERR_INVALID, "T must be >= 1 (got %d)", T);
-    if (!action || !partner || !ngroups) return fail(RISVEC_ERR_INVALID, "action, partner and ngroups are required");
+    if (int rc = check_marl_args(env, T, action, partner, ngroups)) return rc;
     ENTER_DEVICE(env->device);
     MarlArgs a;
     memset(&a, 0, sizeof(a));
@@ -858,10 +899,7 @@ static int rollout_marl_impl(risvec_env_t* env, int T, const float* action, cons
 
 static int rollout_sarl_impl(risvec_env_t* env, int T, const float* action, const float* phase, const int32_t* arrivals,
                              const risvec_sarl_out_t* out, void* stream) {
-    if (!env) return fail(RISVEC_ERR_INVALID, "NULL handle");
-    if (env->dims.variant != RISVEC_VARIANT_SARL) return fail(RISVEC_ERR_INVALID, "handle is not a SARL env");
-    if (T < 1) return fail(RISVEC_ERR_INVALID, "T must be >= 1 (got %d)", T);
-    if (!action || !phase) return fail(RISVEC_ERR_INVALID, "action and phase are required");
+    if (int rc = check_sarl_args(env, T, action, phase)) return rc;
     ENTER_DEVICE(env->device);
     SarlArgs a;
     memset(&a, 0, sizeof(a));
@@ -880,40 +918,20 @@ static int rollout_sarl_impl(risvec_env_t* env, int T, const float* action, cons
     }
 }
 
-// ---- packed record layout (include/risvec.h): one input / one output stream per rollout
-namespace {
-int packed_sarl_mpi(const risvec_env* env) {  // 0 = shape not covered by the packed kernels
-    const int V = env->dims.V, M = env->dims.M;
-    if (V != 8 || env->dims.E % 4 != 0) return 0;
-    return M == 16 ? 2 : (M == 40 ? 5 : 0);
-}
-}  // namespace
-
 int risvec_rollout_sarl_packed(risvec_env_t* env, int T, const void* in_rec, float* out_rec, float* reward,
                                void* stream) {
-    if (!env) return fail(RISVEC_ERR_INVALID, "NULL handle");
-    if (env->dims.variant != RISVEC_VARIANT_SARL) return fail(RISVEC_ERR_INVALID, "handle is not a SARL env");
-    if (T < 1 || !in_rec || !out_rec || !reward) return fail(RISVEC_ERR_INVALID, "T >= 1 and all three buffers are required");
-    const int mpi = packed_sarl_mpi(env);
-    if (!mpi)
-        return fail(RISVEC_ERR_UNSUPPORTED, "packed SARL records need V == 8, E %% 4 == 0 and M in {16, 40} "
-                    "(got V = %d, E = %d, M = %d)", env->dims.V, env->dims.E, env->dims.M);
+    if (int rc = check_sarl_packed_args(env, T, in_rec, out_rec, reward)) return rc;
     ENTER_DEVICE(env->device);
     SarlArgs a;
     memset(&a, 0, sizeof(a));
     a.T = T; a.in_rec = (const float*)in_rec; a.out_rec = out_rec; a.out.reward = reward;
-    return mpi == 2 ? launch_sarl_v8<2>(env, a, (cudaStream_t)stream) : launch_sarl_v8<5>(env, a, (cudaStream_t)stream);
+    return packed_sarl_mpi(env) == 2 ? launch_sarl_v8<2>(env, a, (cudaStream_t)stream)
+                                     : launch_sarl_v8<5>(env, a, (cudaStream_t)stream);
 }
 
 int risvec_rollout_marl_packed(risvec_env_t* env, int T, const void* in_rec, const int32_t* partner,
                                const int32_t* ngroups, float* out_rec, float* reward, void* stream) {
-    if (!env) return fail(RISVEC_ERR_INVALID, "NULL handle");
-    if (env->dims.variant != RISVEC_VARIANT_MARL) return fail(RISVEC_ERR_INVALID, "handle is not a MARL env");
-    if (T < 1 || !in_rec || !partner || !ngroups || !out_rec || !reward)
-        return fail(RISVEC_ERR_INVALID, "T >= 1 and all buffers are required");
-    if (env->dims.V != 8 || env->dims.E % 4 != 0)
-        return fail(RISVEC_ERR_UNSUPPORTED, "packed MARL records need V == 8 and E %% 4 == 0 (got V = %d, E = %d)",
-                    env->dims.V, env->dims.E);
+    if (int rc = check_marl_packed_args(env, T, in_rec, partner, ngroups, out_rec, reward)) return rc;
     ENTER_DEVICE(env->device);
     MarlArgs a;
     memset(&a, 0, sizeof(a));
@@ -923,6 +941,8 @@ int risvec_rollout_marl_packed(risvec_env_t* env, int T, const void* in_rec, con
     k_marl_v8<true, true><<<warps, 32, 0, (cudaStream_t)stream>>>(env->dims, env->st, env->params, a);
     return check_step_launch(env, "k_marl_v8");
 }
+
+}  // extern "C"
 
 // ---- host-buffer variants.  The T steps are cut into chunks and pipelined over three streams:
 // chunk c+1 is copied in (H2D engine) while chunk c computes on the caller's stream and
@@ -935,8 +955,7 @@ int ensure_pipe(risvec_env* env) {
     if (env->pipe_ready) return RISVEC_OK;
     CUDA_TRY(cudaStreamCreateWithFlags(&env->s_in, cudaStreamNonBlocking));
     CUDA_TRY(cudaStreamCreateWithFlags(&env->s_out, cudaStreamNonBlocking));
-    for (int i = 0; i < 2 * kMaxChunks + 2; ++i)
-        CUDA_TRY(cudaEventCreateWithFlags(&env->ev[i], cudaEventDisableTiming));
+    for (cudaEvent_t& e : env->ev) CUDA_TRY(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
     env->pipe_ready = 1;
     return RISVEC_OK;
 }
@@ -956,234 +975,149 @@ int chunk_steps(int T, size_t in_bytes_per_step) {
     return steps;
 }
 
-}  // namespace
+enum HostDir { kIn, kOnce, kOut };  // step-major input | step-independent input | step-major output
 
-int risvec_rollout_marl_host(risvec_env_t* env, int T, const float* action, const int32_t* partner,
-                             const int32_t* ngroups, const int32_t* arrivals, const risvec_marl_out_t* out,
-                             void* stream) {
-    if (!env) return fail(RISVEC_ERR_INVALID, "NULL handle");
-    if (T < 1 || !action || !partner || !ngroups) return fail(RISVEC_ERR_INVALID, "bad arguments");
-    ENTER_DEVICE(env->device);
+// One host array of a `_host` rollout.  A NULL `host` is an array the caller did not pass (an output it does not
+// want, arrivals drawn on the device): it gets no staging, and the launch sees a NULL device pointer.
+struct HostBuf {
+    HostDir dir;
+    const void* host;  // an output's is the caller's writable array
+    size_t bytes;      // per step; kOnce: in all
+    size_t total(int T) const { return dir == kOnce ? bytes : bytes * (size_t)T; }
+};
+
+cudaError_t join(cudaStream_t to, cudaStream_t from, cudaEvent_t ev) {  // `to` waits for all work queued on `from`
+    const cudaError_t e = cudaEventRecord(ev, from);
+    return e != cudaSuccess ? e : cudaStreamWaitEvent(to, ev, 0);
+}
+
+// The pipeline of every `_host` entry point.  The staging holds each array in `b` whole.  The kOnce inputs go first,
+// then the kIn inputs chunk by chunk, all on s_in; each chunk then runs `launch(tn, d)` on `stream`, where d[i] is
+// the device copy of b[i] at the chunk's first step, and its kOut outputs are copied back on s_out.
+// `chunk_bytes_per_step` sets the chunk length (chunk_steps).
+template <size_t N, typename Launch>
+int host_pipeline(risvec_env* env, int T, size_t chunk_bytes_per_step, const HostBuf (&b)[N], void* stream,
+                  Launch launch) {
     if (int rc = ensure_pipe(env)) return rc;
-    const size_t E = env->dims.E, V = env->dims.V, TE = (size_t)T * E;
-    const size_t n_act = TE * 2 * V, n_ev = TE * V;
-    size_t need = 256 * 16 + 4 * (n_act + E * V + E + n_ev) + 4 * (6 * n_ev + TE + TE * RISVEC_NSTAT + n_act);
+    size_t need = 0;
+    for (const HostBuf& x : b)
+        if (x.host) need += align_up(x.total(T), 256);
     if (int rc = ensure_stage(env, need)) return rc;
     Carver c{env->stage, 0};
-    cudaStream_t st = (cudaStream_t)stream, si = env->s_in, so = env->s_out;
-    float* d_act = c.take<float>(n_act);
-    int* d_part = c.take<int>(E * V);
-    int* d_ng = c.take<int>(E);
-    int* d_arr = arrivals ? c.take<int>(n_ev) : nullptr;
-    risvec_marl_out_t d_out;
-    memset(&d_out, 0, sizeof(d_out));
-    risvec_marl_out_t h = out ? *out : d_out;
-    if (h.reward_user) d_out.reward_user = c.take<float>(n_ev);
-    if (h.reward) d_out.reward = c.take<float>(TE);
-    if (h.DataBuf) d_out.DataBuf = c.take<float>(n_ev);
-    if (h.data_t) d_out.data_t = c.take<float>(n_ev);
-    if (h.data_p) d_out.data_p = c.take<float>(n_ev);
-    if (h.rate) d_out.rate = c.take<float>(n_ev);
-    if (h.over_power) d_out.over_power = c.take<float>(n_ev);
-    if (h.stats) d_out.stats = c.take<float>(TE * RISVEC_NSTAT);
-    if (h.last_power) d_out.last_power = c.take<float>(n_act);
+    char* dev[N];
+    for (size_t i = 0; i < N; ++i) dev[i] = b[i].host ? c.take<char>(b[i].total(T)) : nullptr;
 
+    cudaStream_t st = (cudaStream_t)stream, si = env->s_in, so = env->s_out;
     cudaEvent_t* ev_in = env->ev;
     cudaEvent_t* ev_k = env->ev + kMaxChunks;
     cudaEvent_t ev_start = env->ev[2 * kMaxChunks], ev_done = env->ev[2 * kMaxChunks + 1];
+    cudaEvent_t ev_in_done = env->ev[2 * kMaxChunks + 2];
     CUDA_TRY(cudaEventRecord(ev_start, st));  // staging may still be read by earlier work on `stream`
     CUDA_TRY(cudaStreamWaitEvent(si, ev_start, 0));
     CUDA_TRY(cudaStreamWaitEvent(so, ev_start, 0));
-    CUDA_TRY(cudaMemcpyAsync(d_part, partner, E * V * 4, cudaMemcpyHostToDevice, si));
-    CUDA_TRY(cudaMemcpyAsync(d_ng, ngroups, E * 4, cudaMemcpyHostToDevice, si));
-    const int Tc = chunk_steps(T, E * (2 * V + V) * 4);
-    int nchunk = 0;
-    for (int t0 = 0; t0 < T; t0 += Tc, ++nchunk) {
-        const size_t n = (size_t)((T - t0 < Tc) ? T - t0 : Tc) * E, o = (size_t)t0 * E;
-        CUDA_TRY(cudaMemcpyAsync(d_act + o * 2 * V, action + o * 2 * V, n * 2 * V * 4, cudaMemcpyHostToDevice, si));
-        if (arrivals) CUDA_TRY(cudaMemcpyAsync(d_arr + o * V, arrivals + o * V, n * V * 4, cudaMemcpyHostToDevice, si));
-        CUDA_TRY(cudaEventRecord(ev_in[nchunk], si));
-    }
-    int ci = 0;
-    for (int t0 = 0; t0 < T; t0 += Tc, ++ci) {
-        const int tn = (T - t0 < Tc) ? T - t0 : Tc;
-        const size_t n = (size_t)tn * E, o = (size_t)t0 * E;
-        CUDA_TRY(cudaStreamWaitEvent(st, ev_in[ci], 0));
-        risvec_marl_out_t oc;
-        memset(&oc, 0, sizeof(oc));
-#define OFF(member, per) oc.member = d_out.member ? d_out.member + o * (per) : nullptr
-        OFF(reward_user, V); OFF(reward, 1); OFF(DataBuf, V); OFF(data_t, V); OFF(data_p, V); OFF(rate, V);
-        OFF(over_power, V); OFF(stats, RISVEC_NSTAT); OFF(last_power, 2 * V);
-        double* const slots = env->stats_slots;
-        if (t0 + tn < T) env->stats_slots = nullptr;  // the statistics are those of the rollout's last step
-        const int rc = risvec_rollout_marl(env, tn, d_act + o * 2 * V, d_part, d_ng, d_arr ? d_arr + o * V : nullptr, &oc, stream);
-        env->stats_slots = slots;
-        if (rc) return rc;
-        CUDA_TRY(cudaEventRecord(ev_k[ci], st));
-        CUDA_TRY(cudaStreamWaitEvent(so, ev_k[ci], 0));
-#define D2H(member, per) \
-    if (h.member) CUDA_TRY(cudaMemcpyAsync(h.member + o * (per), oc.member, n * (per) * 4, cudaMemcpyDeviceToHost, so))
-        D2H(reward_user, V); D2H(reward, 1); D2H(DataBuf, V); D2H(data_t, V); D2H(data_p, V); D2H(rate, V);
-        D2H(over_power, V); D2H(stats, RISVEC_NSTAT); D2H(last_power, 2 * V);
-    }
-    CUDA_TRY(cudaEventRecord(ev_done, so));
-    CUDA_TRY(cudaStreamWaitEvent(st, ev_done, 0));  // the caller only has to synchronise `stream`
+    const int Tc = chunk_steps(T, chunk_bytes_per_step);
+    const int rc = [&]() -> int {
+        for (size_t i = 0; i < N; ++i)
+            if (b[i].dir == kOnce && b[i].host)
+                CUDA_TRY(cudaMemcpyAsync(dev[i], b[i].host, b[i].bytes, cudaMemcpyHostToDevice, si));
+        for (int t0 = 0, ci = 0; t0 < T; t0 += Tc, ++ci) {
+            const size_t tn = std::min(Tc, T - t0);
+            for (size_t i = 0; i < N; ++i)
+                if (b[i].dir == kIn && b[i].host)
+                    CUDA_TRY(cudaMemcpyAsync(dev[i] + t0 * b[i].bytes, (const char*)b[i].host + t0 * b[i].bytes,
+                                             tn * b[i].bytes, cudaMemcpyHostToDevice, si));
+            CUDA_TRY(cudaEventRecord(ev_in[ci], si));
+        }
+        for (int t0 = 0, ci = 0; t0 < T; t0 += Tc, ++ci) {
+            const int tn = std::min(Tc, T - t0);
+            void* d[N];
+            for (size_t i = 0; i < N; ++i) d[i] = dev[i] && b[i].dir != kOnce ? dev[i] + (size_t)t0 * b[i].bytes : dev[i];
+            CUDA_TRY(cudaStreamWaitEvent(st, ev_in[ci], 0));
+            double* const slots = env->stats_slots;
+            if (t0 + tn < T) env->stats_slots = nullptr;  // the statistics are those of the rollout's last step
+            const int rc = launch(tn, d);
+            env->stats_slots = slots;
+            if (rc) return rc;
+            CUDA_TRY(cudaEventRecord(ev_k[ci], st));
+            CUDA_TRY(cudaStreamWaitEvent(so, ev_k[ci], 0));
+            for (size_t i = 0; i < N; ++i)
+                if (b[i].dir == kOut && b[i].host)
+                    CUDA_TRY(cudaMemcpyAsync((char*)b[i].host + t0 * b[i].bytes, d[i], tn * b[i].bytes,
+                                             cudaMemcpyDeviceToHost, so));
+        }
+        return RISVEC_OK;
+    }();
+    // every exit, a failed chunk's too, joins both copy streams into `stream`: the caller only has to synchronise
+    // `stream`, and the next call cannot overwrite the staging under copies still queued here
+    const cudaError_t ji = join(st, si, ev_in_done), jo = join(st, so, ev_done);
+    if (rc != RISVEC_OK) return rc;
+    if (ji != cudaSuccess || jo != cudaSuccess)
+        return fail(RISVEC_ERR_CUDA, "joining the copy streams: %s", cudaGetErrorString(ji != cudaSuccess ? ji : jo));
     return RISVEC_OK;
 }
 
-int risvec_rollout_sarl_host(risvec_env_t* env, int T, const float* action, const float* phase,
-                             const int32_t* arrivals, const risvec_sarl_out_t* out, void* stream) {
-    if (!env) return fail(RISVEC_ERR_INVALID, "NULL handle");
-    if (T < 1 || !action || !phase) return fail(RISVEC_ERR_INVALID, "bad arguments");
-    ENTER_DEVICE(env->device);
-    if (int rc = ensure_pipe(env)) return rc;
-    const size_t E = env->dims.E, V = env->dims.V, M = env->dims.M, TE = (size_t)T * E;
-    const size_t n_act = TE * 2 * V, n_ev = TE * V, n_ph = TE * M;
-    size_t need = 256 * 16 + 4 * (n_act + n_ph + n_ev) + 4 * (6 * n_ev + TE);
-    if (int rc = ensure_stage(env, need)) return rc;
-    Carver c{env->stage, 0};
-    cudaStream_t st = (cudaStream_t)stream, si = env->s_in, so = env->s_out;
-    float* d_act = c.take<float>(n_act);
-    float* d_ph = c.take<float>(n_ph);
-    int* d_arr = arrivals ? c.take<int>(n_ev) : nullptr;
-    risvec_sarl_out_t d_out;
-    memset(&d_out, 0, sizeof(d_out));
-    risvec_sarl_out_t h = out ? *out : d_out;
-    if (h.reward) d_out.reward = c.take<float>(TE);
-    if (h.DataBuf) d_out.DataBuf = c.take<float>(n_ev);
-    if (h.data_t) d_out.data_t = c.take<float>(n_ev);
-    if (h.data_p) d_out.data_p = c.take<float>(n_ev);
-    if (h.over_power) d_out.over_power = c.take<float>(n_ev);
-    if (h.over_data) d_out.over_data = c.take<float>(n_ev);
-    if (h.rate) d_out.rate = c.take<float>(n_ev);
-
-    cudaEvent_t* ev_in = env->ev;
-    cudaEvent_t* ev_k = env->ev + kMaxChunks;
-    cudaEvent_t ev_start = env->ev[2 * kMaxChunks], ev_done = env->ev[2 * kMaxChunks + 1];
-    CUDA_TRY(cudaEventRecord(ev_start, st));
-    CUDA_TRY(cudaStreamWaitEvent(si, ev_start, 0));
-    CUDA_TRY(cudaStreamWaitEvent(so, ev_start, 0));
-    const int Tc = chunk_steps(T, E * (2 * V + V + M) * 4);
-    int nchunk = 0;
-    for (int t0 = 0; t0 < T; t0 += Tc, ++nchunk) {
-        const size_t n = (size_t)((T - t0 < Tc) ? T - t0 : Tc) * E, o = (size_t)t0 * E;
-        CUDA_TRY(cudaMemcpyAsync(d_act + o * 2 * V, action + o * 2 * V, n * 2 * V * 4, cudaMemcpyHostToDevice, si));
-        CUDA_TRY(cudaMemcpyAsync(d_ph + o * M, phase + o * M, n * M * 4, cudaMemcpyHostToDevice, si));
-        if (arrivals) CUDA_TRY(cudaMemcpyAsync(d_arr + o * V, arrivals + o * V, n * V * 4, cudaMemcpyHostToDevice, si));
-        CUDA_TRY(cudaEventRecord(ev_in[nchunk], si));
-    }
-    int ci = 0;
-    for (int t0 = 0; t0 < T; t0 += Tc, ++ci) {
-        const int tn = (T - t0 < Tc) ? T - t0 : Tc;
-        const size_t n = (size_t)tn * E, o = (size_t)t0 * E;
-        CUDA_TRY(cudaStreamWaitEvent(st, ev_in[ci], 0));
-        risvec_sarl_out_t oc;
-        memset(&oc, 0, sizeof(oc));
-        OFF(reward, 1); OFF(DataBuf, V); OFF(data_t, V); OFF(data_p, V); OFF(over_power, V); OFF(over_data, V);
-        OFF(rate, V);
-        double* const slots = env->stats_slots;
-        if (t0 + tn < T) env->stats_slots = nullptr;  // the statistics are those of the rollout's last step
-        const int rc = risvec_rollout_sarl(env, tn, d_act + o * 2 * V, d_ph + o * M, d_arr ? d_arr + o * V : nullptr, &oc, stream);
-        env->stats_slots = slots;
-        if (rc) return rc;
-        CUDA_TRY(cudaEventRecord(ev_k[ci], st));
-        CUDA_TRY(cudaStreamWaitEvent(so, ev_k[ci], 0));
-        D2H(reward, 1); D2H(DataBuf, V); D2H(data_t, V); D2H(data_p, V); D2H(over_power, V); D2H(over_data, V);
-        D2H(rate, V);
-    }
-#undef D2H
-#undef OFF
-    CUDA_TRY(cudaEventRecord(ev_done, so));
-    CUDA_TRY(cudaStreamWaitEvent(st, ev_done, 0));
-    return RISVEC_OK;
-}
-
-}  // extern "C"
-
-// packed host pipeline shared by both variants: records in, records + reward out
-namespace {
-template <typename Launch>
-int packed_host_pipeline(risvec_env* env, int T, size_t in_words, size_t out_words, const void* in_rec, float* out_rec,
-                         float* reward, size_t extra_dev_bytes, char** extra_dev, void* stream, Launch launch) {
-    if (int rc = ensure_pipe(env)) return rc;
-    const size_t E = env->dims.E, TE = (size_t)T * E;
-    const size_t need = 256 * 8 + 4 * TE * (in_words + out_words + 1) + extra_dev_bytes;
-    if (int rc = ensure_stage(env, need)) return rc;
-    Carver c{env->stage, 0};
-    float* d_in = c.take<float>(TE * in_words);
-    float* d_out = c.take<float>(TE * out_words);
-    float* d_rew = c.take<float>(TE);
-    *extra_dev = extra_dev_bytes ? (char*)c.take<char>(extra_dev_bytes) : nullptr;
-    cudaStream_t st = (cudaStream_t)stream, si = env->s_in, so = env->s_out;
-    cudaEvent_t* ev_in = env->ev;
-    cudaEvent_t* ev_k = env->ev + kMaxChunks;
-    cudaEvent_t ev_start = env->ev[2 * kMaxChunks], ev_done = env->ev[2 * kMaxChunks + 1];
-    CUDA_TRY(cudaEventRecord(ev_start, st));
-    CUDA_TRY(cudaStreamWaitEvent(si, ev_start, 0));
-    CUDA_TRY(cudaStreamWaitEvent(so, ev_start, 0));
-    const int Tc = chunk_steps(T, E * in_words * 4);
-    int n = 0;
-    for (int t0 = 0; t0 < T; t0 += Tc, ++n) {
-        const size_t cnt = (size_t)((T - t0 < Tc) ? T - t0 : Tc) * E * in_words, o = (size_t)t0 * E * in_words;
-        CUDA_TRY(cudaMemcpyAsync(d_in + o, (const float*)in_rec + o, cnt * 4, cudaMemcpyHostToDevice, si));
-        CUDA_TRY(cudaEventRecord(ev_in[n], si));
-    }
-    int ci = 0;
-    for (int t0 = 0; t0 < T; t0 += Tc, ++ci) {
-        const int tn = (T - t0 < Tc) ? T - t0 : Tc;
-        const size_t o = (size_t)t0 * E;
-        CUDA_TRY(cudaStreamWaitEvent(st, ev_in[ci], 0));
-        if (int rc = launch(tn, d_in + o * in_words, d_out + o * out_words, d_rew + o)) return rc;
-        CUDA_TRY(cudaEventRecord(ev_k[ci], st));
-        CUDA_TRY(cudaStreamWaitEvent(so, ev_k[ci], 0));
-        CUDA_TRY(cudaMemcpyAsync(out_rec + o * out_words, d_out + o * out_words, (size_t)tn * E * out_words * 4,
-                                 cudaMemcpyDeviceToHost, so));
-        CUDA_TRY(cudaMemcpyAsync(reward + o, d_rew + o, (size_t)tn * E * 4, cudaMemcpyDeviceToHost, so));
-    }
-    CUDA_TRY(cudaEventRecord(ev_done, so));
-    CUDA_TRY(cudaStreamWaitEvent(st, ev_done, 0));
-    return RISVEC_OK;
-}
 }  // namespace
 
 extern "C" {
 
+int risvec_rollout_marl_host(risvec_env_t* env, int T, const float* action, const int32_t* partner,
+                             const int32_t* ngroups, const int32_t* arrivals, const risvec_marl_out_t* out,
+                             void* stream) {
+    if (int rc = check_marl_args(env, T, action, partner, ngroups)) return rc;
+    ENTER_DEVICE(env->device);
+    const size_t E = env->dims.E, ev = E * env->dims.V * 4;  // ev: bytes of one step of an [T,E,V] array
+    const risvec_marl_out_t h = out ? *out : risvec_marl_out_t{};
+    const HostBuf b[] = {{kIn, action, 2 * ev}, {kIn, arrivals, ev}, {kOnce, partner, ev}, {kOnce, ngroups, E * 4},
+                         {kOut, h.reward_user, ev}, {kOut, h.reward, E * 4}, {kOut, h.DataBuf, ev}, {kOut, h.data_t, ev},
+                         {kOut, h.data_p, ev}, {kOut, h.rate, ev}, {kOut, h.over_power, ev},
+                         {kOut, h.stats, E * RISVEC_NSTAT * 4}, {kOut, h.last_power, 2 * ev}};
+    // the chunk length counts the arrivals whether or not they are passed
+    return host_pipeline(env, T, 3 * ev, b, stream, [&](int tn, void* const* d) {
+        const risvec_marl_out_t o = {(float*)d[4], (float*)d[5], (float*)d[6], (float*)d[7], (float*)d[8],
+                                     (float*)d[9], (float*)d[10], (float*)d[11], (float*)d[12]};
+        return risvec_rollout_marl(env, tn, (float*)d[0], (int32_t*)d[2], (int32_t*)d[3], (int32_t*)d[1], &o, stream);
+    });
+}
+
+int risvec_rollout_sarl_host(risvec_env_t* env, int T, const float* action, const float* phase,
+                             const int32_t* arrivals, const risvec_sarl_out_t* out, void* stream) {
+    if (int rc = check_sarl_args(env, T, action, phase)) return rc;
+    ENTER_DEVICE(env->device);
+    const size_t E = env->dims.E, ev = E * env->dims.V * 4, em = E * env->dims.M * 4;
+    const risvec_sarl_out_t h = out ? *out : risvec_sarl_out_t{};
+    const HostBuf b[] = {{kIn, action, 2 * ev}, {kIn, phase, em}, {kIn, arrivals, ev}, {kOut, h.reward, E * 4},
+                         {kOut, h.DataBuf, ev}, {kOut, h.data_t, ev}, {kOut, h.data_p, ev}, {kOut, h.over_power, ev},
+                         {kOut, h.over_data, ev}, {kOut, h.rate, ev}};
+    // the chunk length counts the arrivals whether or not they are passed
+    return host_pipeline(env, T, 3 * ev + em, b, stream, [&](int tn, void* const* d) {
+        const risvec_sarl_out_t o = {(float*)d[3], (float*)d[4], (float*)d[5], (float*)d[6],
+                                     (float*)d[7], (float*)d[8], (float*)d[9]};
+        return risvec_rollout_sarl(env, tn, (float*)d[0], (float*)d[1], (int32_t*)d[2], &o, stream);
+    });
+}
+
 int risvec_rollout_sarl_packed_host(risvec_env_t* env, int T, const void* in_rec, float* out_rec, float* reward,
                                     void* stream) {
-    if (!env) return fail(RISVEC_ERR_INVALID, "NULL handle");
-    if (T < 1 || !in_rec || !out_rec || !reward) return fail(RISVEC_ERR_INVALID, "bad arguments");
-    if (!packed_sarl_mpi(env))
-        return fail(RISVEC_ERR_UNSUPPORTED, "packed SARL records need V == 8, E %% 4 == 0 and M in {16, 40}");
+    if (int rc = check_sarl_packed_args(env, T, in_rec, out_rec, reward)) return rc;
     ENTER_DEVICE(env->device);
-    char* extra = nullptr;
-    return packed_host_pipeline(env, T, RISVEC_SARL_IN_WORDS(env->dims.M), RISVEC_SARL_OUT_WORDS, in_rec, out_rec, reward,
-                                0, &extra, stream, [&](int tn, const float* di, float* dout, float* dr) {
-                                    return risvec_rollout_sarl_packed(env, tn, di, dout, dr, stream);
-                                });
+    const size_t E = env->dims.E, in = E * RISVEC_SARL_IN_WORDS(env->dims.M) * 4;
+    const HostBuf b[] = {{kIn, in_rec, in}, {kOut, out_rec, E * RISVEC_SARL_OUT_WORDS * 4}, {kOut, reward, E * 4}};
+    return host_pipeline(env, T, in, b, stream, [&](int tn, void* const* d) {
+        return risvec_rollout_sarl_packed(env, tn, d[0], (float*)d[1], (float*)d[2], stream);
+    });
 }
 
 int risvec_rollout_marl_packed_host(risvec_env_t* env, int T, const void* in_rec, const int32_t* partner,
                                     const int32_t* ngroups, float* out_rec, float* reward, void* stream) {
-    if (!env) return fail(RISVEC_ERR_INVALID, "NULL handle");
-    if (T < 1 || !in_rec || !partner || !ngroups || !out_rec || !reward) return fail(RISVEC_ERR_INVALID, "bad arguments");
-    if (env->dims.V != 8 || env->dims.E % 4 != 0)
-        return fail(RISVEC_ERR_UNSUPPORTED, "packed MARL records need V == 8 and E %% 4 == 0");
+    if (int rc = check_marl_packed_args(env, T, in_rec, partner, ngroups, out_rec, reward)) return rc;
     ENTER_DEVICE(env->device);
-    if (int rc = ensure_pipe(env)) return rc;
-    const size_t E = env->dims.E;
-    char* extra = nullptr;
-    bool copied = false;
-    return packed_host_pipeline(env, T, RISVEC_MARL_IN_WORDS, RISVEC_MARL_OUT_WORDS, in_rec, out_rec, reward,
-                                (E * 8 + E) * 4 + 256, &extra, stream, [&](int tn, const float* di, float* dout, float* dr) {
-                                    int* d_part = (int*)extra;
-                                    int* d_ng = d_part + ((E * 8 + 63) / 64) * 64;
-                                    if (!copied) {  // small per-rollout tables, on the compute stream
-                                        cudaMemcpyAsync(d_part, partner, E * 8 * 4, cudaMemcpyHostToDevice, (cudaStream_t)stream);
-                                        cudaMemcpyAsync(d_ng, ngroups, E * 4, cudaMemcpyHostToDevice, (cudaStream_t)stream);
-                                        copied = true;
-                                    }
-                                    return risvec_rollout_marl_packed(env, tn, di, d_part, d_ng, dout, dr, stream);
-                                });
+    const size_t E = env->dims.E, in = E * RISVEC_MARL_IN_WORDS * 4;
+    const HostBuf b[] = {{kIn, in_rec, in}, {kOnce, partner, E * 8 * 4}, {kOnce, ngroups, E * 4},
+                         {kOut, out_rec, E * RISVEC_MARL_OUT_WORDS * 4}, {kOut, reward, E * 4}};
+    return host_pipeline(env, T, in, b, stream, [&](int tn, void* const* d) {
+        return risvec_rollout_marl_packed(env, tn, d[0], (int32_t*)d[1], (int32_t*)d[2], (float*)d[3], (float*)d[4],
+                                          stream);
+    });
 }
 
 int risvec_observe(risvec_env_t* env, float* obs, void* stream) {
