@@ -439,6 +439,25 @@ int risvec_shard_stats(risvec_env_t* env, double* out, int accumulate, void* str
 int risvec_attach_stats_accumulator(risvec_env_t* env, double* slots);
 int risvec_collect_stats(risvec_env_t* env, double* slots, double* out, int accumulate, void* stream);
 
+/* Per-episode statistics of staggered episodes: per-env running sums on the device and a log of completed episodes.
+ * n_user = V for MARL, 0 for SARL.  All memory is owned by the caller.
+ * running [E, RISVEC_EPLOG_RUN_COLS(n_user)] f64, zero-filled by the caller, one row per env:
+ *   col 0 = steps accumulated, cols 1..16 = sums of the RISVEC_F_STATS columns, col 17 = sum of RISVEC_F_REWARD,
+ *   cols 18.. = sums of RISVEC_F_REWARD_USER (MARL only).
+ * records [capacity, RISVEC_EPLOG_REC_COLS(n_user)] f64: col 0 = global env index (env_index_base + e),
+ *   col 1 = the env's RISVEC_F_STEP_CTR after the step, then the env's running row as it stood at its done step.
+ * count: one u64 (device) = records claimed since the caller last zeroed it.
+ * Call once after each driver step (T = 1).  For every env: the step's stats, reward and reward_user are converted to
+ * float64 and added to its running row, and col 0 gains 1.  If done[e] != 0 (done NULL: done_all != 0; done is the
+ * done_out of risvec_episode_tick for this step), the env claims slot k = count++, writes its record when
+ * k < capacity, and its running row is zeroed.  A record with k >= capacity is dropped but still counted, so
+ * count - capacity episodes were lost.  One launch, nothing decided on the host: the call can be captured in a CUDA
+ * graph.  Slots are claimed in no fixed order across warps; sort the records by (step, env). */
+#define RISVEC_EPLOG_RUN_COLS(n_user) (RISVEC_NSTAT + 2 + (n_user))
+#define RISVEC_EPLOG_REC_COLS(n_user) (RISVEC_NSTAT + 4 + (n_user))
+int risvec_episode_accumulate(risvec_env_t* env, double* running, const uint8_t* done, int done_all,
+                              double* records, int64_t capacity, unsigned long long* count, void* stream);
+
 /* Statistics reduction WITHOUT a collective (one node, NVLink / NVSwitch): one rank creates a small device buffer
  * and publishes its 64-byte CUDA IPC handle; every other rank (= process) maps it and passes the mapped pointer as
  * `out` of risvec_shard_stats(accumulate != 0).  k_shard_stats then adds the shard's sums into the owner's HBM with

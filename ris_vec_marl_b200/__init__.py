@@ -8,9 +8,10 @@ from ._lib import (EP_STAGES, PARTNER_NONE, PARTNER_SECOND, PARTNER_SINGLE, STAT
                    RisvecLibraryError, build_library, load_library)
 from .batched import (MARL_TRACES, SARL_TRACES, BatchedEnviron, default_pairing, default_params, encode_groups,
                       marl_yaml_overrides, mask_schedule)
+from .episode_log import EpisodeLog
 from .replay import ReplayBuffer
 
-__all__ = ["BatchedEnviron", "ReplayBuffer", "default_params", "default_pairing", "mask_schedule", "encode_groups",
-           "marl_yaml_overrides", "build_library",
+__all__ = ["BatchedEnviron", "EpisodeLog", "ReplayBuffer", "default_params", "default_pairing", "mask_schedule",
+           "encode_groups", "marl_yaml_overrides", "build_library",
            "load_library", "RisvecError", "RisvecLibraryError", "MARL_TRACES", "SARL_TRACES", "STAT_COLUMNS",
            "PARTNER_NONE", "PARTNER_SECOND", "PARTNER_SINGLE", "EP_STAGES"]

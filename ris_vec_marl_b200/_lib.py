@@ -35,6 +35,15 @@ def sarl_in_words(M):
     return 24 + M
 
 
+# episode log (risvec_episode_accumulate): width of the per-env running row and of a completed-episode record
+def eplog_run_cols(n_user):
+    return NSTAT + 2 + n_user
+
+
+def eplog_rec_cols(n_user):
+    return NSTAT + 4 + n_user
+
+
 STAT_COLUMNS = ("delay_mean", "energy_mean", "delay_local_mean", "delay_edge_q_mean", "delay_edge_c_mean",
                 "t_tx_mean", "backlog_kbit_mean", "mec_utilization", "local_util_mean", "qos_violation",
                 "off_kbit_sum", "local_kbit_sum", "mec_queue_cycles")
@@ -179,6 +188,8 @@ EXPORTS = {
     "risvec_shard_stats": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     "risvec_step_marl_fused": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "risvec_step_sarl_fused": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "risvec_episode_accumulate": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int64,
+                                            C.c_void_p, C.c_void_p]),
     "risvec_attach_stats_accumulator": (C.c_int, [C.c_void_p, C.c_void_p]),
     "risvec_collect_stats": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     "risvec_shared_buffer_create": (C.c_int, [C.c_int, C.c_uint64, C.POINTER(C.c_void_p), C.c_char_p]),

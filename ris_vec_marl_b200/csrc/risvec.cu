@@ -17,6 +17,7 @@
 #include "marl_tma.cuh"
 #include "pairing.cuh"
 #include "episode.cuh"
+#include "episode_log.cuh"
 #include "replay.cuh"
 
 using namespace risvec;
@@ -1619,6 +1620,21 @@ int risvec_shard_stats(risvec_env_t* env, double* out, int accumulate, void* str
     if (blocks > 148) blocks = 148;
     k_shard_stats<<<blocks, 1024, 0, (cudaStream_t)stream>>>(env->dims, env->st, out);
     return check_launch(env, "k_shard_stats");
+}
+
+int risvec_episode_accumulate(risvec_env_t* env, double* running, const uint8_t* done, int done_all,
+                              double* records, int64_t capacity, unsigned long long* count, void* stream) {
+    if (!env || !running || !records || !count) return fail(RISVEC_ERR_INVALID, "NULL argument");
+    if (capacity < 1) return fail(RISVEC_ERR_INVALID, "capacity must be >= 1 (got %lld)", (long long)capacity);
+    ENTER_DEVICE(env->device);
+    EpisodeLogArgs a;
+    a.running = running; a.done = done; a.done_all = done_all;
+    a.n_user = env->dims.variant == RISVEC_VARIANT_MARL ? env->dims.V : 0;
+    a.records = records; a.capacity = capacity; a.count = count;
+    const int per = episode_log_envs_per_block(a.n_user);
+    k_episode_accumulate<<<(env->dims.E + per - 1) / per, kEpLogThreads, 0, (cudaStream_t)stream>>>(env->dims, env->st,
+                                                                                                    a);
+    return check_launch(env, "k_episode_accumulate");
 }
 
 int risvec_attach_stats_accumulator(risvec_env_t* env, double* slots) {
