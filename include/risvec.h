@@ -422,6 +422,31 @@ int risvec_replay_store_marl(risvec_replay_t* rb, int E, const float* state, con
 int risvec_replay_sample(risvec_replay_t* rb, int B, const int64_t* idx, float* states, float* actions,
                          float* rewards_g, float* rewards_l, float* states_, uint8_t* dones, float* masks,
                          void* stream);
+/* Device-counter mode (opt-in): the ring counter lives on the device, in the handle's memory, and every store reads
+ * and advances it there, so stores and draws can be captured in a CUDA graph and each replay lands in fresh slots.
+ * risvec_replay_use_device_counter seeds the device counter from the host mem_cntr (a 1-thread launch on `stream`)
+ * and returns its address (*dev_count, one int64; writing it moves the ring, a negative value counts as 0).  Call it
+ * once, outside capture; a second call is refused.  From then on risvec_replay_store, risvec_replay_store_marl and
+ * risvec_replay_set_count return RISVEC_ERR_INVALID and risvec_replay_count returns -1, so the two counters can
+ * never silently diverge.  risvec_replay_sample (caller indices) keeps working: it does not read the counter. */
+int risvec_replay_use_device_counter(risvec_replay_t* rb, int64_t** dev_count, void* stream);
+/* risvec_replay_store / risvec_replay_store_marl with the count on the device: same arguments and checks, transition
+ * e goes to slot (count + e) % mem_size, then count += E, all in one launch with no host decision (the last block to
+ * finish advances the count).  RISVEC_ERR_INVALID on a handle not in device-counter mode. */
+int risvec_replay_store_devcnt(risvec_replay_t* rb, int E, const float* state, const float* action,
+                               const float* reward_g, const float* reward_l, const float* state_, const uint8_t* done,
+                               int done_all, const float* mask_flat, void* stream);
+int risvec_replay_store_marl_devcnt(risvec_replay_t* rb, int E, const float* state, const float* intent_probs,
+                                    const float* power_raw, const float* reward_g, const float* reward_l,
+                                    const float* state_, const uint8_t* done, int done_all, const uint8_t* mask_u8,
+                                    void* stream);
+/* sample_buffer with the count on the device: draws [B] i64 (device, uniform over [0, 2^62) for a uniform draw, read
+ * as unsigned); row b is slot draws[b] % min(count, mem_size), so the modulo bias is below mem_size / 2^62.  With
+ * count == 0 every row is slot 0 (all zeros until the first store), where buffer.py's np.random.choice(0, B) raises.
+ * The randomness is the caller's: the library draws nothing.  Outputs as risvec_replay_sample. */
+int risvec_replay_sample_devcnt(risvec_replay_t* rb, int B, const int64_t* draws, float* states, float* actions,
+                                float* rewards_g, float* rewards_l, float* states_, uint8_t* dones, float* masks,
+                                void* stream);
 
 /* Episode statistics for the multi-GPU reduction: sums over this shard's E envs of the
  * RISVEC_F_STATS columns and of RISVEC_F_REWARD, written (accumulate = 0) or added (accumulate != 0)

@@ -185,6 +185,12 @@ EXPORTS = {
     "risvec_replay_store": (C.c_int, [C.c_void_p, C.c_int] + [C.c_void_p] * 6 + [C.c_int, C.c_void_p, C.c_void_p]),
     "risvec_replay_store_marl": (C.c_int, [C.c_void_p, C.c_int] + [C.c_void_p] * 7 + [C.c_int, C.c_void_p, C.c_void_p]),
     "risvec_replay_sample": (C.c_int, [C.c_void_p, C.c_int] + [C.c_void_p] * 8 + [C.c_void_p]),
+    "risvec_replay_use_device_counter": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p), C.c_void_p]),
+    "risvec_replay_store_devcnt": (C.c_int, [C.c_void_p, C.c_int] + [C.c_void_p] * 6 + [C.c_int, C.c_void_p,
+                                                                                         C.c_void_p]),
+    "risvec_replay_store_marl_devcnt": (C.c_int, [C.c_void_p, C.c_int] + [C.c_void_p] * 7 + [C.c_int, C.c_void_p,
+                                                                                              C.c_void_p]),
+    "risvec_replay_sample_devcnt": (C.c_int, [C.c_void_p, C.c_int] + [C.c_void_p] * 8 + [C.c_void_p]),
     "risvec_shard_stats": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     "risvec_step_marl_fused": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "risvec_step_sarl_fused": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),

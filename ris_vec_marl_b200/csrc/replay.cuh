@@ -24,6 +24,33 @@ struct ReplaySrc {
     int done_all;
 };
 
+// Ring counter of a handle in device-counter mode (risvec_replay_use_device_counter): `count` is mem_cntr, `ticket`
+// counts the blocks of the running store that are done reading it.  Both live in the replay arena.
+struct ReplayCtr {
+    long long* count;
+    unsigned* ticket;
+};
+
+// DEVCNT stores: thread 0 of each block reads the count, then takes a ticket (__threadfence, then atomicAdd) before
+// the block writes anything.  The block that draws the last ticket knows every block of the launch has read the count,
+// so it advances the count by E and resets the ticket for the next store.  One launch, nothing for the host to reset
+// between replays.  Claiming at the start keeps the fence away from the block's stores: a fence after them would wait
+// for them to drain and hold the block's slot on the SM.
+__device__ __forceinline__ long long devcnt_claim(const ReplayCtr& c, int E) {
+    __shared__ long long s_count;
+    if (threadIdx.x == 0) {
+        const long long count = max(*(volatile long long*)c.count, 0LL);   // a negative count is taken as 0
+        s_count = count;
+        __threadfence();
+        if (atomicAdd(c.ticket, 1u) == gridDim.x * gridDim.y - 1) {
+            *(volatile long long*)c.count = count + E;
+            *(volatile unsigned*)c.ticket = 0;
+        }
+    }
+    __syncthreads();
+    return s_count;
+}
+
 template <int VEC>
 struct RVec;
 template <>
@@ -34,9 +61,11 @@ struct RVec<4> { using T = float4; };
 // Flat copy: the E rows of a call land in consecutive ring slots, so every field is one (at most
 // once wrapped) contiguous destination range.  A thread moves VEC consecutive floats of one field
 // of one row; VEC = 4 needs every row width to be a multiple of 4 (true at V = 8: 40, 80, 8, 64).
-template <int VEC, int MARL>
-__global__ void k_replay_store(ReplayMem m, long long first, int E, ReplaySrc src) {
+// DEVCNT = 1: `first` is ignored, the block reads it from `ctr` (see devcnt_claim).
+template <int VEC, int MARL, int DEVCNT>
+__global__ void k_replay_store(ReplayMem m, long long first, int E, ReplaySrc src, ReplayCtr ctr) {
     using V4 = typename RVec<VEC>::T;
+    if constexpr (DEVCNT) first = devcnt_claim(ctr, E);
     const int N = m.N, NN = N * N, AW = N + 2;
     const long long uS = (long long)E * (m.S / VEC), uA = (long long)E * (m.A / VEC), uN = (long long)E * (N / VEC),
                     uM = (long long)E * (NN / VEC);
@@ -113,9 +142,15 @@ __global__ void k_replay_store(ReplayMem m, long long first, int E, ReplaySrc sr
 // float4 form of the same store without per-element row arithmetic: blockIdx.y selects the field; because
 // the E rows land in consecutive ring slots, every field is a FLAT copy of E * width floats whose
 // destination is contiguous up to one wrap of the ring (n_wrap = rows before the wrap).  Only the assembled
-// MARL action rows need a row index (one 32-bit division per 16 bytes).
-template <int MARL>
-__global__ void __launch_bounds__(256) k_replay_store_flat(ReplayMem m, long long slot0, int n_wrap, int E, ReplaySrc src) {
+// MARL action rows need a row index (one 32-bit division per 16 bytes).  DEVCNT = 1: `slot0` / `n_wrap` are ignored,
+// the block computes them from the count it reads from `ctr`.
+template <int MARL, int DEVCNT>
+__global__ void __launch_bounds__(256) k_replay_store_flat(ReplayMem m, long long slot0, int n_wrap, int E, ReplaySrc src,
+                                                           ReplayCtr ctr) {
+    if constexpr (DEVCNT) {
+        slot0 = devcnt_claim(ctr, E) % m.mem_size;
+        n_wrap = (int)(m.mem_size - slot0 < E ? m.mem_size - slot0 : E);
+    }
     const int N = m.N, NN = N * N, AW = N + 2;
     const unsigned tid = blockIdx.x * blockDim.x + threadIdx.x, nthr = gridDim.x * blockDim.x;
     auto flat_copy = [&](float* dst_field, const float* src_field, int W) {  // W floats per row, W % 4 == 0
@@ -180,14 +215,23 @@ __global__ void __launch_bounds__(256) k_replay_store_flat(ReplayMem m, long lon
     }
 }
 
-// sample_buffer (buffer.py:27-39) for caller-drawn indices: one block per sampled row
+// sample_buffer (buffer.py:27-39) for caller-drawn indices: one block per sampled row.  DEVCNT = 1: `idx` holds
+// draws, row b is slot draws[b] % min(count, mem_size) (slot 0 while count == 0), read as unsigned: never outside.
+template <int DEVCNT>
 __global__ void k_replay_sample(ReplayMem m, int B, const long long* __restrict__ idx, float* __restrict__ states,
                                 float* __restrict__ actions, float* __restrict__ rewards_g,
                                 float* __restrict__ rewards_l, float* __restrict__ states_,
-                                unsigned char* __restrict__ dones, float* __restrict__ masks) {
+                                unsigned char* __restrict__ dones, float* __restrict__ masks,
+                                const long long* __restrict__ count) {
     const int b = blockIdx.x;
     if (b >= B) return;
-    const long long slot = min(max(idx[b], 0LL), m.mem_size - 1);   // out-of-range indices are clamped, never read outside
+    long long slot;
+    if constexpr (DEVCNT) {
+        const unsigned long long n = (unsigned long long)min(max(*count, 0LL), m.mem_size);
+        slot = n ? (long long)((unsigned long long)idx[b] % n) : 0;
+    } else {
+        slot = min(max(idx[b], 0LL), m.mem_size - 1);   // out-of-range indices are clamped, never read outside
+    }
     const int NN = m.N * m.N;
     for (int c = threadIdx.x; c < m.S; c += blockDim.x) {
         states[(size_t)b * m.S + c] = m.state[slot * m.S + c];

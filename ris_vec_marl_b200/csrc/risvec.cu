@@ -106,7 +106,9 @@ struct risvec_env {
 struct risvec_replay {
     ReplayMem m;
     int device;
-    long long mem_cntr;
+    long long mem_cntr;      // host-counter mode
+    int devcnt;              // device-counter mode (risvec_replay_use_device_counter): the count is *ctr.count
+    ReplayCtr ctr;           // in the arena's tail, zero at creation
     char* base;
     size_t off[RISVEC_RB_COUNT + 1];
     int64_t launches;
@@ -1481,7 +1483,8 @@ int risvec_replay_create(int device, int64_t mem_size, int input_shape, int n_ac
                                         (size_t)mem_size * m.N * m.N * 4};
     size_t off = 0;
     for (int i = 0; i < RISVEC_RB_COUNT; ++i) { rb->off[i] = off; off = align_up(off + sz[i], 256); }
-    rb->off[RISVEC_RB_COUNT] = off;
+    rb->off[RISVEC_RB_COUNT] = off;   // tail: the device counter (int64) and its ticket (uint32)
+    off += sizeof(long long) + sizeof(unsigned);
     cudaError_t ce = cudaMalloc((void**)&rb->base, off);
     if (ce == cudaSuccess) ce = cudaMemset(rb->base, 0, off);
     if (ce != cudaSuccess) {
@@ -1495,6 +1498,8 @@ int risvec_replay_create(int device, int64_t mem_size, int input_shape, int n_ac
     m.state_ = (float*)(rb->base + rb->off[RISVEC_RB_NEW_STATE]);
     m.terminal = (unsigned char*)(rb->base + rb->off[RISVEC_RB_TERMINAL]);
     m.mask = (float*)(rb->base + rb->off[RISVEC_RB_MASK]);
+    rb->ctr.count = (long long*)(rb->base + rb->off[RISVEC_RB_COUNT]);
+    rb->ctr.ticket = (unsigned*)(rb->ctr.count + 1);
     *out = rb;
     return RISVEC_OK;
 }
@@ -1519,14 +1524,44 @@ int risvec_replay_field(risvec_replay_t* rb, int field, void** dev_ptr, int64_t*
     return RISVEC_OK;
 }
 
-int64_t risvec_replay_count(const risvec_replay_t* rb) { return rb ? rb->mem_cntr : 0; }
+int64_t risvec_replay_count(const risvec_replay_t* rb) { return rb ? (rb->devcnt ? -1 : rb->mem_cntr) : 0; }
+
+static const char kDevcntMsg[] =
+    "the handle counts on the device: use risvec_replay_store_devcnt / risvec_replay_store_marl_devcnt / "
+    "risvec_replay_sample_devcnt, and the counter pointer of risvec_replay_use_device_counter for the count";
+
 int risvec_replay_set_count(risvec_replay_t* rb, int64_t mem_cntr) {
     if (!rb || mem_cntr < 0) return fail(RISVEC_ERR_INVALID, "NULL handle or negative count");
+    if (rb->devcnt) return fail(RISVEC_ERR_INVALID, "%s", kDevcntMsg);
     rb->mem_cntr = mem_cntr;
     return RISVEC_OK;
 }
 
-static int replay_store(risvec_replay* rb, int E, const ReplaySrc& src, int marl, cudaStream_t st) {
+}  // extern "C"
+namespace risvec {
+__global__ void k_replay_seed_counter(ReplayCtr c, long long count) {
+    *c.count = count;
+    *c.ticket = 0;
+}
+}  // namespace risvec
+extern "C" {
+
+int risvec_replay_use_device_counter(risvec_replay_t* rb, int64_t** dev_count, void* stream) {
+    if (!rb || !dev_count) return fail(RISVEC_ERR_INVALID, "NULL argument");
+    if (rb->devcnt) return fail(RISVEC_ERR_INVALID, "the handle already counts on the device");
+    ENTER_DEVICE(rb->device);
+    k_replay_seed_counter<<<1, 1, 0, (cudaStream_t)stream>>>(rb->ctr, rb->mem_cntr);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return fail(RISVEC_ERR_CUDA, "launch of k_replay_seed_counter failed: %s", cudaGetErrorString(e));
+    rb->launches += 1;
+    rb->devcnt = 1;
+    *dev_count = (int64_t*)rb->ctr.count;
+    return RISVEC_OK;
+}
+
+// The path choice (flat float4, vec4 or scalar) depends on shapes and pointers only, never on the count, so a
+// device-counter store takes the same path as a host-counter store of the same arguments.
+static int replay_store(risvec_replay* rb, int E, const ReplaySrc& src, int marl, int devcnt, cudaStream_t st) {
     const ReplayMem& m = rb->m;
     auto al16 = [](const void* q) { return ((uintptr_t)q & 15) == 0; };   // float4 path needs aligned sources
     const bool vec4 = m.S % 4 == 0 && m.A % 4 == 0 && m.N % 4 == 0 && al16(src.state) && al16(src.state_) &&
@@ -1538,46 +1573,62 @@ static int replay_store(risvec_replay* rb, int E, const ReplaySrc& src, int marl
     if (blocks > 148 * 64) blocks = 148 * 64;   // grid-stride beyond 64 blocks per SM
     const bool mask_ok = marl ? (src.mask_u8 == nullptr || (((uintptr_t)src.mask_u8) & 3) == 0)
                               : (src.mask_f == nullptr || al16(src.mask_f));
+    const ReplayCtr ctr = devcnt ? rb->ctr : ReplayCtr{};
+    const long long first = devcnt ? 0 : rb->mem_cntr;
     if (vec4 && mask_ok && (long long)E * (m.A > m.N * m.N ? m.A : m.N * m.N) < (1ll << 31)) {
         // flat float4 copies, one grid row per field (no per-element row arithmetic)
-        const long long slot0 = rb->mem_cntr % m.mem_size;
+        const long long slot0 = first % m.mem_size;
         const int n_wrap = (int)((m.mem_size - slot0) < E ? (m.mem_size - slot0) : E);
         const long long big = (long long)E * ((m.A > m.S ? m.A : m.S) / 4);
         long long bx = (big + threads - 1) / threads;
         if (bx > 148 * 8) bx = 148 * 8;
-        if (marl) k_replay_store_flat<1><<<dim3((unsigned)bx, 6), threads, 0, st>>>(m, slot0, n_wrap, E, src);
-        else k_replay_store_flat<0><<<dim3((unsigned)bx, 6), threads, 0, st>>>(m, slot0, n_wrap, E, src);
-    } else if (vec4 && marl) k_replay_store<4, 1><<<(int)blocks, threads, 0, st>>>(m, rb->mem_cntr, E, src);
-    else if (vec4) k_replay_store<4, 0><<<(int)blocks, threads, 0, st>>>(m, rb->mem_cntr, E, src);
-    else if (marl) k_replay_store<1, 1><<<(int)blocks, threads, 0, st>>>(m, rb->mem_cntr, E, src);
-    else k_replay_store<1, 0><<<(int)blocks, threads, 0, st>>>(m, rb->mem_cntr, E, src);
+        const dim3 grid((unsigned)bx, 6);
+        if (marl && devcnt) k_replay_store_flat<1, 1><<<grid, threads, 0, st>>>(m, slot0, n_wrap, E, src, ctr);
+        else if (marl) k_replay_store_flat<1, 0><<<grid, threads, 0, st>>>(m, slot0, n_wrap, E, src, ctr);
+        else if (devcnt) k_replay_store_flat<0, 1><<<grid, threads, 0, st>>>(m, slot0, n_wrap, E, src, ctr);
+        else k_replay_store_flat<0, 0><<<grid, threads, 0, st>>>(m, slot0, n_wrap, E, src, ctr);
+    } else {
+        using K = void (*)(ReplayMem, long long, int, ReplaySrc, ReplayCtr);
+        static const K ks[2][2][2] = {{{k_replay_store<1, 0, 0>, k_replay_store<1, 0, 1>},
+                                       {k_replay_store<1, 1, 0>, k_replay_store<1, 1, 1>}},
+                                      {{k_replay_store<4, 0, 0>, k_replay_store<4, 0, 1>},
+                                       {k_replay_store<4, 1, 0>, k_replay_store<4, 1, 1>}}};
+        ks[vec4][marl != 0][devcnt != 0]<<<(int)blocks, threads, 0, st>>>(m, first, E, src, ctr);
+    }
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return fail(RISVEC_ERR_CUDA, "launch of k_replay_store failed: %s", cudaGetErrorString(e));
     rb->launches += 1;
-    rb->mem_cntr += E;
+    if (!devcnt) rb->mem_cntr += E;
     return RISVEC_OK;
 }
 
-int risvec_replay_store(risvec_replay_t* rb, int E, const float* state, const float* action, const float* reward_g,
-                        const float* reward_l, const float* state_, const uint8_t* done, int done_all,
-                        const float* mask_flat, void* stream) {
-    if (!rb || !state || !action || !reward_g || !reward_l || !state_) return fail(RISVEC_ERR_INVALID, "NULL argument");
+static int store_checks(risvec_replay* rb, int E, int devcnt) {
     if (E < 1 || E > rb->m.mem_size) return fail(RISVEC_ERR_INVALID, "E = %d must be in [1, mem_size]", E);
+    if (rb->devcnt && !devcnt) return fail(RISVEC_ERR_INVALID, "%s", kDevcntMsg);
+    if (!rb->devcnt && devcnt)
+        return fail(RISVEC_ERR_INVALID, "the handle counts on the host: call risvec_replay_use_device_counter first");
+    return RISVEC_OK;
+}
+
+static int store_flat(risvec_replay_t* rb, int E, const float* state, const float* action, const float* reward_g,
+                      const float* reward_l, const float* state_, const uint8_t* done, int done_all,
+                      const float* mask_flat, void* stream, int devcnt) {
+    if (!rb || !state || !action || !reward_g || !reward_l || !state_) return fail(RISVEC_ERR_INVALID, "NULL argument");
+    if (int rc = store_checks(rb, E, devcnt)) return rc;
     ENTER_DEVICE(rb->device);
     ReplaySrc src;
     memset(&src, 0, sizeof(src));
     src.state = state; src.state_ = state_; src.action = action; src.reward_g = reward_g; src.reward_l = reward_l;
     src.mask_f = mask_flat; src.done = done; src.done_all = done_all;
-    return replay_store(rb, E, src, 0, (cudaStream_t)stream);
+    return replay_store(rb, E, src, 0, devcnt, (cudaStream_t)stream);
 }
 
-int risvec_replay_store_marl(risvec_replay_t* rb, int E, const float* state, const float* intent_probs,
-                             const float* power_raw, const float* reward_g, const float* reward_l,
-                             const float* state_, const uint8_t* done, int done_all, const uint8_t* mask_u8,
-                             void* stream) {
+static int store_marl(risvec_replay_t* rb, int E, const float* state, const float* intent_probs,
+                      const float* power_raw, const float* reward_g, const float* reward_l, const float* state_,
+                      const uint8_t* done, int done_all, const uint8_t* mask_u8, void* stream, int devcnt) {
     if (!rb || !state || !intent_probs || !power_raw || !reward_g || !reward_l || !state_)
         return fail(RISVEC_ERR_INVALID, "NULL argument");
-    if (E < 1 || E > rb->m.mem_size) return fail(RISVEC_ERR_INVALID, "E = %d must be in [1, mem_size]", E);
+    if (int rc = store_checks(rb, E, devcnt)) return rc;
     if (rb->m.A != rb->m.N * (rb->m.N + 2))
         return fail(RISVEC_ERR_INVALID, "store_marl needs n_actions = n_agents + 2 (got %d per agent)", rb->m.A / rb->m.N);
     ENTER_DEVICE(rb->device);
@@ -1585,22 +1636,69 @@ int risvec_replay_store_marl(risvec_replay_t* rb, int E, const float* state, con
     memset(&src, 0, sizeof(src));
     src.state = state; src.state_ = state_; src.probs = intent_probs; src.power = power_raw; src.reward_g = reward_g;
     src.reward_l = reward_l; src.mask_u8 = mask_u8; src.done = done; src.done_all = done_all;
-    return replay_store(rb, E, src, 1, (cudaStream_t)stream);
+    return replay_store(rb, E, src, 1, devcnt, (cudaStream_t)stream);
+}
+
+int risvec_replay_store(risvec_replay_t* rb, int E, const float* state, const float* action, const float* reward_g,
+                        const float* reward_l, const float* state_, const uint8_t* done, int done_all,
+                        const float* mask_flat, void* stream) {
+    return store_flat(rb, E, state, action, reward_g, reward_l, state_, done, done_all, mask_flat, stream, 0);
+}
+
+int risvec_replay_store_devcnt(risvec_replay_t* rb, int E, const float* state, const float* action,
+                               const float* reward_g, const float* reward_l, const float* state_, const uint8_t* done,
+                               int done_all, const float* mask_flat, void* stream) {
+    return store_flat(rb, E, state, action, reward_g, reward_l, state_, done, done_all, mask_flat, stream, 1);
+}
+
+int risvec_replay_store_marl(risvec_replay_t* rb, int E, const float* state, const float* intent_probs,
+                             const float* power_raw, const float* reward_g, const float* reward_l,
+                             const float* state_, const uint8_t* done, int done_all, const uint8_t* mask_u8,
+                             void* stream) {
+    return store_marl(rb, E, state, intent_probs, power_raw, reward_g, reward_l, state_, done, done_all, mask_u8,
+                      stream, 0);
+}
+
+int risvec_replay_store_marl_devcnt(risvec_replay_t* rb, int E, const float* state, const float* intent_probs,
+                                    const float* power_raw, const float* reward_g, const float* reward_l,
+                                    const float* state_, const uint8_t* done, int done_all, const uint8_t* mask_u8,
+                                    void* stream) {
+    return store_marl(rb, E, state, intent_probs, power_raw, reward_g, reward_l, state_, done, done_all, mask_u8,
+                      stream, 1);
+}
+
+static int replay_sample(risvec_replay_t* rb, int B, const int64_t* idx, float* states, float* actions,
+                         float* rewards_g, float* rewards_l, float* states_, uint8_t* dones, float* masks,
+                         void* stream, int devcnt) {
+    if (!rb || !idx || !states || !actions || !rewards_g || !rewards_l || !states_ || !dones || !masks)
+        return fail(RISVEC_ERR_INVALID, "NULL argument");
+    if (B < 1) return fail(RISVEC_ERR_INVALID, "B must be >= 1");
+    if (devcnt && !rb->devcnt)
+        return fail(RISVEC_ERR_INVALID, "the handle counts on the host: call risvec_replay_use_device_counter first");
+    ENTER_DEVICE(rb->device);
+    if (devcnt)
+        k_replay_sample<1><<<B, 128, 0, (cudaStream_t)stream>>>(rb->m, B, (const long long*)idx, states, actions,
+                                                               rewards_g, rewards_l, states_, dones, masks,
+                                                               rb->ctr.count);
+    else
+        k_replay_sample<0><<<B, 128, 0, (cudaStream_t)stream>>>(rb->m, B, (const long long*)idx, states, actions,
+                                                               rewards_g, rewards_l, states_, dones, masks, nullptr);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return fail(RISVEC_ERR_CUDA, "launch of k_replay_sample failed: %s", cudaGetErrorString(e));
+    rb->launches += 1;
+    return RISVEC_OK;
 }
 
 int risvec_replay_sample(risvec_replay_t* rb, int B, const int64_t* idx, float* states, float* actions,
                          float* rewards_g, float* rewards_l, float* states_, uint8_t* dones, float* masks,
                          void* stream) {
-    if (!rb || !idx || !states || !actions || !rewards_g || !rewards_l || !states_ || !dones || !masks)
-        return fail(RISVEC_ERR_INVALID, "NULL argument");
-    if (B < 1) return fail(RISVEC_ERR_INVALID, "B must be >= 1");
-    ENTER_DEVICE(rb->device);
-    k_replay_sample<<<B, 128, 0, (cudaStream_t)stream>>>(rb->m, B, (const long long*)idx, states, actions, rewards_g,
-                                                        rewards_l, states_, dones, masks);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return fail(RISVEC_ERR_CUDA, "launch of k_replay_sample failed: %s", cudaGetErrorString(e));
-    rb->launches += 1;
-    return RISVEC_OK;
+    return replay_sample(rb, B, idx, states, actions, rewards_g, rewards_l, states_, dones, masks, stream, 0);
+}
+
+int risvec_replay_sample_devcnt(risvec_replay_t* rb, int B, const int64_t* draws, float* states, float* actions,
+                                float* rewards_g, float* rewards_l, float* states_, uint8_t* dones, float* masks,
+                                void* stream) {
+    return replay_sample(rb, B, draws, states, actions, rewards_g, rewards_l, states_, dones, masks, stream, 1);
 }
 
 }  // extern "C"

@@ -6,10 +6,11 @@
     pair_reset), alternated in the same run: all envs and 1 % of the envs (the separate chain has no per-env form, so
     it always runs on all envs), at E = 4096, V = 8, M = 40 with the config.yaml parameters; and the config-4 shape
     (E = 1024, V = 32, M = 256), where begin_episode takes the per-stage fallback.
-(b) The `--driver` loop of bench_actor_loop.py in three forms: lock-step episodes as there (host branch on the step
+(b) The `--driver` loop of bench_actor_loop.py in four forms: lock-step episodes as there (host branch on the step
     counter); staggered episodes (episode_tick + pair_noma_episodes + fused step + replay store with the per-env done
-    flags); and the staggered loop with the env part (tick, actors, pairing, intent head, step) replayed as a CUDA
-    graph.  The replay store keeps its slot counter on the host, so it stays an eager launch after each replay.
+    flags); the staggered loop with the env part (tick, actors, pairing, intent head, step) replayed as a CUDA graph
+    and the store of a host-counter replay buffer issued eagerly after each replay (`staggered_graph`); and the whole
+    staggered step, store included, as one graph on a device-counter replay buffer (`staggered_graph_full`).
 
 Writes one JSON object (stdout and --out)."""
 import argparse
@@ -100,6 +101,7 @@ def part_b(E, steps, rounds):
     env.begin_episode(stages=("reset",) + DRIVER)
     actors = Actors(V, dev)
     rb = ReplayBuffer(min(1_000_000, max(4 * E, 65536)), 5, V + 2, V, device=0)
+    rb_dev = ReplayBuffer(min(1_000_000, max(4 * E, 65536)), 5, V + 2, V, device=0, device_counter=True)
     obs, obs2 = torch.empty(E, V, 5, device=dev), torch.empty(E, V, 5, device=dev)
     bufs = [obs, obs2]
     env.observe(out=obs)
@@ -138,8 +140,12 @@ def part_b(E, steps, rounds):
 
     # staggered start: envs e start their episodes at offsets e % 100
     env.ep_step.copy_(torch.arange(E, dtype=torch.int32, device=dev) % 100)
-    # two graphs, one per observation-buffer parity: replay, then the eager store
-    graphs = []
+    def full_step(cur, nxt):  # the whole staggered step, store on the device-counter buffer included
+        raw, probs, done = env_part(cur, nxt)
+        rb_dev.store_marl(cur, probs, raw, env.reward, env.reward_user, nxt, done=done, mask_u8=env.pair_mask)
+
+    # two graphs per form, one per observation-buffer parity: env part (then the eager store), and the full step
+    graphs, full_graphs = [], []
     s = torch.cuda.Stream()
     s.wait_stream(torch.cuda.current_stream())
     with torch.cuda.stream(s):
@@ -152,6 +158,11 @@ def part_b(E, steps, rounds):
             with torch.cuda.graph(g, stream=s):
                 outs = env_part(cur, nxt)
             graphs.append((g, cur, nxt, outs))
+        for cur, nxt in ((obs, obs2), (obs2, obs)):
+            g = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(g, stream=s):
+                full_step(cur, nxt)
+            full_graphs.append(g)
     torch.cuda.current_stream().wait_stream(s)
     gi = [0]
 
@@ -161,23 +172,31 @@ def part_b(E, steps, rounds):
         g.replay()
         rb.store_marl(cur, probs, raw, env.reward, env.reward_user, nxt, done=done, mask_u8=env.pair_mask)
 
+    fi = [0]
+
+    def staggered_graph_full():
+        full_graphs[fi[0]].replay()
+        fi[0] ^= 1
+
     def loop(fn):
         return lambda: [fn() for _ in range(steps)]
 
     # the graph form always starts from buffer parity 0; keep the eager forms on an even number of steps too
     assert steps % 2 == 0
-    res = ab({"lockstep": loop(lockstep), "staggered": loop(staggered), "staggered_graph": loop(staggered_graph)}, 1,
-             rounds)
-    for k in ("lockstep", "staggered", "staggered_graph"):
+    arms = {"lockstep": loop(lockstep), "staggered": loop(staggered), "staggered_graph": loop(staggered_graph),
+            "staggered_graph_full": loop(staggered_graph_full)}
+    res = ab(arms, 1, rounds)
+    for k in arms:
         r = res[k]
         r["us_per_step"] = r["median_us"] / steps
         r["env_steps_per_s"] = E * steps / (r["median_us"] * 1e-6)
     res["config"] = {"envs": E, "V": V, "M": M, "steps_per_timing": steps, "rounds": rounds,
                      "actor": "8 x MLP 5-512-256-{2, V} (bmm), fp32",
                      "graph_part": "episode_tick, actors, map_actions, pair_noma_episodes, intent head, step_marl_fused",
-                     "eager_after_each_replay": "replay store: its slot counter mem_cntr lives on the host, so the store "
-                                               "is not graph-safe (out of scope here)"}
+                     "staggered_graph": "graph_part as a graph, then the store of a host-counter buffer, eager",
+                     "staggered_graph_full": "graph_part and the store of a device-counter buffer, one graph"}
     res["replay_rows"] = int(rb.mem_cntr)
+    res["replay_rows_device_counter"] = int(rb_dev.mem_cntr)
     env.close()
     return res
 

@@ -1,6 +1,8 @@
 #!/usr/bin/env python
 """Replay-memory write path (SURVEY.md 8f row 4): fused `store_marl` of E transitions per call, CUDA-event timed,
-against the achieved-bytes roofline (pure copy: reads + writes of one 936 B row per env at V = 8)."""
+against the achieved-bytes roofline (pure copy: reads + writes of one 936 B row per env at V = 8).  Also the same
+store on a device-counter buffer (`device_counter=True`), eager and as a graph of 20 stores: there every captured
+store lands in fresh slots on every replay, which the run checks from the count."""
 import argparse
 import json
 import os
@@ -58,6 +60,24 @@ def main():
     except Exception as exc:  # capture is best-effort
         us_graph = None
         print("graph capture failed:", repr(exc)[:200], file=sys.stderr)
+    # device-counter buffer: the count is read and advanced on the device, so the 20 captured stores write 20 * E
+    # fresh rows per replay (a host-counter capture rewrites the same slots every replay)
+    rbd = ReplayBuffer(a.size, 5, V + 2, V, device_counter=True)
+    state3, state3_ = state.view(E, V, 5), state_.view(E, V, 5)
+    store_d = lambda: rbd.store_marl(state3, probs, power, rg, rl, state3_, False, mask)  # noqa: E731
+    us_d = timed(store_d)
+    gd = torch.cuda.CUDAGraph()
+    side = torch.cuda.Stream()
+    side.wait_stream(torch.cuda.current_stream())
+    with torch.cuda.stream(side):
+        with torch.cuda.graph(gd, stream=side):
+            for _ in range(20):
+                store_d()
+    torch.cuda.current_stream().wait_stream(side)
+    n0 = rbd.mem_cntr
+    us_d_graph = timed(gd.replay) / 20
+    rows_per_replay = (rbd.mem_cntr - n0) / (a.reps + 3)
+    assert rows_per_replay == 20 * E, rows_per_replay
     row_w = 4 * (2 * 5 * V + V * (V + 2) + 1 + V + V * V) + 1
     row_r = 4 * (2 * 5 * V + V * V + 2 * V + 1 + V) + V * V
     B = 4096
@@ -71,7 +91,9 @@ def main():
     print(json.dumps({"config": {"envs": E, "V": V, "mem_size": a.size}, "store_marl_us": us,
                       "store_marl_us_device_graph": us_graph,
                       "transitions_per_s": E / (us * 1e-6), "bytes_per_row": {"read": row_r, "written": row_w},
-                      "achieved_GBps": gbs, "frac_of_hbm_peak": gbs / peak, "sample_4096_us": us_s}))
+                      "achieved_GBps": gbs, "frac_of_hbm_peak": gbs / peak, "sample_4096_us": us_s,
+                      "device_counter": {"store_marl_us": us_d, "store_marl_us_device_graph": us_d_graph,
+                                         "rows_per_replay_of_20_stores": rows_per_replay}}))
 
 
 if __name__ == "__main__":
