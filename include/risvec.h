@@ -506,12 +506,14 @@ int risvec_set_rng_counters(risvec_env_t* env, const uint64_t in[3]);
 
 /* number of kernels this handle has launched so far (bench.py reports it as gpu_launches) */
 int64_t risvec_launch_count(const risvec_env_t* env);
-/* name of the kernel(s) the latest risvec_rollout_* call on this handle launched ("k_sarl_mma_tma", "k_sarl_mma",
- * "k_sarl_umma", "k_sarl_mma_big", "k_sarl_v8", "k_sarl_rollout", "k_sarl_cascade2+k_sarl_scan", "k_marl_tma",
- * "k_marl_v8", "k_marl_rollout"; "" before the first rollout).  The choice follows the shape; RISVEC_SARL_PATH =
- * auto | mma | mma-ldg | mma-sync | v8 | generic (read at risvec_create) pins the SARL one for tests and A/B
- * measurements (mma-sync: the mma.sync kernel instead of the tcgen05 one for V > 8 or M > 64).  bench.py reports it
- * as roofline.kernel. */
+/* name of the kernel(s) the latest risvec_rollout_* or risvec_step_*_fused call on this handle launched
+ * ("k_sarl_mma_tma", "k_sarl_mma", "k_sarl_umma", "k_sarl_mma_big", "k_sarl_v8", "k_sarl_rollout",
+ * "k_sarl_cascade2+k_sarl_scan", "k_marl_tma", "k_marl_v8", "k_marl_rollout"; "" before the first rollout).  The
+ * choice follows the shape, the traces and arrivals given, their alignment and the packed / fused entry point.
+ * Read at risvec_create, for tests and A/B measurements: RISVEC_SARL_PATH = auto (also spelled mma; any unknown
+ * value) | mma-ldg (k_sarl_mma instead of k_sarl_mma_tma, no k_sarl_umma) | mma-sync (k_sarl_mma_big instead of
+ * k_sarl_umma) | v8 | generic (the FP32-pipe kernels); RISVEC_MARL_PATH = v8 (k_marl_v8 instead of k_marl_tma);
+ * RISVEC_FORCE_GENERIC = 1 (the shape-generic kernels of both variants).  bench.py reports it as roofline.kernel. */
 const char* risvec_last_step_kernel(const risvec_env_t* env);
 
 #ifdef __cplusplus

@@ -65,10 +65,26 @@ struct FieldDesc {
 };
 
 inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
-inline int pow2ceil(int x) {
-    int p = 1;
-    while (p < x) p <<= 1;
-    return p;
+
+// RISVEC_SARL_PATH pins the SARL rollout kernel for tests and A/B runs: auto (also spelled mma, and any unknown
+// spelling) | mma-ldg (k_sarl_mma, no TMA staging) | mma-sync (k_sarl_mma_big for the shapes of k_sarl_umma) | v8 |
+// generic (the FP32-pipe kernels)
+enum SarlPath { kPathAuto, kPathMmaLdg, kPathMmaSync, kPathV8, kPathGeneric };
+struct Overrides {
+    SarlPath sarl;       // RISVEC_FORCE_GENERIC=1 makes it kPathGeneric
+    bool marl_v8;        // RISVEC_MARL_PATH=v8: the MARL fast path stays on k_marl_v8
+    bool force_generic;  // RISVEC_FORCE_GENERIC=1: the shape-generic kernels everywhere (tests)
+};
+Overrides read_overrides() {  // at risvec_create
+    const char *fg = getenv("RISVEC_FORCE_GENERIC"), *sp = getenv("RISVEC_SARL_PATH"), *mp = getenv("RISVEC_MARL_PATH");
+    const char* const sarl_names[] = {"auto", "mma-ldg", "mma-sync", "v8", "generic"};  // SarlPath order
+    Overrides o{};
+    o.force_generic = fg != nullptr && fg[0] == '1';
+    o.marl_v8 = mp != nullptr && !strcmp(mp, "v8");
+    for (int i = 1; i < 5; ++i)
+        if (sp != nullptr && !strcmp(sp, sarl_names[i])) o.sarl = (SarlPath)i;
+    if (o.force_generic) o.sarl = kPathGeneric;
+    return o;
 }
 
 }  // namespace
@@ -91,11 +107,7 @@ struct risvec_env {
     int pipe_ready;
     cudaStream_t s_in, s_out;
     cudaEvent_t ev[2 * 64 + 3];  // 2 * kMaxChunks + 3: per chunk in / kernel, start, in done, done
-    int force_generic;  // RISVEC_FORCE_GENERIC=1: always use the shape-generic kernels (tests)
-    int sarl_umma;      // large shapes: k_sarl_umma (tcgen05) unless RISVEC_SARL_PATH=mma-sync (k_sarl_mma_big)
-    int sarl_path;      // RISVEC_SARL_PATH = auto (0) | mma (1) | v8 (2) | generic (3): tests / A-B runs
-    int sarl_tma;       // RISVEC_SARL_TMA = 0 keeps the mma path on its LDG kernel (tests / A-B runs)
-    int marl_tma;       // RISVEC_MARL_PATH = v8 keeps the MARL fast path on k_marl_v8 (tests / A-B runs)
+    Overrides ovr;  // the kernel overrides of tests and A/B runs
     const char* step_kernel;  // name of the kernel(s) the latest rollout launched (risvec_last_step_kernel)
     double* stats_slots;      // attached statistics accumulator (risvec_attach_stats_accumulator) or null
     int stats_folded;         // the latest rollout kernel added its statistics itself
@@ -165,15 +177,6 @@ int ensure_stage(risvec_env* env, size_t bytes) {
 }
 
 // -------------------------------------------------------------------------- launch helpers
-template <int VP>
-int launch_marl(risvec_env* env, const MarlArgs& a, cudaStream_t st) {
-    const int threads = 128;
-    const long long total = (long long)env->dims.E * VP;
-    const int blocks = (int)((total + threads - 1) / threads);
-    k_marl_rollout<VP><<<blocks, threads, 0, st>>>(env->dims, env->st, env->params, a);
-    return check_step_launch(env, "k_marl_rollout");
-}
-
 int ensure_scratch(risvec_env* env, size_t bytes) {
     if (bytes <= env->scratch_bytes) return RISVEC_OK;
     if (env->scratch) cudaFree(env->scratch);
@@ -184,72 +187,18 @@ int ensure_scratch(risvec_env* env, size_t bytes) {
     return RISVEC_OK;
 }
 
-template <int VP, int MPL, int WPE>
-int launch_sarl_cfg(risvec_env* env, const SarlArgs& a_in, cudaStream_t st) {
-    constexpr int EPW = 32 / VP;
-    SarlArgs a = a_in;
-    const int E = env->dims.E, V = env->dims.V;
-    const int blocks = (E + EPW - 1) / EPW;
-    const size_t MS = (size_t)((env->dims.M + 4 * WPE + 7) / 4) * 4;  // must match the kernel
-    const size_t smem = 6 * EPW * MS * sizeof(float) + (WPE > 1 ? 2 * WPE * 32 * sizeof(float2) : 0);
-    if (WPE == 1) {  // one warp per env group: fused step kernel
-        auto kern = k_sarl_rollout<VP, MPL, WPE>;
-        if (smem > 48 * 1024) CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        kern<<<blocks, 32 * WPE, smem, st>>>(env->dims, env->st, env->params, a);
-        return check_step_launch(env, "k_sarl_rollout");
-    }
-    // several warps per env (large M): cascade kernel over (env group, time chunk) -> |S|^2 scratch,
-    // then the per-vehicle scan kernel
-    if (int rc = ensure_scratch(env, (size_t)a.T * E * V * sizeof(float))) return rc;
-    a.g2 = (float*)env->scratch;
-    int chunk = 32;
-    while (chunk > 2 && (long long)blocks * ((a.T + chunk - 1) / chunk) < 4 * 148) chunk >>= 1;  // fill the SMs
-    a.t_chunk = chunk;
-    if constexpr (WPE > 1) {
-        const size_t smem2 = 8 * EPW * MS * sizeof(float) + 4 * WPE * 32 * sizeof(float2);
-        auto kern = k_sarl_cascade2<VP, MPL, WPE>;
-        if (smem2 > 48 * 1024)
-            CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2));
-        kern<<<dim3(blocks, (a.T + chunk - 1) / chunk), 32 * WPE, smem2, st>>>(env->dims, env->st, a);
-        if (int rc = check_launch(env, "k_sarl_cascade2")) return rc;
-    }
-    const long long total = (long long)E * VP;
-    k_sarl_scan<VP><<<(int)((total + 127) / 128), 128, 0, st>>>(env->dims, env->st, env->params, a);
-    if (int rc = check_launch(env, "k_sarl_scan")) return rc;
-    env->step_kernel = "k_sarl_cascade2+k_sarl_scan";
-    return RISVEC_OK;
+// f(std::integral_constant<int, VP>{}) for the least power of two VP >= V (V <= 32); dispatch_vp<8> starts at 8
+template <int VP = 1, typename F>
+int dispatch_vp(int V, F&& f) {
+    if constexpr (VP < 32)
+        if (V > VP) return dispatch_vp<2 * VP>(V, f);
+    return f(std::integral_constant<int, VP>{});
 }
 
-template <int MPI>
-int launch_sarl_v8(risvec_env* env, const SarlArgs& a, cudaStream_t st) {
-    const int warps = (env->dims.E + 3) / 4;
-    const bool mfull = env->dims.M == 8 * MPI;
-    const risvec_sarl_out_t& o = a.out;
-    const bool full = a.arrivals && o.reward && o.DataBuf && o.data_t && o.data_p && o.over_power && o.over_data &&
-                      o.rate;
-    if (a.in_rec != nullptr)  // packed records (caller guarantees V == 8, M == 8 * MPI)
-        k_sarl_v8<MPI, true, true, true><<<warps, 32, 0, st>>>(env->dims, env->st, env->params, a);
-    else if (mfull && full)
-        k_sarl_v8<MPI, true, true, false><<<warps, 32, 0, st>>>(env->dims, env->st, env->params, a);
-    else if (mfull)
-        k_sarl_v8<MPI, true, false, false><<<warps, 32, 0, st>>>(env->dims, env->st, env->params, a);
-    else
-        k_sarl_v8<MPI, false, false, false><<<warps, 32, 0, st>>>(env->dims, env->st, env->params, a);
-    return check_step_launch(env, "k_sarl_v8");
-}
+inline bool aligned16(const void* p) { return ((uintptr_t)p & 15u) == 0; }
+inline bool aligned8(const void* p) { return ((uintptr_t)p & 7u) == 0; }
 
-// tensor-core path (sarl_mma.cuh): one warp per env, 4 envs per block; V <= 8, M even, M <= 8 KT
-template <int KT>
-int launch_sarl_mma(risvec_env* env, const SarlArgs& a, cudaStream_t st) {
-    const int blocks = (env->dims.E + 3) / 4;
-    const risvec_sarl_out_t& o = a.out;
-    const bool full = env->dims.V == 8 && env->dims.M == 8 * KT && a.arrivals && o.reward && o.DataBuf && o.data_t &&
-                      o.data_p && o.over_power && o.over_data && o.rate;
-    (void)full;  // the fully-specified BASELINE shape normally runs k_sarl_mma_tma; this is the generic form
-    k_sarl_mma<KT, false><<<blocks, 128, 0, st>>>(env->dims, env->st, env->params, a);
-    return check_step_launch(env, "k_sarl_mma");
-}
-// ---- TMA-staged variant (k_sarl_mma_tma): 2-D tensor maps over the caller's arrays, encoded per call
+// ---- tensor maps over the caller's arrays, encoded per call
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
                                   const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
                                   CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
@@ -279,143 +228,292 @@ bool tensor_map_2d(CUtensorMap* m, CUtensorMapDataType dt, const void* base, uin
                CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) ==
            CUDA_SUCCESS;
 }
+// the [T][E * V] float traces of a rollout, 16 steps x box_inner floats per box
+template <int N>
+bool trace_maps(CUtensorMap (&m)[N], float* const (&traces)[N], const Dims& d, int T, uint32_t box_inner) {
+    for (int n = 0; n < N; ++n)
+        if (!tensor_map_2d(&m[n], CU_TENSOR_MAP_DATA_TYPE_FLOAT32, traces[n], (uint64_t)d.E * d.V, T, box_inner, 16))
+            return false;
+    return true;
+}
 
-template <int KT>
+// ---- SARL: the rollout kernels in the order they are tried (choose_sarl)
+enum SarlKernel { kSarlMmaTma, kSarlMma, kSarlUmma, kSarlMmaBig, kSarlV8, kSarlRollout, kSarlCascade };
+
+bool sarl_traces(const risvec_sarl_out_t& o) {  // every per-vehicle trace given, 16-byte aligned
+    const float* const t[6] = {o.DataBuf, o.data_t, o.data_p, o.over_power, o.over_data, o.rate};
+    for (const float* p : t)
+        if (!p || !aligned16(p)) return false;
+    return true;
+}
+// k_sarl_mma_tma covers the BASELINE shape: V = 8, E % 4 == 0, M = 16 or 40, every trace + the arrivals supplied,
+// 16-byte aligned streams, 32-bit element indices
+bool sarl_tma_covers(const Dims& d, const SarlArgs& a) {
+    return d.V == 8 && d.E % 4 == 0 && (d.M == 16 || d.M == 40) && sarl_traces(a.out) && a.arrivals &&
+           a.out.reward && aligned16(a.phase) && aligned16(a.action) && aligned16(a.arrivals) &&
+           aligned16(a.out.reward) && (uint64_t)a.T * d.E * std::max(d.M, 16) < (1ull << 31);
+}
+// k_sarl_umma / k_sarl_mma_big: one block per env for many vehicles or elements (config 4)
+bool sarl_big_covers(const Dims& d, const SarlArgs& a) {
+    return d.V % 4 == 0 && d.V <= 32 && d.M % 2 == 0 && d.M <= 256 && (d.V > 8 || d.M > 64) && sarl_traces(a.out) &&
+           aligned8(a.phase) && (uint64_t)a.T * d.E * std::max(d.M, 2 * d.V) < (1ull << 31);
+}
+
+// The kernel of a SARL rollout (`a.in_rec`: packed records, `a.raw`: the fused driver step), the first candidate
+// from `from` on that takes the call; a caller whose tensor maps cannot be encoded asks again from the next one.
+SarlKernel choose_sarl(const risvec_env* env, const SarlArgs& a, int from = kSarlMmaTma) {
+    const Dims& d = env->dims;
+    const SarlPath p = env->ovr.sarl;
+    if (a.in_rec) return kSarlV8;  // the caller checked the packed shape
+    const bool mma = p == kPathAuto || p == kPathMmaLdg || p == kPathMmaSync;
+    // tensor cores, one warp per env: V <= 8, M even, M <= 64
+    const bool mma_fits = mma && d.V <= 8 && d.M % 2 == 0 && d.M <= 64 && (!a.raw || aligned8(a.raw));
+    if (from <= kSarlMmaTma && mma_fits && p != kPathMmaLdg && sarl_tma_covers(d, a)) return kSarlMmaTma;
+    if (from <= kSarlMma && mma_fits) return kSarlMma;
+    const bool big = mma && p != kPathMmaLdg && sarl_big_covers(d, a);
+    if (from <= kSarlUmma && big && p != kPathMmaSync) return kSarlUmma;
+    if (from <= kSarlMmaBig && big && p == kPathMmaSync) return kSarlMmaBig;
+    if (d.V <= 8 && d.M <= 40 && p != kPathGeneric) return kSarlV8;  // elements split over the env's 8 lanes
+    return d.M <= 40 ? kSarlRollout : kSarlCascade;
+}
+
+// tensor cores + TMA staging (sarl_mma.cuh); dynamic + static shared memory stay under the 48 KB default
 int launch_sarl_mma_tma(risvec_env* env, const SarlArgs& a, cudaStream_t st, bool* launched) {
-    *launched = false;
-    const int E = env->dims.E, V = env->dims.V, M = env->dims.M, T = a.T;
+    const Dims& d = env->dims;
+    const int E = d.E, V = d.V, M = d.M, T = a.T;
     CUtensorMap tm_ph, tm_ac, tm_ar;
     SarlOutMaps tm_out;
     const risvec_sarl_out_t& o = a.out;
-    float* const traces[6] = {o.DataBuf, o.data_t, o.data_p, o.over_power, o.over_data, o.rate};
-    bool ok = tensor_map_2d(&tm_ph, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, a.phase, (uint64_t)E * M, T, M, kSarlTmaRows) &&
-              tensor_map_2d(&tm_ac, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, a.action, (uint64_t)E * 2 * V, T, 2 * V, kSarlTmaRows) &&
-              tensor_map_2d(&tm_ar, CU_TENSOR_MAP_DATA_TYPE_INT32, a.arrivals, (uint64_t)E * V, T, V, kSarlTmaRows) &&
-              tensor_map_2d(&tm_out.reward, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, o.reward, (uint64_t)E, T, 4, kSarlTmaRows);
-    for (int n = 0; n < 6 && ok; ++n)  // the block's four envs x 8 vehicles = one 128-byte line per (trace, step)
-        ok = tensor_map_2d(&tm_out.trace[n], CU_TENSOR_MAP_DATA_TYPE_FLOAT32, traces[n], (uint64_t)E * V, T, 4 * V, kSarlTmaRows);
-    if (!ok) return RISVEC_OK;  // not encodable here: the caller falls back to the LDG kernel
-    auto kern = k_sarl_mma_tma<KT>;
-    const int smem = sarl_tma_smem_bytes(KT);
-    static bool attr_set = false;
-    if (!attr_set) {
-        CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-        attr_set = true;
-    }
+    // the block's four envs x 8 vehicles = one 128-byte line per (trace, step)
+    if (!tensor_map_2d(&tm_ph, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, a.phase, (uint64_t)E * M, T, M, kSarlTmaRows) ||
+        !tensor_map_2d(&tm_ac, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, a.action, (uint64_t)E * 2 * V, T, 2 * V, kSarlTmaRows) ||
+        !tensor_map_2d(&tm_ar, CU_TENSOR_MAP_DATA_TYPE_INT32, a.arrivals, (uint64_t)E * V, T, V, kSarlTmaRows) ||
+        !tensor_map_2d(&tm_out.reward, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, o.reward, (uint64_t)E, T, 4, kSarlTmaRows) ||
+        !trace_maps(tm_out.trace, {o.DataBuf, o.data_t, o.data_p, o.over_power, o.over_data, o.rate}, d, T, 4 * V))
+        return RISVEC_OK;
     SarlArgs af = a;
     af.stats_slots = env->stats_slots;  // the statistics pass rides in the kernel's tail
     env->stats_folded = env->stats_slots != nullptr;
-    kern<<<E / 4, 128, smem, st>>>(env->dims, env->st, sarl_consts(env->params), af, tm_ph, tm_ac, tm_ar, tm_out);
+    const int KT = M == 16 ? 2 : 5;
+    auto kern = KT == 2 ? k_sarl_mma_tma<2> : k_sarl_mma_tma<5>;
+    kern<<<E / 4, 128, sarl_tma_smem_bytes(KT), st>>>(d, env->st, sarl_consts(env->params), af, tm_ph, tm_ac, tm_ar,
+                                                       tm_out);
     *launched = true;
     return check_step_launch(env, "k_sarl_mma_tma");
 }
-inline bool aligned16(const void* p) { return ((uintptr_t)p & 15u) == 0; }
-// the TMA kernel covers the BASELINE shape: V = 8, E % 4 == 0, M = 16 or 40, every trace + the arrivals
-// supplied, 16-byte aligned streams, 32-bit element indices
-inline bool sarl_tma_covers(const risvec_env* env, const SarlArgs& a) {
-    const risvec_sarl_out_t& o = a.out;
-    const int M = env->dims.M;
-    return env->dims.V == 8 && env->dims.E % 4 == 0 && (M == 16 || M == 40) && a.arrivals && o.reward && o.DataBuf &&
-           o.data_t && o.data_p && o.over_power && o.over_data && o.rate && aligned16(a.phase) && aligned16(a.action) &&
-           aligned16(a.arrivals) && aligned16(o.reward) && aligned16(o.DataBuf) && aligned16(o.data_t) &&
-           aligned16(o.data_p) && aligned16(o.over_power) && aligned16(o.over_data) && aligned16(o.rate) &&
-           (uint64_t)a.T * env->dims.E * (M > 16 ? M : 16) < (1ull << 31);
-}
-// ---- many vehicles / elements (config 4): one block per env, k_sarl_mma_big
-template <int KQ>
-int launch_sarl_mma_big(risvec_env* env, const SarlArgs& a, cudaStream_t st, bool* launched) {
-    *launched = false;
-    const int E = env->dims.E, V = env->dims.V, T = a.T;
-    SarlBigOutMaps tm;
-    const risvec_sarl_out_t& o = a.out;
-    float* const traces[6] = {o.DataBuf, o.data_t, o.data_p, o.over_power, o.over_data, o.rate};
-    for (int n = 0; n < 6; ++n)
-        if (!tensor_map_2d(&tm.trace[n], CU_TENSOR_MAP_DATA_TYPE_FLOAT32, traces[n], (uint64_t)E * V, T, V, 16))
-            return RISVEC_OK;  // not encodable: the caller falls back to the FP32-pipe kernels
-    auto kern = k_sarl_mma_big<KQ>;
-    const int smem = sarl_big_smem_bytes(KQ, V);
-    CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    kern<<<E, kBigThreads, smem, st>>>(env->dims, env->st, sarl_consts(env->params), a, tm);
-    *launched = true;
-    return check_step_launch(env, "k_sarl_mma_big");
-}
-// tcgen05 form of the same rollout (sarl_umma.cuh): the default for these shapes; RISVEC_SARL_PATH=mma-sync keeps
-// the mma.sync kernel above for A/B runs
-template <int KQ>
-int launch_sarl_umma(risvec_env* env, const SarlArgs& a, cudaStream_t st, bool* launched) {
-    *launched = false;
-    const int E = env->dims.E, V = env->dims.V, T = a.T;
-    SarlBigOutMaps tm;
-    const risvec_sarl_out_t& o = a.out;
-    float* const traces[6] = {o.DataBuf, o.data_t, o.data_p, o.over_power, o.over_data, o.rate};
-    for (int n = 0; n < 6; ++n)
-        if (!tensor_map_2d(&tm.trace[n], CU_TENSOR_MAP_DATA_TYPE_FLOAT32, traces[n], (uint64_t)E * V, T, V, 16))
-            return RISVEC_OK;  // not encodable: the caller falls back
-    CUtensorMap tm_ac, tm_ar;  // a stage's action rows [16][2 V] and arrivals [16][V] of the block's env
-    if (!tensor_map_2d(&tm_ac, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, a.action, (uint64_t)E * 2 * V, T, 2 * V, 16)) return RISVEC_OK;
-    if (a.arrivals == nullptr)
-        tm_ar = tm_ac;  // unused: arrivals are drawn on the device
-    else if (!tensor_map_2d(&tm_ar, CU_TENSOR_MAP_DATA_TYPE_INT32, a.arrivals, (uint64_t)E * V, T, V, 16))
-        return RISVEC_OK;
-    auto kern = k_sarl_umma<KQ>;
-    const int smem = sarl_umma_smem_request(KQ, V);
-    CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    kern<<<E, kUmmaThreads, smem, st>>>(env->dims, env->st, sarl_consts(env->params), a, tm, tm_ac, tm_ar);
-    *launched = true;
-    return check_step_launch(env, "k_sarl_umma");
-}
-inline bool sarl_big_covers(const risvec_env* env, const SarlArgs& a) {
-    const risvec_sarl_out_t& o = a.out;
-    const int V = env->dims.V, M = env->dims.M;
-    return V % 4 == 0 && V <= 32 && M % 2 == 0 && M <= 256 && (V > 8 || M > 64) && o.DataBuf && o.data_t && o.data_p &&
-           o.over_power && o.over_data && o.rate && aligned16(o.DataBuf) && aligned16(o.data_t) && aligned16(o.data_p) &&
-           aligned16(o.over_power) && aligned16(o.over_data) && aligned16(o.rate) && (((uintptr_t)a.phase) & 7u) == 0 &&
-           (uint64_t)a.T * env->dims.E * (M > 2 * V ? M : 2 * V) < (1ull << 31);
-}
-inline bool sarl_mma_covers(const risvec_env* env) {
-    return env->dims.V <= 8 && env->dims.M % 2 == 0 && env->dims.M <= 64;
+
+// tensor cores, LDG (sarl_mma.cuh): one warp per env, 4 envs per block; KT k-tiles of 8 elements, M <= 8 KT
+int launch_sarl_mma(risvec_env* env, const SarlArgs& a, cudaStream_t st) {
+    using Kern = decltype(&k_sarl_mma<1>);
+    static const Kern kerns[2][5] = {{k_sarl_mma<1>, k_sarl_mma<2>, k_sarl_mma<3>, k_sarl_mma<5>, k_sarl_mma<8>},
+                                     {k_sarl_mma<1, true>, k_sarl_mma<2, true>, k_sarl_mma<3, true>,
+                                      k_sarl_mma<5, true>, k_sarl_mma<8, true>}};
+    const int M = env->dims.M, kt = M <= 8 ? 0 : M <= 16 ? 1 : M <= 24 ? 2 : M <= 40 ? 3 : 4;
+    kerns[a.raw != nullptr][kt]<<<(env->dims.E + 3) / 4, 128, 0, st>>>(env->dims, env->st, env->params, a);
+    return check_step_launch(env, "k_sarl_mma");
 }
 
-template <int VP>
-int launch_sarl(risvec_env* env, const SarlArgs& a, cudaStream_t st) {
-    const int M = env->dims.M;
-    enum { kAuto = 0, kMma = 1, kV8 = 2, kGeneric = 3 };
-    const int path = env->force_generic ? kGeneric : env->sarl_path;
-    if (VP <= 8 && sarl_mma_covers(env) && a.in_rec == nullptr && (path == kAuto || path == kMma)) {
-        if (sarl_tma_covers(env, a) && env->sarl_tma) {
-            bool launched = false;
-            const int rc = M == 16 ? launch_sarl_mma_tma<2>(env, a, st, &launched) : launch_sarl_mma_tma<5>(env, a, st, &launched);
-            if (rc != RISVEC_OK || launched) return rc;
+// one block per env: k_sarl_umma (tcgen05, sarl_umma.cuh) or, RISVEC_SARL_PATH=mma-sync, its mma.sync form
+// k_sarl_mma_big; KQ = 2, 4, 8 for M <= 64, 128, 256
+int launch_sarl_big(risvec_env* env, const SarlArgs& a, cudaStream_t st, bool umma, bool* launched) {
+    const Dims& d = env->dims;
+    const int E = d.E, V = d.V, M = d.M, T = a.T;
+    const risvec_sarl_out_t& o = a.out;
+    SarlBigOutMaps tm;
+    if (!trace_maps(tm.trace, {o.DataBuf, o.data_t, o.data_p, o.over_power, o.over_data, o.rate}, d, T, V))
+        return RISVEC_OK;
+    CUtensorMap tm_ac, tm_ar;  // k_sarl_umma: a stage's action rows [16][2 V] and arrivals [16][V] of the block's env
+    const uint64_t EV = (uint64_t)E * V;
+    if (umma && (!tensor_map_2d(&tm_ac, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, a.action, 2 * EV, T, 2 * V, 16) ||
+                 (a.arrivals && !tensor_map_2d(&tm_ar, CU_TENSOR_MAP_DATA_TYPE_INT32, a.arrivals, EV, T, V, 16))))
+        return RISVEC_OK;
+    if (umma && !a.arrivals) tm_ar = tm_ac;  // unused: arrivals are drawn on the device
+    auto go = [&](auto kq) -> int {
+        constexpr int KQ = decltype(kq)::value;
+        const SarlConsts c = sarl_consts(env->params);
+        if (umma) {
+            const int smem = sarl_umma_smem_request(KQ, V);
+            CUDA_TRY(cudaFuncSetAttribute(k_sarl_umma<KQ>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+            k_sarl_umma<KQ><<<E, kUmmaThreads, smem, st>>>(d, env->st, c, a, tm, tm_ac, tm_ar);
+        } else {
+            const int smem = sarl_big_smem_bytes(KQ, V);
+            CUDA_TRY(cudaFuncSetAttribute(k_sarl_mma_big<KQ>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+            k_sarl_mma_big<KQ><<<E, kBigThreads, smem, st>>>(d, env->st, c, a, tm);
         }
-        if (M <= 8) return launch_sarl_mma<1>(env, a, st);
-        if (M <= 16) return launch_sarl_mma<2>(env, a, st);
-        if (M <= 24) return launch_sarl_mma<3>(env, a, st);
-        if (M <= 40) return launch_sarl_mma<5>(env, a, st);
-        return launch_sarl_mma<8>(env, a, st);
+        *launched = true;
+        return check_step_launch(env, umma ? "k_sarl_umma" : "k_sarl_mma_big");
+    };
+    return M <= 64 ? go(std::integral_constant<int, 2>{})
+                   : M <= 128 ? go(std::integral_constant<int, 4>{}) : go(std::integral_constant<int, 8>{});
+}
+
+// FP32 pipe, the env's 8 lanes split the elements (MPI per lane); packed records: V == 8, M == 8 MPI
+template <int MPI>
+int launch_sarl_v8(risvec_env* env, const SarlArgs& a, cudaStream_t st) {
+    const int warps = (env->dims.E + 3) / 4;
+    const bool mfull = env->dims.M == 8 * MPI;
+    const risvec_sarl_out_t& o = a.out;
+    const bool full = a.arrivals && o.reward && o.DataBuf && o.data_t && o.data_p && o.over_power && o.over_data &&
+                      o.rate;
+    if (a.in_rec != nullptr)
+        k_sarl_v8<MPI, true, true, true><<<warps, 32, 0, st>>>(env->dims, env->st, env->params, a);
+    else if (mfull && full)
+        k_sarl_v8<MPI, true, true, false><<<warps, 32, 0, st>>>(env->dims, env->st, env->params, a);
+    else if (mfull)
+        k_sarl_v8<MPI, true, false, false><<<warps, 32, 0, st>>>(env->dims, env->st, env->params, a);
+    else
+        k_sarl_v8<MPI, false, false, false><<<warps, 32, 0, st>>>(env->dims, env->st, env->params, a);
+    return check_step_launch(env, "k_sarl_v8");
+}
+
+// FP32 pipe, 32 / VP envs per warp: M / WPE elements per lane, a register-resident table of MPL complex floats
+template <int VP, int MPL, int WPE>
+int launch_sarl_cfg(risvec_env* env, const SarlArgs& a_in, cudaStream_t st) {
+    constexpr int EPW = 32 / VP;
+    SarlArgs a = a_in;
+    const int E = env->dims.E, V = env->dims.V;
+    const int blocks = (E + EPW - 1) / EPW;
+    const size_t MS = (size_t)((env->dims.M + 4 * WPE + 7) / 4) * 4;  // must match the kernel
+    if constexpr (WPE == 1) {  // one warp per env group: fused step kernel
+        const size_t smem = 6 * EPW * MS * sizeof(float);
+        auto kern = k_sarl_rollout<VP, MPL, WPE>;
+        if (smem > 48 * 1024) CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        kern<<<blocks, 32 * WPE, smem, st>>>(env->dims, env->st, env->params, a);
+        return check_step_launch(env, "k_sarl_rollout");
+    } else {
+        // several warps per env (large M): cascade kernel over (env group, time chunk) -> |S|^2 scratch,
+        // then the per-vehicle scan kernel
+        if (int rc = ensure_scratch(env, (size_t)a.T * E * V * sizeof(float))) return rc;
+        a.g2 = (float*)env->scratch;
+        int chunk = 32;
+        while (chunk > 2 && (long long)blocks * ((a.T + chunk - 1) / chunk) < 4 * 148) chunk >>= 1;  // fill the SMs
+        a.t_chunk = chunk;
+        const size_t smem2 = 8 * EPW * MS * sizeof(float) + 4 * WPE * 32 * sizeof(float2);
+        auto kern = k_sarl_cascade2<VP, MPL, WPE>;
+        if (smem2 > 48 * 1024)
+            CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2));
+        kern<<<dim3(blocks, (a.T + chunk - 1) / chunk), 32 * WPE, smem2, st>>>(env->dims, env->st, a);
+        if (int rc = check_launch(env, "k_sarl_cascade2")) return rc;
+        const long long total = (long long)E * VP;
+        k_sarl_scan<VP><<<(int)((total + 127) / 128), 128, 0, st>>>(env->dims, env->st, env->params, a);
+        if (int rc = check_launch(env, "k_sarl_scan")) return rc;
+        env->step_kernel = "k_sarl_cascade2+k_sarl_scan";
+        return RISVEC_OK;
     }
-    if ((path == kAuto || path == kMma) && a.in_rec == nullptr && sarl_big_covers(env, a) && env->sarl_tma) {
-        bool launched = false;
-        int rc;
-        if (env->sarl_umma)
-            rc = M <= 64 ? launch_sarl_umma<2>(env, a, st, &launched)
-                         : (M <= 128 ? launch_sarl_umma<4>(env, a, st, &launched) : launch_sarl_umma<8>(env, a, st, &launched));
-        else
-            rc = M <= 64 ? launch_sarl_mma_big<2>(env, a, st, &launched)
-                         : (M <= 128 ? launch_sarl_mma_big<4>(env, a, st, &launched)
-                                     : launch_sarl_mma_big<8>(env, a, st, &launched));
-        if (rc != RISVEC_OK || launched) return rc;
-    }
-    if (VP <= 8 && M <= 40 && path != kGeneric)  // elements split over the env's 8 lanes (FP32 pipe)
-        return M <= 16 ? launch_sarl_v8<2>(env, a, st) : launch_sarl_v8<5>(env, a, st);
-    // elements per lane: M / WPE, register-resident table of MPL complex floats
+}
+template <int VP>
+int launch_sarl_fp32(risvec_env* env, const SarlArgs& a, cudaStream_t st) {
+    const int M = env->dims.M;
     if (M <= 16) return launch_sarl_cfg<VP, 16, 1>(env, a, st);
     if (M <= 40) return launch_sarl_cfg<VP, 40, 1>(env, a, st);
-    if (M <= 64) return launch_sarl_cfg<VP, 32, 2>(env, a, st);
-    if (M <= 128) return launch_sarl_cfg<VP, 32, 4>(env, a, st);
-    if (M <= 256) return launch_sarl_cfg<VP, 32, 8>(env, a, st);
-    if (M <= 512) return launch_sarl_cfg<VP, 32, 16>(env, a, st);
-    if (M <= 1024) return launch_sarl_cfg<VP, 64, 16>(env, a, st);
-    return fail(RISVEC_ERR_UNSUPPORTED, "M = %d > 1024 is not covered by the SARL rollout kernel", M);
+    if constexpr (VP >= 8) {  // M > 40 runs at VP >= 8: 32 / VP envs per warp would not fit shared memory
+        if (M <= 64) return launch_sarl_cfg<VP, 32, 2>(env, a, st);
+        if (M <= 128) return launch_sarl_cfg<VP, 32, 4>(env, a, st);
+        if (M <= 256) return launch_sarl_cfg<VP, 32, 8>(env, a, st);
+        if (M <= 512) return launch_sarl_cfg<VP, 32, 16>(env, a, st);
+        if (M <= 1024) return launch_sarl_cfg<VP, 64, 16>(env, a, st);
+        return fail(RISVEC_ERR_UNSUPPORTED, "M = %d > 1024 is not covered by the SARL rollout kernel", M);
+    } else {  // choose_sarl sends M > 40 only with VP >= 8 (dispatch_vp<8>): not reached
+        return fail(RISVEC_ERR_INVALID, "internal: M = %d > 40 with VP = %d < 8", M, VP);
+    }
+}
+
+int launch_sarl(risvec_env* env, const SarlArgs& a, cudaStream_t st) {
+    const int V = env->dims.V, M = env->dims.M;
+    auto fp32 = [&](auto vp) { return launch_sarl_fp32<decltype(vp)::value>(env, a, st); };
+    for (int from = kSarlMmaTma;;) {
+        const SarlKernel k = choose_sarl(env, a, from);
+        bool launched = false;
+        int rc = RISVEC_OK;
+        switch (k) {
+            case kSarlMmaTma: rc = launch_sarl_mma_tma(env, a, st, &launched); break;
+            case kSarlMma: return launch_sarl_mma(env, a, st);
+            case kSarlUmma:
+            case kSarlMmaBig: rc = launch_sarl_big(env, a, st, k == kSarlUmma, &launched); break;
+            case kSarlV8: return M <= 16 ? launch_sarl_v8<2>(env, a, st) : launch_sarl_v8<5>(env, a, st);
+            case kSarlRollout: return dispatch_vp(V, fp32);
+            case kSarlCascade: return dispatch_vp<8>(V, fp32);
+        }
+        if (rc != RISVEC_OK || launched) return rc;
+        from = k + 1;  // a tensor map could not be encoded here: the next candidate
+    }
+}
+
+// ---- MARL: the rollout kernels in the order they are tried (choose_marl)
+enum MarlKernel { kMarlTma, kMarlV8, kMarlRollout };
+
+// the six bench traces + injected arrivals, no over_power
+bool marl_full(const MarlArgs& a) {
+    const risvec_marl_out_t& o = a.out;
+    return a.arrivals && o.reward_user && o.reward && o.DataBuf && o.data_t && o.data_p && o.rate && !o.over_power;
+}
+// k_marl_tma covers the BASELINE shape: V = 8, E % 4 == 0, marl_full, 16-byte aligned streams, 32-bit indices
+bool marl_tma_covers(const Dims& d, const MarlArgs& a) {
+    const risvec_marl_out_t& o = a.out;
+    return marl_full(a) && d.V == 8 && d.E % 4 == 0 && aligned16(a.action) && aligned16(a.arrivals) &&
+           aligned16(o.reward_user) && aligned16(o.reward) && aligned16(o.DataBuf) && aligned16(o.data_t) &&
+           aligned16(o.data_p) && aligned16(o.rate) && (uint64_t)a.T * d.E * 16 < (1ull << 31);
+}
+// The kernel of a MARL rollout (`a.in_rec`: packed records, `a.raw`: the fused driver step), as choose_sarl
+MarlKernel choose_marl(const risvec_env* env, const MarlArgs& a, int from = kMarlTma) {
+    if (a.in_rec) return kMarlV8;  // the caller checked the packed shape
+    // 4 envs per warp, lane = vehicle
+    const bool v8 = env->dims.V <= 8 && !env->ovr.force_generic && !a.out.stats && !a.out.last_power &&
+                    (!a.raw || aligned8(a.raw));
+    if (from <= kMarlTma && v8 && !env->ovr.marl_v8 && marl_tma_covers(env->dims, a)) return kMarlTma;
+    return v8 ? kMarlV8 : kMarlRollout;
+}
+
+// time-parallel, one warp per env, TMA in / out (marl_tma.cuh); dynamic + static shared memory stay under the
+// 48 KB default
+int launch_marl_tma(risvec_env* env, const MarlArgs& a_in, cudaStream_t st, bool* launched) {
+    const Dims& d = env->dims;
+    const int E = d.E, V = 8, T = a_in.T;
+    const risvec_marl_out_t& o = a_in.out;
+    CUtensorMap tm_ac, tm_ar;
+    MarlOutMaps tm;
+    if (!tensor_map_2d(&tm_ac, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, a_in.action, (uint64_t)E * 2 * V, T, 2 * V, 16) ||
+        !tensor_map_2d(&tm_ar, CU_TENSOR_MAP_DATA_TYPE_INT32, a_in.arrivals, (uint64_t)E * V, T, V, 16) ||
+        !tensor_map_2d(&tm.reward, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, o.reward, (uint64_t)E, T, 4, 16) ||
+        !trace_maps(tm.trace, {o.reward_user, o.DataBuf, o.data_t, o.data_p, o.rate}, d, T, 4 * V))
+        return RISVEC_OK;
+    MarlArgs a = a_in;
+    a.stats_slots = env->stats_slots;  // the statistics pass rides in the kernel's tail
+    env->stats_folded = env->stats_slots != nullptr;
+    k_marl_tma<<<E / 4, 128, kMarlSmemBytes, st>>>(d, env->st, marl_consts(env->params), a, tm_ac, tm_ar, tm);
+    *launched = true;
+    return check_step_launch(env, "k_marl_tma");
+}
+
+int launch_marl_v8(risvec_env* env, const MarlArgs& a, cudaStream_t st) {
+    const int warps = (env->dims.E + 3) / 4;
+    if (a.in_rec)
+        k_marl_v8<true, true><<<warps, 32, 0, st>>>(env->dims, env->st, env->params, a);
+    else if (a.raw)  // action mapping in the prologue, marl_get_state of the new state in the epilogue
+        k_marl_v8<false, false, true><<<warps, 32, 0, st>>>(env->dims, env->st, env->params, a);
+    else if (marl_full(a))
+        k_marl_v8<true, false><<<warps, 32, 0, st>>>(env->dims, env->st, env->params, a);
+    else
+        k_marl_v8<false, false><<<warps, 32, 0, st>>>(env->dims, env->st, env->params, a);
+    return check_step_launch(env, "k_marl_v8");
+}
+
+int launch_marl(risvec_env* env, const MarlArgs& a, cudaStream_t st) {
+    for (int from = kMarlTma;;) {
+        const MarlKernel k = choose_marl(env, a, from);
+        if (k == kMarlV8) return launch_marl_v8(env, a, st);
+        if (k == kMarlRollout)
+            return dispatch_vp(env->dims.V, [&](auto vp) {
+                constexpr int VP = decltype(vp)::value;
+                const long long total = (long long)env->dims.E * VP;
+                k_marl_rollout<VP><<<(int)((total + 127) / 128), 128, 0, st>>>(env->dims, env->st, env->params, a);
+                return check_step_launch(env, "k_marl_rollout");
+            });
+        bool launched = false;
+        const int rc = launch_marl_tma(env, a, st, &launched);
+        if (rc != RISVEC_OK || launched) return rc;
+        from = k + 1;  // a tensor map could not be encoded here: the next candidate
+    }
 }
 
 struct Carver {
@@ -528,26 +626,8 @@ int risvec_create(const risvec_params_t* params, int variant, int E, int V, int 
     memset(env, 0, sizeof(*env));
     env->device = device;
     env->params = *params;
-    {
-        const char* fg = getenv("RISVEC_FORCE_GENERIC");
-        env->force_generic = (fg != nullptr && fg[0] == '1');
-        const char* sp = getenv("RISVEC_SARL_PATH");
-        env->sarl_path = !sp ? 0 : (!strcmp(sp, "mma") ? 1 : (!strcmp(sp, "v8") ? 2 : (!strcmp(sp, "generic") ? 3 : 0)));
-        env->step_kernel = "";
-        const char* mp = getenv("RISVEC_MARL_PATH");
-        env->marl_tma = !(mp != nullptr && !strcmp(mp, "v8"));
-        const char* tm = getenv("RISVEC_SARL_TMA");
-        env->sarl_tma = !(tm != nullptr && tm[0] == '0');
-        if (sp && !strcmp(sp, "mma-ldg")) {  // the tensor-core path without the TMA staging
-            env->sarl_path = 1;
-            env->sarl_tma = 0;
-        }
-        env->sarl_umma = 1;
-        if (sp && !strcmp(sp, "mma-sync")) {  // large shapes: the mma.sync kernel instead of the tcgen05 one
-            env->sarl_path = 1;
-            env->sarl_umma = 0;
-        }
-    }
+    env->ovr = read_overrides();
+    env->step_kernel = "";
     Dims& d = env->dims;
     d.E = E; d.V = V; d.M = M; d.ncand = 1 << control_bit; d.variant = variant;
     d.seed = seed; d.env_base = env_index_base;
@@ -555,8 +635,6 @@ int risvec_create(const risvec_params_t* params, int variant, int E, int V, int 
     d.angle_BR = (kRisX - kBsX) / d.dist_BR;  // MARL:175-177
 
     struct Spec { int f; int64_t rows, cols; int eb, fl; };
-    const int64_t EV = (int64_t)E * V;
-    (void)EV;
     const Spec specs[RISVEC_F_COUNT] = {
         {RISVEC_F_POS_X, E, V, 8, 1}, {RISVEC_F_POS_Y, E, V, 8, 1}, {RISVEC_F_DIR, E, V, 4, 0},
         {RISVEC_F_VEL, E, V, 4, 0}, {RISVEC_F_DIST, E, V, 8, 1}, {RISVEC_F_ANGLE, E, V, 8, 1},
@@ -728,7 +806,7 @@ int launch_compute_parms(risvec_env* env, EnvGate g, void* stream) {
     return check_launch(env, "k_compute_parms");
 }
 int launch_bcd(risvec_env* env, EnvGate g, void* stream) {
-    if (env->dims.ncand <= 8 && env->dims.V <= 8 && env->dims.M <= 256 && !env->force_generic) {
+    if (env->dims.ncand <= 8 && env->dims.V <= 8 && env->dims.M <= 256 && !env->ovr.force_generic) {
         // 4 envs per warp, lane = (env, candidate)
         const int wpb = env->dims.M <= 64 ? 4 : 1;
         const int blocks = (env->dims.E + 4 * wpb - 1) / (4 * wpb);
@@ -748,21 +826,14 @@ int launch_bcd(risvec_env* env, EnvGate g, void* stream) {
 int launch_gains(risvec_env* env, const double* chan_rand, const double* chan_normal, const double* chan_exp, EnvGate g,
                  void* stream) {
     if (env->params.channel_model == RISVEC_CHANNEL_FREE) {
-        if (!env->force_generic) {  // lane = (env, vehicle), sequential over the elements
-            const int VP = pow2ceil(env->dims.V);
-            const long long n = (long long)env->dims.E * VP;
-            const int threads = 128, blocks = (int)((n + threads - 1) / threads);
-            cudaStream_t st = (cudaStream_t)stream;
-            switch (VP) {
-                case 1: k_gains_free_v<1><<<blocks, threads, 0, st>>>(env->dims, env->st, g); break;
-                case 2: k_gains_free_v<2><<<blocks, threads, 0, st>>>(env->dims, env->st, g); break;
-                case 4: k_gains_free_v<4><<<blocks, threads, 0, st>>>(env->dims, env->st, g); break;
-                case 8: k_gains_free_v<8><<<blocks, threads, 0, st>>>(env->dims, env->st, g); break;
-                case 16: k_gains_free_v<16><<<blocks, threads, 0, st>>>(env->dims, env->st, g); break;
-                default: k_gains_free_v<32><<<blocks, threads, 0, st>>>(env->dims, env->st, g); break;
-            }
-            return check_launch(env, "k_gains_free_v");
-        }
+        if (!env->ovr.force_generic)  // lane = (env, vehicle), sequential over the elements
+            return dispatch_vp(env->dims.V, [&](auto vp) {
+                constexpr int VP = decltype(vp)::value;
+                const long long n = (long long)env->dims.E * VP;
+                const int threads = 128, blocks = (int)((n + threads - 1) / threads);
+                k_gains_free_v<VP><<<blocks, threads, 0, (cudaStream_t)stream>>>(env->dims, env->st, g);
+                return check_launch(env, "k_gains_free_v");
+            });
         const int wpb = 4, threads = 32 * wpb, blocks = (env->dims.E + wpb - 1) / wpb;
         k_gains_free<<<blocks, threads, 0, (cudaStream_t)stream>>>(env->dims, env->st, g);
         return check_launch(env, "k_gains_free");
@@ -792,16 +863,11 @@ int check_sarl_args(const risvec_env* env, int T, const void* action, const void
     return RISVEC_OK;
 }
 // ---- packed record layout (include/risvec.h): one input / one output stream per rollout
-int packed_sarl_mpi(const risvec_env* env) {  // 0 = shape not covered by the packed kernels
-    const int V = env->dims.V, M = env->dims.M;
-    if (V != 8 || env->dims.E % 4 != 0) return 0;
-    return M == 16 ? 2 : (M == 40 ? 5 : 0);
-}
 int check_sarl_packed_args(const risvec_env* env, int T, const void* in_rec, const void* out_rec, const void* reward) {
     if (!env) return fail(RISVEC_ERR_INVALID, "NULL handle");
     if (env->dims.variant != RISVEC_VARIANT_SARL) return fail(RISVEC_ERR_INVALID, "handle is not a SARL env");
     if (T < 1 || !in_rec || !out_rec || !reward) return fail(RISVEC_ERR_INVALID, "T >= 1 and all three buffers are required");
-    if (!packed_sarl_mpi(env))
+    if (env->dims.V != 8 || env->dims.E % 4 != 0 || (env->dims.M != 16 && env->dims.M != 40))
         return fail(RISVEC_ERR_UNSUPPORTED, "packed SARL records need V == 8, E %% 4 == 0 and M in {16, 40} "
                     "(got V = %d, E = %d, M = %d)", env->dims.V, env->dims.E, env->dims.M);
     return RISVEC_OK;
@@ -852,52 +918,7 @@ static int rollout_marl_impl(risvec_env_t* env, int T, const float* action, cons
     memset(&a, 0, sizeof(a));
     a.T = T; a.action = action; a.partner = partner; a.ngroups = ngroups; a.arrivals = arrivals;
     if (out) a.out = *out;
-    cudaStream_t st = (cudaStream_t)stream;
-    if (env->dims.V <= 8 && !env->force_generic && !a.out.stats && !a.out.last_power) {
-        // fast path: 4 envs per warp, lane = vehicle (FULL = the six bench traces + injected arrivals)
-        const risvec_marl_out_t& o = a.out;
-        const bool full = arrivals && o.reward_user && o.reward && o.DataBuf && o.data_t && o.data_p && o.rate &&
-                          !o.over_power;
-        // BASELINE shape: the time-parallel kernel (one warp per env, TMA in / out); RISVEC_MARL_PATH=v8 pins the old one
-        if (full && env->marl_tma && env->dims.V == 8 && env->dims.E % 4 == 0 && aligned16(action) && aligned16(arrivals) &&
-            aligned16(o.reward_user) && aligned16(o.reward) && aligned16(o.DataBuf) && aligned16(o.data_t) &&
-            aligned16(o.data_p) && aligned16(o.rate) && (uint64_t)T * env->dims.E * 16 < (1ull << 31)) {
-            const int E = env->dims.E, V = 8;
-            CUtensorMap tm_ac, tm_ar;
-            MarlOutMaps tm;
-            float* const traces[5] = {o.reward_user, o.DataBuf, o.data_t, o.data_p, o.rate};
-            bool ok = tensor_map_2d(&tm_ac, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, action, (uint64_t)E * 2 * V, T, 2 * V, 16) &&
-                      tensor_map_2d(&tm_ar, CU_TENSOR_MAP_DATA_TYPE_INT32, arrivals, (uint64_t)E * V, T, V, 16) &&
-                      tensor_map_2d(&tm.reward, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, o.reward, (uint64_t)E, T, 4, 16);
-            for (int n = 0; n < 5 && ok; ++n)
-                ok = tensor_map_2d(&tm.trace[n], CU_TENSOR_MAP_DATA_TYPE_FLOAT32, traces[n], (uint64_t)E * V, T, 4 * V, 16);
-            if (ok) {
-                static bool attr_set = false;
-                if (!attr_set) {
-                    CUDA_TRY(cudaFuncSetAttribute(k_marl_tma, cudaFuncAttributeMaxDynamicSharedMemorySize, kMarlSmemBytes));
-                    attr_set = true;
-                }
-                a.stats_slots = env->stats_slots;  // the statistics pass rides in the kernel's tail
-                env->stats_folded = env->stats_slots != nullptr;
-                k_marl_tma<<<E / 4, 128, kMarlSmemBytes, st>>>(env->dims, env->st, marl_consts(env->params), a, tm_ac, tm_ar, tm);
-                return check_step_launch(env, "k_marl_tma");
-            }
-        }
-        const int warps = (env->dims.E + 3) / 4;
-        if (full)
-            k_marl_v8<true, false><<<warps, 32, 0, st>>>(env->dims, env->st, env->params, a);
-        else
-            k_marl_v8<false, false><<<warps, 32, 0, st>>>(env->dims, env->st, env->params, a);
-        return check_step_launch(env, "k_marl_v8");
-    }
-    switch (pow2ceil(env->dims.V)) {
-        case 1: return launch_marl<1>(env, a, st);
-        case 2: return launch_marl<2>(env, a, st);
-        case 4: return launch_marl<4>(env, a, st);
-        case 8: return launch_marl<8>(env, a, st);
-        case 16: return launch_marl<16>(env, a, st);
-        default: return launch_marl<32>(env, a, st);
-    }
+    return launch_marl(env, a, (cudaStream_t)stream);
 }
 
 static int rollout_sarl_impl(risvec_env_t* env, int T, const float* action, const float* phase, const int32_t* arrivals,
@@ -908,17 +929,7 @@ static int rollout_sarl_impl(risvec_env_t* env, int T, const float* action, cons
     memset(&a, 0, sizeof(a));
     a.T = T; a.action = action; a.phase = phase; a.arrivals = arrivals;
     if (out) a.out = *out;
-    cudaStream_t st = (cudaStream_t)stream;
-    int vp = pow2ceil(env->dims.V);
-    if (vp < 8 && env->dims.M > 40) vp = 8;  // few vehicles x many elements: 32 / VP envs per warp would not fit shared memory
-    switch (vp) {
-        case 1: return launch_sarl<1>(env, a, st);
-        case 2: return launch_sarl<2>(env, a, st);
-        case 4: return launch_sarl<4>(env, a, st);
-        case 8: return launch_sarl<8>(env, a, st);
-        case 16: return launch_sarl<16>(env, a, st);
-        default: return launch_sarl<32>(env, a, st);
-    }
+    return launch_sarl(env, a, (cudaStream_t)stream);
 }
 
 int risvec_rollout_sarl_packed(risvec_env_t* env, int T, const void* in_rec, float* out_rec, float* reward,
@@ -928,8 +939,7 @@ int risvec_rollout_sarl_packed(risvec_env_t* env, int T, const void* in_rec, flo
     SarlArgs a;
     memset(&a, 0, sizeof(a));
     a.T = T; a.in_rec = (const float*)in_rec; a.out_rec = out_rec; a.out.reward = reward;
-    return packed_sarl_mpi(env) == 2 ? launch_sarl_v8<2>(env, a, (cudaStream_t)stream)
-                                     : launch_sarl_v8<5>(env, a, (cudaStream_t)stream);
+    return launch_sarl(env, a, (cudaStream_t)stream);
 }
 
 int risvec_rollout_marl_packed(risvec_env_t* env, int T, const void* in_rec, const int32_t* partner,
@@ -940,9 +950,7 @@ int risvec_rollout_marl_packed(risvec_env_t* env, int T, const void* in_rec, con
     memset(&a, 0, sizeof(a));
     a.T = T; a.in_rec = (const float*)in_rec; a.partner = partner; a.ngroups = ngroups; a.out_rec = out_rec;
     a.out.reward = reward;
-    const int warps = (env->dims.E + 3) / 4;
-    k_marl_v8<true, true><<<warps, 32, 0, (cudaStream_t)stream>>>(env->dims, env->st, env->params, a);
-    return check_step_launch(env, "k_marl_v8");
+    return launch_marl(env, a, (cudaStream_t)stream);
 }
 
 }  // extern "C"
@@ -1154,15 +1162,13 @@ int risvec_step_marl_fused(risvec_env_t* env, const float* raw, const int32_t* p
     if (!raw || !partner || !ngroups || !obs) return fail(RISVEC_ERR_INVALID, "raw, partner, ngroups and obs are required");
     ENTER_DEVICE(env->device);
     const Dims& d = env->dims;
-    cudaStream_t st = (cudaStream_t)stream;
-    if (d.V <= 8 && !env->force_generic && (((uintptr_t)raw) & 7u) == 0) {
+    MarlArgs a;
+    memset(&a, 0, sizeof(a));
+    a.T = 1; a.raw = raw; a.obs = obs; a.partner = partner; a.ngroups = ngroups; a.arrivals = arrivals;
+    if (choose_marl(env, a) == kMarlV8) {
         // ONE launch: action mapping in the prologue, Environ.step, marl_get_state of the new state in the epilogue
-        MarlArgs a;
-        memset(&a, 0, sizeof(a));
-        a.T = 1; a.raw = raw; a.obs = obs; a.partner = partner; a.ngroups = ngroups; a.arrivals = arrivals;
-        k_marl_v8<false, false, false, true><<<(d.E + 3) / 4, 32, 0, st>>>(d, env->st, env->params, a);
         env->stats_folded = 0;  // an attached statistics accumulator is served by k_shard_stats
-        return finish_rollout(env, check_step_launch(env, "k_marl_v8"), stream);
+        return finish_rollout(env, launch_marl_v8(env, a, (cudaStream_t)stream), stream);
     }
     // shapes the fused kernel does not take: the same three steps as separate launches (scratch action in the stage)
     if (int rc = ensure_stage(env, (size_t)d.E * 2 * d.V * 4 + 256)) return rc;
@@ -1179,21 +1185,13 @@ int risvec_step_sarl_fused(risvec_env_t* env, const float* raw, const int32_t* a
     if (!raw || !obs) return fail(RISVEC_ERR_INVALID, "raw and obs are required");
     ENTER_DEVICE(env->device);
     const Dims& d = env->dims;
-    cudaStream_t st = (cudaStream_t)stream;
-    const bool mma_ok = !env->force_generic && (env->sarl_path == 0 || env->sarl_path == 1) && sarl_mma_covers(env);
-    if (mma_ok && (((uintptr_t)raw) & 7u) == 0) {
+    SarlArgs a;
+    memset(&a, 0, sizeof(a));
+    a.T = 1; a.raw = raw; a.obs = obs; a.arrivals = arrivals;
+    if (choose_sarl(env, a) == kSarlMma) {
         // ONE launch: action mapping in the prologue, Environ.step, get_state of the new state in the epilogue
-        SarlArgs a;
-        memset(&a, 0, sizeof(a));
-        a.T = 1; a.raw = raw; a.obs = obs; a.arrivals = arrivals;
-        const int M = d.M, blocks = (d.E + 3) / 4;
-        if (M <= 8) k_sarl_mma<1, false, true><<<blocks, 128, 0, st>>>(d, env->st, env->params, a);
-        else if (M <= 16) k_sarl_mma<2, false, true><<<blocks, 128, 0, st>>>(d, env->st, env->params, a);
-        else if (M <= 24) k_sarl_mma<3, false, true><<<blocks, 128, 0, st>>>(d, env->st, env->params, a);
-        else if (M <= 40) k_sarl_mma<5, false, true><<<blocks, 128, 0, st>>>(d, env->st, env->params, a);
-        else k_sarl_mma<8, false, true><<<blocks, 128, 0, st>>>(d, env->st, env->params, a);
         env->stats_folded = 0;  // an attached statistics accumulator is served by k_shard_stats
-        return finish_rollout(env, check_step_launch(env, "k_sarl_mma"), stream);
+        return finish_rollout(env, launch_sarl_mma(env, a, (cudaStream_t)stream), stream);
     }
     // shapes the fused kernel does not take: the same three steps as separate launches (scratch in the stage)
     if (int rc = ensure_stage(env, (size_t)d.E * (2 * d.V + d.M) * 4 + 512)) return rc;
@@ -1369,7 +1367,7 @@ constexpr int kEpAll = RISVEC_EP_RESET | RISVEC_EP_POSITIONS | RISVEC_EP_CHANNEL
 bool episode_fused(const risvec_env* env) {
     const Dims& d = env->dims;
     return d.V <= 8 && d.ncand <= 8 && d.M <= 256 && env->params.channel_model == RISVEC_CHANNEL_FREE &&
-           !env->force_generic;
+           !env->ovr.force_generic;
 }
 
 template <bool CLOCK>

@@ -61,18 +61,16 @@ struct SarlMmaIn {     // inputs of one 8-step tile, as one lane needs them
     int arr[2];
 };
 
-// KT = k-tiles of 8 RIS elements (M <= 8 KT, M even); FULL = V == 8, M == 8 KT, every trace and the
-// arrivals supplied (no per-access predicates).  Block = 4 warps = 4 adjacent envs.
+// KT = k-tiles of 8 RIS elements (M <= 8 KT, M even).  Block = 4 warps = 4 adjacent envs.
 // FUSED = the one-launch driver step (risvec_step_sarl_fused): inputs from the actor's raw row, observation out
-template <int KT, bool FULL, bool FUSED = false>
+template <int KT, bool FUSED = false>
 __global__ void __launch_bounds__(128, 4) k_sarl_mma(Dims d, State s, risvec_params_t p, SarlArgs a) {
-    static_assert(!(FULL && FUSED), "the fused driver step is a variant of the generic form");
     const int lane = threadIdx.x & 31, g = lane >> 2, tig = lane & 3;
     const int E = d.E, V = d.V, M = d.M, T = a.T;
     const int e = blockIdx.x * 4 + (threadIdx.x >> 5);
     if (e >= E) return;  // warps are independent: no block-level synchronisation below
-    const bool vact = FULL ? true : (g < V);
-    const int vc = FULL ? g : min(g, V - 1);
+    const bool vact = g < V;
+    const int vc = min(g, V - 1);
     const size_t ev = (size_t)e * V + vc;
 
     // ---- A operand: phasors of vehicle g at the elements m = 8 j + 2 tig + {0, 1} of every k-tile
@@ -87,8 +85,8 @@ __global__ void __launch_bounds__(128, 4) k_sarl_mma(Dims d, State s, risvec_par
         for (int j = 0; j < KT; ++j) {
             const int ma = 8 * j + 2 * tig;
             double2 wa = w, wb = cmul64(w, z);
-            if (!(vact && (FULL || ma < M))) wa = make_double2(0.0, 0.0);
-            if (!(vact && (FULL || ma + 1 < M))) wb = make_double2(0.0, 0.0);
+            if (!(vact && ma < M)) wa = make_double2(0.0, 0.0);
+            if (!(vact && ma + 1 < M)) wb = make_double2(0.0, 0.0);
             split_h2(wa.x, -wa.y, Ah[j][0], Al[j][0]);  // row g     (Re S_g): ( Re w, -Im w)
             split_h2(wa.y, wa.x, Ah[j][1], Al[j][1]);   // row g + 8 (Im S_g): ( Im w,  Re w)
             split_h2(wb.x, -wb.y, Ah[j][2], Al[j][2]);
@@ -110,7 +108,7 @@ __global__ void __launch_bounds__(128, 4) k_sarl_mma(Dims d, State s, risvec_par
     const size_t sM = (size_t)E * M, s2V = (size_t)E * 2 * V, sV = (size_t)E * V;
     const float* const ph_b = a.phase + (size_t)e * M + 2 * tig;
     const float* const ac_b = a.action + (size_t)e * 2 * V + vc;
-    const int* const ar_b = (FULL || a.arrivals != nullptr) ? a.arrivals + ev : nullptr;
+    const int* const ar_b = a.arrivals != nullptr ? a.arrivals + ev : nullptr;
     const int Tm1 = T - 1;
 
     // fused driver step: the action mapping of ddpg_train.py:151-160 (k_map_actions_sarl) applied to the raw row
@@ -132,7 +130,7 @@ __global__ void __launch_bounds__(128, 4) k_sarl_mma(Dims d, State s, risvec_par
         const float* q = ph_b + (size_t)min(t0 + g, Tm1) * sM;  // B fragment column g = step t0 + g
 #pragma unroll
         for (int j = 0; j < KT; ++j)
-            ph[j] = (FULL || 8 * j + 2 * tig < M) ? __ldg(reinterpret_cast<const float2*>(q + 8 * j))
+            ph[j] = 8 * j + 2 * tig < M ? __ldg(reinterpret_cast<const float2*>(q + 8 * j))
                                                   : make_float2(0.f, 0.f);
     };
     auto load_scalars = [&](SarlMmaIn& in, int t0) {
@@ -146,7 +144,7 @@ __global__ void __launch_bounds__(128, 4) k_sarl_mma(Dims d, State s, risvec_par
                 in.a0[i] = __ldg(ac_b + t * s2V);
                 in.a1[i] = __ldg(ac_b + t * s2V + V);
             }
-            in.arr[i] = (FULL || ar_b != nullptr) ? __ldg(ar_b + t * sV) : 0;
+            in.arr[i] = ar_b != nullptr ? __ldg(ar_b + t * sV) : 0;
         }
     };
     // L2 prefetch of the env's rows of a later tile: lane (g, tig) covers sectors of row t0 + g
@@ -154,10 +152,10 @@ __global__ void __launch_bounds__(128, 4) k_sarl_mma(Dims d, State s, risvec_par
         if (fused) return;  // one step: nothing to pull ahead
         const size_t t = (size_t)min(t0 + g, Tm1);
         const float* q = a.phase + t * sM + (size_t)e * M + tig * 8;  // M <= 64: at most two sectors per lane
-        if (FULL || tig * 8 < M) asm volatile("prefetch.global.L2 [%0];" ::"l"(q));
-        if (tig * 8 + 32 < (FULL ? 8 * KT : M)) asm volatile("prefetch.global.L2 [%0];" ::"l"(q + 32));
+        if (tig * 8 < M) asm volatile("prefetch.global.L2 [%0];" ::"l"(q));
+        if (tig * 8 + 32 < M) asm volatile("prefetch.global.L2 [%0];" ::"l"(q + 32));
         if (tig * 8 < 2 * V) asm volatile("prefetch.global.L2 [%0];" ::"l"(a.action + t * s2V + (size_t)e * 2 * V + tig * 8));
-        if (tig == 3 && (FULL || ar_b != nullptr)) asm volatile("prefetch.global.L2 [%0];" ::"l"(a.arrivals + t * sV + (size_t)e * V));
+        if (tig == 3 && ar_b != nullptr) asm volatile("prefetch.global.L2 [%0];" ::"l"(a.arrivals + t * sV + (size_t)e * V));
     };
 
     // values of the two steps of the latest tile (the owner of step T - 1 writes them to the state)
@@ -194,7 +192,7 @@ __global__ void __launch_bounds__(128, 4) k_sarl_mma(Dims d, State s, risvec_par
             dt[i] = __fmul_rn(rate[i], c_dt);
             dp[i] = __fmul_rn(cbrt_sfu(in.a1[i]), c_dp);                    // SARL:331
             arr[i] = in.arr[i];
-            if (!FULL && ar_b == nullptr) arr[i] = (vact && ok[i]) ? draw_arrival(d, e, vc, step0 + t, lam) : 0;
+            if (ar_b == nullptr) arr[i] = (vact && ok[i]) ? draw_arrival(d, e, vc, step0 + t, lam) : 0;
             // steps past the end of the rollout are the identity of the recursion (DataBuf >= 0)
             dd[i] = ok[i] ? __dadd_rn((double)dt[i], (double)dp[i]) : 0.0;
             inc[i] = ok[i] ? __dmul_rn(__dmul_rn((double)arr[i], tf), 1000.0) : 0.0;
@@ -233,13 +231,13 @@ __global__ void __launch_bounds__(128, 4) k_sarl_mma(Dims d, State s, risvec_par
             cur = __dadd_rn(nb, inc[i]);  // SARL:354-356
             if (vact && ok[i]) {
                 const size_t o = (size_t)t * sV + ev;
-                if (FULL || a.out.DataBuf) a.out.DataBuf[o] = (float)cur;
-                if (FULL || a.out.data_t) a.out.data_t[o] = dt[i];
-                if (FULL || a.out.data_p) a.out.data_p[o] = dp[i];
-                if (FULL || a.out.over_power) a.out.over_power[o] = overp;
-                if (FULL || a.out.over_data) a.out.over_data[o] = overd;
-                if (FULL || a.out.rate) a.out.rate[o] = rate[i];
-                if (g == 0 && (FULL || a.out.reward)) a.out.reward[(size_t)t * E + e] = rew;
+                if (a.out.DataBuf) a.out.DataBuf[o] = (float)cur;
+                if (a.out.data_t) a.out.data_t[o] = dt[i];
+                if (a.out.data_p) a.out.data_p[o] = dp[i];
+                if (a.out.over_power) a.out.over_power[o] = overp;
+                if (a.out.over_data) a.out.over_data[o] = overd;
+                if (a.out.rate) a.out.rate[o] = rate[i];
+                if (g == 0 && a.out.reward) a.out.reward[(size_t)t * E + e] = rew;
             }
             o_rate[i] = rate[i]; o_dt[i] = dt[i]; o_dp[i] = dp[i]; o_overp[i] = overp; o_overd[i] = overd;
             o_rew[i] = rew; o_arr[i] = arr[i];

@@ -871,14 +871,13 @@ struct SarlHeavyOut {  // state-independent results of a step
     float rate, data_p;
 };
 
-// ALLACT: V == 8 and E % 4 == 0, i.e. every lane of every warp owns a vehicle (always so with the
-// packed records).  `act` is then a compile-time constant: no predicated store regions, which
-// otherwise cut the loop body into separately scheduled blocks (packed SARL: 0.156 -> 0.148 ms,
-// packed MARL: 0.133 -> 0.118 ms).  The per-array MARL kernel measured slower without its
-// predicates (0.116 -> 0.131 ms), so only the packed instantiations use it.
-template <int MPI, bool MFULL, bool FULL, bool PACKED, bool ALLACT = PACKED>
+// PACKED records have V == 8 and E % 4 == 0, i.e. every lane of every warp owns a vehicle.  `act` is then a
+// compile-time constant: no predicated store regions, which otherwise cut the loop body into separately scheduled
+// blocks (packed SARL: 0.156 -> 0.148 ms, packed MARL: 0.133 -> 0.118 ms).  The per-array MARL kernel measured
+// slower without its predicates (0.116 -> 0.131 ms), so only the packed instantiations drop them.
+template <int MPI, bool MFULL, bool FULL, bool PACKED>
 __global__ void __launch_bounds__(32) k_sarl_v8(Dims d, State s, risvec_params_t p, SarlArgs a) {
-    static_assert(!PACKED || (MFULL && FULL && ALLACT), "the packed record layout carries every stream");
+    static_assert(!PACKED || (MFULL && FULL), "the packed record layout carries every stream");
     constexpr int RIN = 24 + 8 * MPI;            // packed input record (words): a0[8] a1[8] arr[8] phase[M]
     constexpr int ROUT = RISVEC_SARL_OUT_WORDS;  // packed output record: six traces x 8 vehicles
     const int lane = threadIdx.x & 31, el = lane >> 3, part = lane & 7;
@@ -886,7 +885,7 @@ __global__ void __launch_bounds__(32) k_sarl_v8(Dims d, State s, risvec_params_t
     const int e_raw = blockIdx.x * 4 + el;
     const bool env_ok = e_raw < E;
     const int e = min(e_raw, E - 1), v = part, vc = min(v, V - 1);  // clamped copies are load-only
-    const bool act = ALLACT ? true : (env_ok && v < V);
+    const bool act = PACKED || (env_ok && v < V);
     const size_t ev = (size_t)e * V + vc;
 
     // ---- geometry phasors of my elements for the 8 vehicles (slot = v ^ part) -> registers
@@ -1140,17 +1139,17 @@ struct MarlHeavy {
 };
 
 // FUSED = the one-launch driver step (risvec_step_marl_fused): actions from the actors' raw outputs, observation out
-template <bool FULL, bool PACKED, bool ALLACT = PACKED, bool FUSED = false>
+template <bool FULL, bool PACKED, bool FUSED = false>
 __global__ void __launch_bounds__(32) k_marl_v8(Dims d, State s, risvec_params_t p, MarlArgs a) {
     static_assert(!FUSED || (!FULL && !PACKED), "the fused driver step is a variant of the generic form");
-    static_assert(!PACKED || (FULL && ALLACT), "the packed record layout carries every stream");
+    static_assert(!PACKED || FULL, "the packed record layout carries every stream");
     constexpr int RIN = RISVEC_MARL_IN_WORDS, ROUT = RISVEC_MARL_OUT_WORDS;
     const int lane = threadIdx.x & 31, el = lane >> 3, v = lane & 7;
     const int E = d.E, V = d.V, T = a.T;
     const int e_raw = blockIdx.x * 4 + el;
     const bool env_ok = e_raw < E;
     const int e = min(e_raw, E - 1), vc = min(v, V - 1);
-    const bool act = ALLACT ? true : (env_ok && v < V);
+    const bool act = PACKED || (env_ok && v < V);
     const size_t ev = (size_t)e * V + vc;
 
     double buf = act ? s.databuf[ev] : 0.0;

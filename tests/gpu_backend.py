@@ -1,5 +1,8 @@
 """Adapter: golden scenario inputs -> `BatchedEnviron` (the CUDA library through the C ABI).
 Same interface as `tests.replay.OracleBackend`, so `tests.replay.replay` drives both."""
+import contextlib
+import os
+
 import numpy as np
 import torch
 
@@ -13,26 +16,22 @@ def np64(t):
 FAST_MARL_TRACES = ("reward_user", "reward", "DataBuf", "data_t", "data_p", "rate")
 
 
-class sarl_path:
-    """`with sarl_path("v8"): env = BatchedEnviron("sarl", ...)` pins the SARL rollout kernel of the handles
-    created inside (RISVEC_SARL_PATH = auto | mma | v8 | generic is read by risvec_create)."""
-
-    def __init__(self, path):
-        self.path = path
-
-    def __enter__(self):
-        import os
-
-        self.old = os.environ.get("RISVEC_SARL_PATH")
-        os.environ["RISVEC_SARL_PATH"] = self.path
-
-    def __exit__(self, *exc):
-        import os
-
-        if self.old is None:
-            os.environ.pop("RISVEC_SARL_PATH", None)
-        else:
-            os.environ["RISVEC_SARL_PATH"] = self.old
+@contextlib.contextmanager
+def kernel_paths(sarl=None, marl=None):
+    """`with kernel_paths(sarl="v8"): env = BatchedEnviron("sarl", ...)` pins the rollout kernels of the handles
+    created inside: risvec_create reads RISVEC_SARL_PATH = auto | mma | mma-ldg | mma-sync | v8 | generic and
+    RISVEC_MARL_PATH (v8 keeps the MARL fast path on k_marl_v8).  A None path leaves its variable as it is."""
+    paths = {k: v for k, v in (("RISVEC_SARL_PATH", sarl), ("RISVEC_MARL_PATH", marl)) if v is not None}
+    old = {k: os.environ.get(k) for k in paths}
+    os.environ.update(paths)
+    try:
+        yield
+    finally:
+        for k, v in old.items():
+            if v is None:
+                os.environ.pop(k, None)
+            else:
+                os.environ[k] = v
 
 
 class GpuBackend:
@@ -41,8 +40,6 @@ class GpuBackend:
     does).  mode="generic": RISVEC_FORCE_GENERIC=1, the shape-generic kernels with every trace."""
 
     def __init__(self, g, device=0, mode="fast"):
-        import os
-
         over = marl_yaml_overrides() if (g["variant"] == "marl" and g["params"] == "yaml") else {}
         self.g, self.mode = g, mode
         old = os.environ.get("RISVEC_FORCE_GENERIC")

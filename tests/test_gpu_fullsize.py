@@ -28,9 +28,9 @@ def _sarl_env(path, E, V, M):
     """SARL env whose rollouts go through one named kernel path (ris_vec_marl_b200/csrc/risvec.cu
     `launch_sarl`): RISVEC_SARL_PATH is read once, when the handle is created."""
     from ris_vec_marl_b200 import BatchedEnviron
-    from tests.gpu_backend import sarl_path
+    from tests.gpu_backend import kernel_paths
 
-    with sarl_path({"packed": "v8"}.get(path, path)):
+    with kernel_paths(sarl={"packed": "v8"}.get(path, path)):
         return BatchedEnviron("sarl", E, V, M)
 
 
@@ -102,12 +102,10 @@ def test_sarl_4096_envs_rollout_matches_oracle(path, V, M, E, kernel):
 
 @pytest.mark.parametrize("path,kernel,T", [("tma", "k_marl_tma", 40), ("tma", "k_marl_tma", 32), ("v8", "k_marl_v8", 12)])
 def test_marl_4096_envs_rollout_matches_oracle(path, kernel, T):
-    import os
-
     from ris_vec_marl_b200 import BatchedEnviron, marl_yaml_overrides
+    from tests.gpu_backend import kernel_paths
 
     E, V, M = 4096, 8, 40
-    os.environ["RISVEC_MARL_PATH"] = path  # read when the handle is created
     rng = np.random.default_rng(77)
     ri = reset_draws(rng, E, V)
     mob = rng.random((E, 8 * V))
@@ -117,10 +115,8 @@ def test_marl_4096_envs_rollout_matches_oracle(path, kernel, T):
     part, ng = encode_groups([[0, 1], [3, 2], [4, 5], [6], [7]], V)
     partner, ngroups = np.tile(part, (E, 1)), np.full(E, ng, dtype=np.int32)
 
-    try:
+    with kernel_paths(marl=path):
         env = BatchedEnviron("marl", E, V, M, **marl_yaml_overrides())
-    finally:
-        os.environ.pop("RISVEC_MARL_PATH", None)
     env.make_new_game(ri); env.renew_positions(mob); env.compute_parms()
     phase0 = np.zeros((E, M), dtype=np.float32)
     env.get_next_phase(phase0)  # theta = 1: includes destructive-interference gains

@@ -212,7 +212,7 @@ def test_packed_records_are_bit_identical_to_per_array_api():
     """The packed record entry points (device and pinned-host pipelines) against the per-array
     ones: same kernels' arithmetic, so every trace and the final state must match bit for bit."""
     from ris_vec_marl_b200 import BatchedEnviron, RisvecError, encode_groups, marl_yaml_overrides
-    from tests.gpu_backend import sarl_path
+    from tests.gpu_backend import kernel_paths
 
     E, V, M, T = 1028, 8, 40, 37  # odd T; E % 4 == 0 as the tiled layout requires
     gen = torch.Generator().manual_seed(21)
@@ -221,7 +221,7 @@ def test_packed_records_are_bit_identical_to_per_array_api():
     arr = torch.poisson(torch.full((T, E, V), 2.0), generator=gen).to(torch.int32)
     for variant in ("sarl", "marl"):
         over = marl_yaml_overrides() if variant == "marl" else {}
-        with sarl_path("v8"):  # the packed SARL records run k_sarl_v8: compare with the same kernel's per-array form
+        with kernel_paths(sarl="v8"):  # the packed SARL records run k_sarl_v8: compare with the same kernel's per-array form
             envs = [BatchedEnviron(variant, E, V, M, seed=5, **over) for _ in range(3)]
         for e in envs:
             e.make_new_game(); e.renew_positions(); e.compute_parms()
@@ -484,10 +484,10 @@ def test_fused_sarl_driver_step_is_bit_identical_to_the_three_calls(V, M, inject
     """risvec_step_sarl_fused against map_actions -> step_sarl -> observe on a twin env ((12, 48): a shape the
     fused kernel does not take runs the three kernels from the one call)."""
     from ris_vec_marl_b200 import BatchedEnviron
-    from tests.gpu_backend import sarl_path
+    from tests.gpu_backend import kernel_paths
 
     E = 70
-    with sarl_path("mma"):   # both twins on the tensor-core kernel (the fused form lives in k_sarl_mma)
+    with kernel_paths(sarl="mma"):   # both twins on the tensor-core kernel (the fused form lives in k_sarl_mma)
         envs = [BatchedEnviron("sarl", E, V, M, seed=21) for _ in range(2)]
     for env in envs:
         env.make_new_game(); env.renew_positions(); env.compute_parms()
@@ -511,20 +511,13 @@ def test_attached_statistics_accumulator_equals_shard_stats(variant, path, kerne
     """risvec_attach_stats_accumulator: the statistics pass folded into the rollout (k_sarl_mma_tma / k_marl_tma add
     their last step's sums in the kernel tail; other kernels are followed by k_shard_stats) gives what a
     shard_stats() call after every rollout gives (float64 sums of the same float32 values: order only)."""
-    import os
-
     from ris_vec_marl_b200 import BatchedEnviron, encode_groups, marl_yaml_overrides
-    from tests.gpu_backend import sarl_path
+    from tests.gpu_backend import kernel_paths
 
     V, M, T = 8, 40, 40
-    old = os.environ.get("RISVEC_MARL_PATH")
-    os.environ["RISVEC_MARL_PATH"] = path if variant == "marl" else "tma"
-    try:
-        with sarl_path(path if variant == "sarl" else "auto"):
-            over = marl_yaml_overrides() if variant == "marl" else {}
-            envs = [BatchedEnviron(variant, E, V, M, seed=9, **over) for _ in range(2)]
-    finally:
-        os.environ.pop("RISVEC_MARL_PATH", None) if old is None else os.environ.__setitem__("RISVEC_MARL_PATH", old)
+    with kernel_paths(sarl=path if variant == "sarl" else "auto", marl=path if variant == "marl" else "tma"):
+        over = marl_yaml_overrides() if variant == "marl" else {}
+        envs = [BatchedEnviron(variant, E, V, M, seed=9, **over) for _ in range(2)]
     rng = np.random.default_rng(5)
     for env in envs:
         env.make_new_game(); env.renew_positions(); env.compute_parms()

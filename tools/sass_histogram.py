@@ -13,7 +13,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 LIB = os.path.join(ROOT, "ris_vec_marl_b200", "librisvec.so")
 KERNELS = [("k_sarl_mma_tma<5>", r"k_sarl_mma_tmaILi5E"), ("k_sarl_mma<5,false>", r"k_sarl_mmaILi5ELb0E"),
            ("k_sarl_umma<8>", r"k_sarl_ummaILi8E"), ("k_sarl_mma_big<8>", r"k_sarl_mma_bigILi8E"), ("k_marl_tma", r"k_marl_tma"),
-           ("k_sarl_v8<5,...,packed>", r"k_sarl_v8ILi5ELb1ELb1ELb1ELb1E"), ("k_marl_v8<true,false>", r"k_marl_v8ILb1ELb0ELb0E"),
+           ("k_sarl_v8<5,...,packed>", r"k_sarl_v8ILi5ELb1ELb1ELb1EE"), ("k_marl_v8<true,false>", r"k_marl_v8ILb1ELb0ELb0E"),
            ("k_sarl_cascade2<32,32,8>", r"k_sarl_cascade2ILi32ELi32ELi8E"), ("k_replay_store_flat<1>", r"k_replay_store_flatILi1E")]
 MARK = ("HMMA", "UTMALDG", "UTMASTG", "SYNCS", "UBLKCP", "FFMA2", "FMUL2", "FADD2", "DADD", "DFMA", "DMUL", "MUFU", "SHFL", "LDS", "STS",
         "LDG", "STG", "BAR", "UTCHMMA", "UTCBAR", "LDTM", "STTM")
