@@ -464,6 +464,36 @@ int risvec_shard_stats(risvec_env_t* env, double* out, int accumulate, void* str
 int risvec_attach_stats_accumulator(risvec_env_t* env, double* slots);
 int risvec_collect_stats(risvec_env_t* env, double* slots, double* out, int accumulate, void* stream);
 
+/* Per-env step parameters: the reference drivers write these attributes on each env object between episodes, so a
+ * batch of envs can run each env with its own power budget, noise, arrival rate and reward weights (domain
+ * randomisation, one launch for a whole parameter sweep, a new value for the next episode of one env only).
+ * `table` [E, RISVEC_ENVP_COLS] f64, row-major, 8-byte aligned, a device pointer on the handle's device, owned by the
+ * caller; NULL detaches.  While it is attached, every kernel that reads one of these parameters reads row e for env e
+ * instead of the handle's value (risvec_params_t): MARL reads columns 0-9 (risvec_rollout_marl, the fused step,
+ * risvec_pair_noma / _episodes: P_MAX and NOISE_POWER in the QoS test); SARL reads BANDWIDTH, RATE and columns 10-13;
+ * the other columns are ignored.  The table is read at each launch and never copied: rewrite it between launches,
+ * also inside a captured CUDA graph (the pointer stays fixed).  Rows are not validated, as the reference does not
+ * validate its attributes.  While a table is attached the tensor-core kernels with TMA or tcgen05 (k_marl_tma,
+ * k_sarl_mma_tma, k_sarl_umma, k_sarl_mma_big) and k_sarl_v8 are not chosen, and the packed-record entry points
+ * (risvec_rollout_*_packed*) return RISVEC_ERR_UNSUPPORTED.
+ * Every other parameter stays per handle and comes from risvec_params_t:
+ *   time_slow, time_fast   - the time base of the episode clock and of every step;
+ *   map, lanes, data_buf_size - positions and reset draws are per handle;
+ *   channel_model and its 3GPP knobs (fc_GHz, shadow_std_*, rician_K_dB, veh_ant_gain) - the episode-start kernels;
+ *   cpu_share_floor, power_scale - the action mapping reads them;
+ *   reward_clip, qos_enable, cycles_per_bit, MARL k - folded into per-handle constants of the step;
+ *   SARL k, L      - they enter the step through cbrt, evaluated once per handle;
+ *   R_min_bpsHz    - the pairing's SINR threshold is found on the host by bisection over host log2; a device twin
+ *                    of that bisection would not be bit-identical. */
+enum risvec_env_param {
+    RISVEC_ENVP_P_MAX = 0, RISVEC_ENVP_NOISE_POWER, RISVEC_ENVP_BANDWIDTH, RISVEC_ENVP_RATE,
+    RISVEC_ENVP_F_LOCAL_MAX, RISVEC_ENVP_F_EDGE_MAX, RISVEC_ENVP_W_D, RISVEC_ENVP_W_E,
+    RISVEC_ENVP_QOS_PENALTY, RISVEC_ENVP_D_MAX_S,
+    RISVEC_ENVP_T_FACTOR1, RISVEC_ENVP_T_FACTOR2, RISVEC_ENVP_PENALTY1, RISVEC_ENVP_PENALTY2,
+    RISVEC_ENVP_COLS
+};
+int risvec_attach_env_params(risvec_env_t* env, const double* table);
+
 /* Per-episode statistics of staggered episodes: per-env running sums on the device and a log of completed episodes.
  * n_user = V for MARL, 0 for SARL.  All memory is owned by the caller.
  * running [E, RISVEC_EPLOG_RUN_COLS(n_user)] f64, zero-filled by the caller, one row per env:

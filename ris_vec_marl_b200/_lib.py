@@ -53,6 +53,10 @@ FIELDS = ("pos_x", "pos_y", "dir", "vel", "dist", "angle", "amp", "theta_re", "t
           "reward", "mec_queue_cycles", "stats", "last_power_W", "step_ctr",
           "V2I_Shadowing", "pair_hist", "unpaired_streak", "pair_tau", "pair_k", "pair_mask", "pair_rounds",
           "noma_partner", "noma_ngroups", "noma_pairs", "noma_npairs", "ep_step", "ep_index")
+# per-env step parameter table (risvec_attach_env_params): the reference attribute of each RISVEC_ENVP_* column,
+# in enum order
+ENV_PARAM_COLUMNS = ("P_max", "noise_power", "bandwidth", "rate", "f_local_max", "f_edge_max", "w_d", "w_e",
+                     "qos_penalty", "D_max_s", "t_factor1", "t_factor2", "penalty1", "penalty2")
 PAIR_MAX_V = 12
 # stage bits of risvec_begin_episode / risvec_episode_tick (RISVEC_EP_*), in the order the stages run
 EP_STAGES = {"reset": 1, "positions": 2, "channel": 4, "pairing": 8}
@@ -197,6 +201,7 @@ EXPORTS = {
     "risvec_episode_accumulate": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int64,
                                             C.c_void_p, C.c_void_p]),
     "risvec_attach_stats_accumulator": (C.c_int, [C.c_void_p, C.c_void_p]),
+    "risvec_attach_env_params": (C.c_int, [C.c_void_p, C.c_void_p]),
     "risvec_collect_stats": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     "risvec_shared_buffer_create": (C.c_int, [C.c_int, C.c_uint64, C.POINTER(C.c_void_p), C.c_char_p]),
     "risvec_shared_buffer_open": (C.c_int, [C.c_int, C.c_char_p, C.POINTER(C.c_void_p)]),

@@ -13,8 +13,8 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import (CHANNEL, EP_STAGES, FIELDS, NSTAT, STAT_COLUMNS, VARIANT, EpisodeSchedule, MarlOut, Pairing,
-                   PairSchedule, Params, SarlOut, check)
+from ._lib import (CHANNEL, ENV_PARAM_COLUMNS, EP_STAGES, FIELDS, NSTAT, STAT_COLUMNS, VARIANT, EpisodeSchedule,
+                   MarlOut, Pairing, PairSchedule, Params, SarlOut, check)
 
 _PARAM_NAMES = {n for n, _ in Params._fields_} - {"_pad0"}
 _PAIRING_NAMES = {n for n, _ in Pairing._fields_}
@@ -113,6 +113,7 @@ class BatchedEnviron:
         for name in ("pair_hist", "pair_mask"):
             self._views[name] = self._views[name].view(self.E, self.V, self.V)
         self.pairing = default_pairing(self.V)
+        self.env_params = None  # the attached per-env parameter table (attach_env_params)
 
     # ------------------------------------------------------------------ params
     def _set_lanes(self, name, vals):
@@ -133,9 +134,61 @@ class BatchedEnviron:
             setattr(self.params, k, type(getattr(self.params, k))(v))
 
     def set_params(self, **kw):
-        """Attribute writes of the reference drivers (marl_train_bcd.py:563-594,750-779)."""
+        """Attribute writes of the reference drivers (marl_train_bcd.py:563-594,750-779), for every env of the handle.
+        While a per-env table is attached (`attach_env_params`), its columns win for the parameters in
+        `ENV_PARAM_COLUMNS`: the steps read those from the table, not from the values set here."""
         self._apply(kw)
         check(self._lib.risvec_set_params(self._h, C.byref(self.params)))
+
+    def attach_env_params(self, attach=True, table=None):
+        """Per-env step parameters (`risvec_attach_env_params`): each env gets its own value of every parameter in
+        `ENV_PARAM_COLUMNS` (power budget, noise, bandwidth, arrival rate, CPU / MEC speeds, reward weights).
+
+        Allocates `self.env_params`, a float64 [E, len(ENV_PARAM_COLUMNS)] device tensor with every row filled from
+        the current `self.params`, attaches it and returns it.  `table` attaches the caller's tensor instead, as it is
+        (for example the rows of this shard of a global table); anything but a contiguous float64 tensor of that shape
+        on this device is refused.  The library reads the table at every launch and never copies it: rewrite it with
+        `set_env_params` or torch ops between steps, also inside a captured CUDA graph.  Rows are not validated.
+        `attach=False` detaches the table and drops it (every env reads `self.params` again).  Attaching while a table
+        is attached raises: a CUDA graph captured earlier holds the attached tensor's address, so a new tensor would
+        silently split the graph from `set_env_params`.  Detach first, or rewrite the attached table in place."""
+        if not attach:
+            check(self._lib.risvec_attach_env_params(self._h, self._p(None)))
+            self.env_params = None
+            return None
+        if self.env_params is not None:
+            raise RuntimeError("a per-env parameter table is already attached: attach_env_params(False) first, or "
+                               "write it in place with set_env_params")
+        shape = (self.E, len(ENV_PARAM_COLUMNS))
+        if table is None:
+            row = [float(getattr(self.params, n)) for n in ENV_PARAM_COLUMNS]
+            table = torch.tensor(row, dtype=torch.float64, device=self.device).repeat(self.E, 1).contiguous()
+        else:
+            self._check("table", table, torch.float64, shape, self.device)
+        check(self._lib.risvec_attach_env_params(self._h, self._p(table)))
+        self.env_params = table
+        return table
+
+    def set_env_params(self, **cols):
+        """Write columns of the attached per-env table in place, by reference name (`P_max=`, `rate=`, `w_d=`, ...):
+        each value is a Python scalar (every env) or a float64 [E] tensor on this device (anything else is refused, not
+        converted: a float32 tensor would round the values).  No host synchronisation, so the call can be captured in
+        a CUDA graph.  Names outside `ENV_PARAM_COLUMNS` raise, per-handle parameters included (those go through
+        `set_params`)."""
+        table = self.env_params
+        if table is None:
+            raise RuntimeError("attach_env_params() first")
+        for name, v in cols.items():
+            if name not in ENV_PARAM_COLUMNS:
+                why = "a per-handle parameter: use set_params" if name in _PARAM_NAMES else "not a parameter"
+                raise ValueError(f"{name!r} is {why}; per-env columns are {ENV_PARAM_COLUMNS}")
+            col = table[:, ENV_PARAM_COLUMNS.index(name)]
+            if isinstance(v, torch.Tensor):
+                if tuple(v.shape) != (self.E,) or v.device != self.device or v.dtype != torch.float64:
+                    raise ValueError(f"{name} must be a float64 [{self.E}] tensor on {self.device}")
+                col.copy_(v)
+            else:
+                col.fill_(float(v))
 
     def get_param(self, name):
         return getattr(self.params, name)
@@ -626,13 +679,16 @@ class BatchedEnviron:
 
     def state_dict(self):
         """Everything a resumed run needs to CONTINUE this one: the state arena, the host-side call counters
-        that key the on-device Philox draws, the scalar parameters and the pairing knobs."""
+        that key the on-device Philox draws, the scalar parameters, the pairing knobs and, when one is attached, the
+        per-env parameter table (`"_env_params"`).  `load_state_dict` of a state without a table detaches one."""
         ctr = (C.c_uint64 * 3)()
         check(self._lib.risvec_get_rng_counters(self._h, ctr))
         sd = {k: v.clone() for k, v in self._views.items()}
         sd["_rng_counters"] = [int(x) for x in ctr]
         sd["_params"] = bytes(self.params)
         sd["_pairing"] = bytes(self.pairing)
+        if self.env_params is not None:
+            sd["_env_params"] = self.env_params.clone()
         return sd
 
     def load_state_dict(self, sd):
@@ -646,3 +702,12 @@ class BatchedEnviron:
             check(self._lib.risvec_set_params(self._h, C.byref(self.params)))
         if "_pairing" in sd:
             C.memmove(C.byref(self.pairing), sd["_pairing"], C.sizeof(Pairing))
+        if "_env_params" in sd:  # the per-env table: copied into the attached one (a captured graph keeps its pointer)
+            t = sd["_env_params"]
+            if tuple(t.shape) != (self.E, len(ENV_PARAM_COLUMNS)) or t.dtype != torch.float64:
+                raise ValueError(f"_env_params must be float64 [{self.E}, {len(ENV_PARAM_COLUMNS)}]")
+            if self.env_params is None:
+                self.attach_env_params()
+            self.env_params.copy_(t.to(self.device))
+        elif self.env_params is not None:  # saved without a table: every env follows the saved params again
+            self.attach_env_params(False)

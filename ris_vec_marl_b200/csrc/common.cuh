@@ -76,6 +76,41 @@ __host__ __device__ inline uint4 philox4x32_10(uint4 c, uint2 k) {
     return c;
 }
 
+// Per-env step parameters (risvec_attach_env_params).  A kernel instantiated with PE = true calls one of these at
+// entry on its by-value params with row e of the table (k_sarl_mma reads the row at each use instead, below): every
+// later expression then reads the env's value exactly as the PE = false instantiation reads the handle's, so a table
+// whose rows equal the params changes no bit.
+__device__ __forceinline__ const double* env_param_row(const double* __restrict__ table, long long e) {
+    return table + e * RISVEC_ENVP_COLS;
+}
+__device__ __forceinline__ void env_params_marl(risvec_params_t& p, const double* __restrict__ row) {
+    p.P_max = __ldg(row + RISVEC_ENVP_P_MAX);
+    p.noise_power = __ldg(row + RISVEC_ENVP_NOISE_POWER);
+    p.bandwidth = __ldg(row + RISVEC_ENVP_BANDWIDTH);
+    p.rate = __ldg(row + RISVEC_ENVP_RATE);
+    p.f_local_max = __ldg(row + RISVEC_ENVP_F_LOCAL_MAX);
+    p.f_edge_max = __ldg(row + RISVEC_ENVP_F_EDGE_MAX);
+    p.w_d = __ldg(row + RISVEC_ENVP_W_D);
+    p.w_e = __ldg(row + RISVEC_ENVP_W_E);
+    p.qos_penalty = __ldg(row + RISVEC_ENVP_QOS_PENALTY);
+    p.D_max_s = __ldg(row + RISVEC_ENVP_D_MAX_S);
+}
+// One column of a row read where it is used: the volatile load is not hoisted, so a kernel at the register cap of
+// its launch bounds keeps the row pointer live across its loop instead of the converted constants.
+__device__ __forceinline__ double env_param_at_use(const double* row, int col) {
+    double v;
+    asm volatile("ld.global.nc.f64 %0, [%1];" : "=d"(v) : "l"(row + col));
+    return v;
+}
+__device__ __forceinline__ void env_params_sarl(risvec_params_t& p, const double* __restrict__ row) {
+    p.bandwidth = __ldg(row + RISVEC_ENVP_BANDWIDTH);
+    p.rate = __ldg(row + RISVEC_ENVP_RATE);
+    p.t_factor1 = __ldg(row + RISVEC_ENVP_T_FACTOR1);
+    p.t_factor2 = __ldg(row + RISVEC_ENVP_T_FACTOR2);
+    p.penalty1 = __ldg(row + RISVEC_ENVP_PENALTY1);
+    p.penalty2 = __ldg(row + RISVEC_ENVP_PENALTY2);
+}
+
 __device__ inline uint4 rng_draw(const Dims& d, long long env_local, unsigned long long call, unsigned slot,
                                  unsigned kind) {
     unsigned long long ge = (unsigned long long)(d.env_base + env_local);

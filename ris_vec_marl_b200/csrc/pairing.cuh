@@ -416,13 +416,18 @@ struct PairCtx {
     }
 };
 
-template <int N>
-__global__ void k_pair_noma(Dims d, State s, PairArgs a) {
+// PE: NOISE_POWER and P_MAX of the QoS test from row e of the attached table `envp` (risvec_attach_env_params)
+template <int N, bool PE = false>
+__global__ void k_pair_noma(Dims d, State s, PairArgs a, const double* __restrict__ envp) {
     extern __shared__ __align__(16) unsigned char pair_smem[];
     constexpr int NN = N * N;
     const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5, wpc = blockDim.x >> 5;
     const long long e = (long long)blockIdx.x * wpc + wib;
     if (e >= d.E) return;    // whole warps leave together; only __syncwarp is used below
+    if constexpr (PE) {
+        a.noise = __ldg(env_param_row(envp, e) + RISVEC_ENVP_NOISE_POWER);
+        a.P_max = __ldg(env_param_row(envp, e) + RISVEC_ENVP_P_MAX);
+    }
     PairCtx<N> c;
     c.carve(pair_smem + pair_smem_bytes(N) * wib, lane);
     int recalc = a.recalc, fresh = a.fresh, topk = a.topk;

@@ -113,6 +113,7 @@ struct risvec_env {
     int stats_folded;         // the latest rollout kernel added its statistics itself
     unsigned char* ep_bits;   // [E] in the arena: stage bits of the current tick (episode clock, unfused shapes)
     int* ep_keys;             // [E] in the arena: episode index that keys the tick's draws (same)
+    const double* env_params; // attached per-env parameter table [E, RISVEC_ENVP_COLS] (risvec_attach_env_params) or null
 };
 
 struct risvec_replay {
@@ -185,6 +186,12 @@ int ensure_scratch(risvec_env* env, size_t bytes) {
     CUDA_TRY(cudaMalloc((void**)&env->scratch, bytes));
     env->scratch_bytes = bytes;
     return RISVEC_OK;
+}
+
+// f(std::true_type{}) while a per-env parameter table is attached (the PE instantiations), else f(std::false_type{})
+template <typename F>
+int dispatch_pe(const risvec_env* env, F&& f) {
+    return env->env_params ? f(std::true_type{}) : f(std::false_type{});
 }
 
 // f(std::integral_constant<int, VP>{}) for the least power of two VP >= V (V <= 32); dispatch_vp<8> starts at 8
@@ -265,15 +272,17 @@ SarlKernel choose_sarl(const risvec_env* env, const SarlArgs& a, int from = kSar
     const Dims& d = env->dims;
     const SarlPath p = env->ovr.sarl;
     if (a.in_rec) return kSarlV8;  // the caller checked the packed shape
+    // an attached per-env parameter table: only k_sarl_mma and the generic kernels have PE instantiations
+    const bool pe = env->env_params != nullptr;
     const bool mma = p == kPathAuto || p == kPathMmaLdg || p == kPathMmaSync;
     // tensor cores, one warp per env: V <= 8, M even, M <= 64
     const bool mma_fits = mma && d.V <= 8 && d.M % 2 == 0 && d.M <= 64 && (!a.raw || aligned8(a.raw));
-    if (from <= kSarlMmaTma && mma_fits && p != kPathMmaLdg && sarl_tma_covers(d, a)) return kSarlMmaTma;
+    if (from <= kSarlMmaTma && mma_fits && !pe && p != kPathMmaLdg && sarl_tma_covers(d, a)) return kSarlMmaTma;
     if (from <= kSarlMma && mma_fits) return kSarlMma;
-    const bool big = mma && p != kPathMmaLdg && sarl_big_covers(d, a);
+    const bool big = mma && !pe && p != kPathMmaLdg && sarl_big_covers(d, a);
     if (from <= kSarlUmma && big && p != kPathMmaSync) return kSarlUmma;
     if (from <= kSarlMmaBig && big && p == kPathMmaSync) return kSarlMmaBig;
-    if (d.V <= 8 && d.M <= 40 && p != kPathGeneric) return kSarlV8;  // elements split over the env's 8 lanes
+    if (d.V <= 8 && d.M <= 40 && p != kPathGeneric && !pe) return kSarlV8;  // elements split over the env's 8 lanes
     return d.M <= 40 ? kSarlRollout : kSarlCascade;
 }
 
@@ -303,13 +312,19 @@ int launch_sarl_mma_tma(risvec_env* env, const SarlArgs& a, cudaStream_t st, boo
 }
 
 // tensor cores, LDG (sarl_mma.cuh): one warp per env, 4 envs per block; KT k-tiles of 8 elements, M <= 8 KT
+// [per-env table][fused][KT]
 int launch_sarl_mma(risvec_env* env, const SarlArgs& a, cudaStream_t st) {
     using Kern = decltype(&k_sarl_mma<1>);
-    static const Kern kerns[2][5] = {{k_sarl_mma<1>, k_sarl_mma<2>, k_sarl_mma<3>, k_sarl_mma<5>, k_sarl_mma<8>},
-                                     {k_sarl_mma<1, true>, k_sarl_mma<2, true>, k_sarl_mma<3, true>,
-                                      k_sarl_mma<5, true>, k_sarl_mma<8, true>}};
+    static const Kern kerns[2][2][5] = {
+        {{k_sarl_mma<1>, k_sarl_mma<2>, k_sarl_mma<3>, k_sarl_mma<5>, k_sarl_mma<8>},
+         {k_sarl_mma<1, true>, k_sarl_mma<2, true>, k_sarl_mma<3, true>, k_sarl_mma<5, true>, k_sarl_mma<8, true>}},
+        {{k_sarl_mma<1, false, true>, k_sarl_mma<2, false, true>, k_sarl_mma<3, false, true>,
+          k_sarl_mma<5, false, true>, k_sarl_mma<8, false, true>},
+         {k_sarl_mma<1, true, true>, k_sarl_mma<2, true, true>, k_sarl_mma<3, true, true>, k_sarl_mma<5, true, true>,
+          k_sarl_mma<8, true, true>}}};
     const int M = env->dims.M, kt = M <= 8 ? 0 : M <= 16 ? 1 : M <= 24 ? 2 : M <= 40 ? 3 : 4;
-    kerns[a.raw != nullptr][kt]<<<(env->dims.E + 3) / 4, 128, 0, st>>>(env->dims, env->st, env->params, a);
+    kerns[env->env_params != nullptr][a.raw != nullptr][kt]<<<(env->dims.E + 3) / 4, 128, 0, st>>>(
+        env->dims, env->st, env->params, a, env->env_params);
     return check_step_launch(env, "k_sarl_mma");
 }
 
@@ -376,10 +391,13 @@ int launch_sarl_cfg(risvec_env* env, const SarlArgs& a_in, cudaStream_t st) {
     const size_t MS = (size_t)((env->dims.M + 4 * WPE + 7) / 4) * 4;  // must match the kernel
     if constexpr (WPE == 1) {  // one warp per env group: fused step kernel
         const size_t smem = 6 * EPW * MS * sizeof(float);
-        auto kern = k_sarl_rollout<VP, MPL, WPE>;
-        if (smem > 48 * 1024) CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        kern<<<blocks, 32 * WPE, smem, st>>>(env->dims, env->st, env->params, a);
-        return check_step_launch(env, "k_sarl_rollout");
+        return dispatch_pe(env, [&](auto pe) {
+            auto kern = k_sarl_rollout<VP, MPL, WPE, decltype(pe)::value>;
+            if (smem > 48 * 1024)
+                CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            kern<<<blocks, 32 * WPE, smem, st>>>(env->dims, env->st, env->params, a, env->env_params);
+            return check_step_launch(env, "k_sarl_rollout");
+        });
     } else {
         // several warps per env (large M): cascade kernel over (env group, time chunk) -> |S|^2 scratch,
         // then the per-vehicle scan kernel
@@ -395,8 +413,13 @@ int launch_sarl_cfg(risvec_env* env, const SarlArgs& a_in, cudaStream_t st) {
         kern<<<dim3(blocks, (a.T + chunk - 1) / chunk), 32 * WPE, smem2, st>>>(env->dims, env->st, a);
         if (int rc = check_launch(env, "k_sarl_cascade2")) return rc;
         const long long total = (long long)E * VP;
-        k_sarl_scan<VP><<<(int)((total + 127) / 128), 128, 0, st>>>(env->dims, env->st, env->params, a);
-        if (int rc = check_launch(env, "k_sarl_scan")) return rc;
+        // the scan reads the step parameters: the cascade only forms |S|^2
+        if (int rc = dispatch_pe(env, [&](auto pe) {
+                k_sarl_scan<VP, decltype(pe)::value><<<(int)((total + 127) / 128), 128, 0, st>>>(
+                    env->dims, env->st, env->params, a, env->env_params);
+                return check_launch(env, "k_sarl_scan");
+            }))
+            return rc;
         env->step_kernel = "k_sarl_cascade2+k_sarl_scan";
         return RISVEC_OK;
     }
@@ -460,7 +483,9 @@ MarlKernel choose_marl(const risvec_env* env, const MarlArgs& a, int from = kMar
     // 4 envs per warp, lane = vehicle
     const bool v8 = env->dims.V <= 8 && !env->ovr.force_generic && !a.out.stats && !a.out.last_power &&
                     (!a.raw || aligned8(a.raw));
-    if (from <= kMarlTma && v8 && !env->ovr.marl_v8 && marl_tma_covers(env->dims, a)) return kMarlTma;
+    // an attached per-env parameter table: k_marl_tma has no PE instantiation
+    if (from <= kMarlTma && v8 && !env->ovr.marl_v8 && !env->env_params && marl_tma_covers(env->dims, a))
+        return kMarlTma;
     return v8 ? kMarlV8 : kMarlRollout;
 }
 
@@ -487,14 +512,21 @@ int launch_marl_tma(risvec_env* env, const MarlArgs& a_in, cudaStream_t st, bool
 
 int launch_marl_v8(risvec_env* env, const MarlArgs& a, cudaStream_t st) {
     const int warps = (env->dims.E + 3) / 4;
-    if (a.in_rec)
-        k_marl_v8<true, true><<<warps, 32, 0, st>>>(env->dims, env->st, env->params, a);
+    const double* const ep = env->env_params;
+    if (a.in_rec)  // the packed entry points refuse an attached table
+        k_marl_v8<true, true><<<warps, 32, 0, st>>>(env->dims, env->st, env->params, a, nullptr);
+    else if (a.raw && ep)
+        k_marl_v8<false, false, true, true><<<warps, 32, 0, st>>>(env->dims, env->st, env->params, a, ep);
     else if (a.raw)  // action mapping in the prologue, marl_get_state of the new state in the epilogue
-        k_marl_v8<false, false, true><<<warps, 32, 0, st>>>(env->dims, env->st, env->params, a);
+        k_marl_v8<false, false, true><<<warps, 32, 0, st>>>(env->dims, env->st, env->params, a, nullptr);
+    else if (marl_full(a) && ep)
+        k_marl_v8<true, false, false, true><<<warps, 32, 0, st>>>(env->dims, env->st, env->params, a, ep);
     else if (marl_full(a))
-        k_marl_v8<true, false><<<warps, 32, 0, st>>>(env->dims, env->st, env->params, a);
+        k_marl_v8<true, false><<<warps, 32, 0, st>>>(env->dims, env->st, env->params, a, nullptr);
+    else if (ep)
+        k_marl_v8<false, false, false, true><<<warps, 32, 0, st>>>(env->dims, env->st, env->params, a, ep);
     else
-        k_marl_v8<false, false><<<warps, 32, 0, st>>>(env->dims, env->st, env->params, a);
+        k_marl_v8<false, false><<<warps, 32, 0, st>>>(env->dims, env->st, env->params, a, nullptr);
     return check_step_launch(env, "k_marl_v8");
 }
 
@@ -506,8 +538,11 @@ int launch_marl(risvec_env* env, const MarlArgs& a, cudaStream_t st) {
             return dispatch_vp(env->dims.V, [&](auto vp) {
                 constexpr int VP = decltype(vp)::value;
                 const long long total = (long long)env->dims.E * VP;
-                k_marl_rollout<VP><<<(int)((total + 127) / 128), 128, 0, st>>>(env->dims, env->st, env->params, a);
-                return check_step_launch(env, "k_marl_rollout");
+                return dispatch_pe(env, [&](auto pe) {
+                    k_marl_rollout<VP, decltype(pe)::value><<<(int)((total + 127) / 128), 128, 0, st>>>(
+                        env->dims, env->st, env->params, a, env->env_params);
+                    return check_step_launch(env, "k_marl_rollout");
+                });
             });
         bool launched = false;
         const int rc = launch_marl_tma(env, a, st, &launched);
@@ -863,6 +898,9 @@ int check_sarl_args(const risvec_env* env, int T, const void* action, const void
     return RISVEC_OK;
 }
 // ---- packed record layout (include/risvec.h): one input / one output stream per rollout
+const char kPackedEnvParamsMsg[] =
+    "packed records take no per-env parameter table: a table is attached (risvec_attach_env_params); detach it or use "
+    "the per-array entry points";
 int check_sarl_packed_args(const risvec_env* env, int T, const void* in_rec, const void* out_rec, const void* reward) {
     if (!env) return fail(RISVEC_ERR_INVALID, "NULL handle");
     if (env->dims.variant != RISVEC_VARIANT_SARL) return fail(RISVEC_ERR_INVALID, "handle is not a SARL env");
@@ -870,6 +908,7 @@ int check_sarl_packed_args(const risvec_env* env, int T, const void* in_rec, con
     if (env->dims.V != 8 || env->dims.E % 4 != 0 || (env->dims.M != 16 && env->dims.M != 40))
         return fail(RISVEC_ERR_UNSUPPORTED, "packed SARL records need V == 8, E %% 4 == 0 and M in {16, 40} "
                     "(got V = %d, E = %d, M = %d)", env->dims.V, env->dims.E, env->dims.M);
+    if (env->env_params) return fail(RISVEC_ERR_UNSUPPORTED, "%s", kPackedEnvParamsMsg);
     return RISVEC_OK;
 }
 int check_marl_packed_args(const risvec_env* env, int T, const void* in_rec, const void* partner, const void* ngroups,
@@ -881,6 +920,7 @@ int check_marl_packed_args(const risvec_env* env, int T, const void* in_rec, con
     if (env->dims.V != 8 || env->dims.E % 4 != 0)
         return fail(RISVEC_ERR_UNSUPPORTED, "packed MARL records need V == 8 and E %% 4 == 0 (got V = %d, E = %d)",
                     env->dims.V, env->dims.E);
+    if (env->env_params) return fail(RISVEC_ERR_UNSUPPORTED, "%s", kPackedEnvParamsMsg);
     return RISVEC_OK;
 }
 }  // namespace
@@ -1289,9 +1329,13 @@ static int pair_noma_launch(risvec_env* env, const risvec_pairing_t* cfg, PairAr
     const size_t per = pair_smem_bytes(V);
     const int wpc = V <= 8 ? 4 : (V <= 10 ? 2 : 1);
     const int blocks = (env->dims.E + wpc - 1) / wpc;
+    const double* const ep = env->env_params;  // per-env noise_power / P_max of the QoS test
     switch (V) {
-#define RISVEC_PAIR_CASE(n) \
-    case n: k_pair_noma<n><<<blocks, 32 * wpc, per * wpc, (cudaStream_t)stream>>>(env->dims, env->st, a); break;
+#define RISVEC_PAIR_CASE(n)                                                                                    \
+    case n:                                                                                                    \
+        if (ep) k_pair_noma<n, true><<<blocks, 32 * wpc, per * wpc, (cudaStream_t)stream>>>(env->dims, env->st, a, ep); \
+        else k_pair_noma<n><<<blocks, 32 * wpc, per * wpc, (cudaStream_t)stream>>>(env->dims, env->st, a, nullptr);     \
+        break;
         RISVEC_PAIR_CASE(1) RISVEC_PAIR_CASE(2) RISVEC_PAIR_CASE(3) RISVEC_PAIR_CASE(4) RISVEC_PAIR_CASE(5)
         RISVEC_PAIR_CASE(6) RISVEC_PAIR_CASE(7) RISVEC_PAIR_CASE(8) RISVEC_PAIR_CASE(9) RISVEC_PAIR_CASE(10)
         RISVEC_PAIR_CASE(11) RISVEC_PAIR_CASE(12)
@@ -1731,6 +1775,25 @@ int risvec_episode_accumulate(risvec_env_t* env, double* running, const uint8_t*
     k_episode_accumulate<<<(env->dims.E + per - 1) / per, kEpLogThreads, 0, (cudaStream_t)stream>>>(env->dims, env->st,
                                                                                                     a);
     return check_launch(env, "k_episode_accumulate");
+}
+
+int risvec_attach_env_params(risvec_env_t* env, const double* table) {
+    if (!env) return fail(RISVEC_ERR_INVALID, "NULL handle");
+    if (table != nullptr) {
+        if (!aligned8(table)) return fail(RISVEC_ERR_INVALID, "the per-env parameter table must be 8-byte aligned");
+        cudaPointerAttributes at;
+        if (cudaPointerGetAttributes(&at, table) != cudaSuccess) {
+            cudaGetLastError();
+            return fail(RISVEC_ERR_INVALID, "the per-env parameter table is not a CUDA pointer");
+        }
+        if (at.type != cudaMemoryTypeDevice && at.type != cudaMemoryTypeManaged)
+            return fail(RISVEC_ERR_INVALID, "the per-env parameter table must be device memory");
+        if (at.device != env->device)
+            return fail(RISVEC_ERR_INVALID, "the per-env parameter table is on device %d, the handle on device %d",
+                        at.device, env->device);
+    }
+    env->env_params = table;
+    return RISVEC_OK;
 }
 
 int risvec_attach_stats_accumulator(risvec_env_t* env, double* slots) {

@@ -63,8 +63,10 @@ struct SarlMmaIn {     // inputs of one 8-step tile, as one lane needs them
 
 // KT = k-tiles of 8 RIS elements (M <= 8 KT, M even).  Block = 4 warps = 4 adjacent envs.
 // FUSED = the one-launch driver step (risvec_step_sarl_fused): inputs from the actor's raw row, observation out
-template <int KT, bool FUSED = false>
-__global__ void __launch_bounds__(128, 4) k_sarl_mma(Dims d, State s, risvec_params_t p, SarlArgs a) {
+// PE: per-env step parameters from the attached table `envp` (risvec_attach_env_params); unused without PE
+template <int KT, bool FUSED = false, bool PE = false>
+__global__ void __launch_bounds__(128, 4) k_sarl_mma(Dims d, State s, risvec_params_t p, SarlArgs a,
+                                                     const double* __restrict__ envp) {
     const int lane = threadIdx.x & 31, g = lane >> 2, tig = lane & 3;
     const int E = d.E, V = d.V, M = d.M, T = a.T;
     const int e = blockIdx.x * 4 + (threadIdx.x >> 5);
@@ -104,6 +106,16 @@ __global__ void __launch_bounds__(128, 4) k_sarl_mma(Dims d, State s, risvec_par
     const float invV = 1.0f / (float)V;
     const float lam = (float)p.rate;
     const double tf = p.time_fast;
+    // PE: the env's step parameters are read at each use from its row (env_param_at_use), in the expressions above
+    const double* const prow = PE ? env_param_row(envp, e) : nullptr;
+    auto at = [&](float handle_value, int col) -> float {
+        if constexpr (PE) return (float)env_param_at_use(prow, col);
+        else return handle_value;
+    };
+    auto c_dt_e = [&]() -> float {
+        if constexpr (PE) return (float)(p.time_fast * env_param_at_use(prow, RISVEC_ENVP_BANDWIDTH) * 1000.0);
+        else return c_dt;
+    };
 
     const size_t sM = (size_t)E * M, s2V = (size_t)E * 2 * V, sV = (size_t)E * V;
     const float* const ph_b = a.phase + (size_t)e * M + 2 * tig;
@@ -189,10 +201,10 @@ __global__ void __launch_bounds__(128, 4) k_sarl_mma(Dims d, State s, risvec_par
             const float re = __fadd_rn(accM[i], accX[i]), im = __fadd_rn(accM[2 + i], accX[2 + i]);
             const float g2 = __fmaf_rn(re, re, __fmul_rn(im, im));
             rate[i] = log1p_sfu(__fmul_rn(in.a0[i], __fmul_rn(coef, g2)));  // natural log, SARL:159
-            dt[i] = __fmul_rn(rate[i], c_dt);
+            dt[i] = __fmul_rn(rate[i], c_dt_e());
             dp[i] = __fmul_rn(cbrt_sfu(in.a1[i]), c_dp);                    // SARL:331
             arr[i] = in.arr[i];
-            if (ar_b == nullptr) arr[i] = (vact && ok[i]) ? draw_arrival(d, e, vc, step0 + t, lam) : 0;
+            if (ar_b == nullptr) arr[i] = (vact && ok[i]) ? draw_arrival(d, e, vc, step0 + t, at(lam, RISVEC_ENVP_RATE)) : 0;
             // steps past the end of the rollout are the identity of the recursion (DataBuf >= 0)
             dd[i] = ok[i] ? __dadd_rn((double)dt[i], (double)dp[i]) : 0.0;
             inc[i] = ok[i] ? __dmul_rn(__dmul_rn((double)arr[i], tf), 1000.0) : 0.0;
@@ -221,8 +233,10 @@ __global__ void __launch_bounds__(128, 4) k_sarl_mma(Dims d, State s, risvec_par
             const float overp = neg ? __fsub_rn(in.a1[i], __fmul_rn(__fmul_rn(b, b), b)) : 0.f;  // SARL:336-339
             const float overd = neg ? (float)(-raw) : 0.f;
             const double nb = neg ? 0.0 : raw;
-            const float base = __fsub_rn(-__fmul_rn(t1, __fadd_rn(in.a0[i], in.a1[i])), __fmul_rn(t2, (float)nb));
-            const float pen = (nb > 0.0) ? pen1 : ((overd > 2.0f) ? pen2 : 0.f);  // SARL:343-352
+            const float base = __fsub_rn(-__fmul_rn(at(t1, RISVEC_ENVP_T_FACTOR1), __fadd_rn(in.a0[i], in.a1[i])),
+                                         __fmul_rn(at(t2, RISVEC_ENVP_T_FACTOR2), (float)nb));
+            const float pen = (nb > 0.0) ? at(pen1, RISVEC_ENVP_PENALTY1)
+                                         : ((overd > 2.0f) ? at(pen2, RISVEC_ENVP_PENALTY2) : 0.f);  // SARL:343-352
             float ru = vact ? __fsub_rn(base, pen) : 0.f;
             ru += __shfl_xor_sync(kFull, ru, 4);   // mean over the vehicles: same tree as seg_sum<8>
             ru += __shfl_xor_sync(kFull, ru, 8);

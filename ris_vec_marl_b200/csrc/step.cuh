@@ -60,12 +60,15 @@ __device__ inline int draw_arrival(const Dims& d, int e, int v, long long step, 
 // ---------------------------------------------------------------------------------------
 // MARL step (row a11 + a10 of SURVEY.md 8a)
 // ---------------------------------------------------------------------------------------
-template <int VP>
-__global__ void __launch_bounds__(128) k_marl_rollout(Dims d, State s, risvec_params_t p, MarlArgs a) {
+// PE: per-env step parameters from the attached table `envp` (risvec_attach_env_params); unused without PE
+template <int VP, bool PE = false>
+__global__ void __launch_bounds__(128) k_marl_rollout(Dims d, State s, risvec_params_t p, MarlArgs a,
+                                                      const double* __restrict__ envp) {
     const int gtid = blockIdx.x * blockDim.x + threadIdx.x;
     const int lane = threadIdx.x & 31;
     const int e = gtid / VP, v = gtid % VP;
     const int E = d.E, V = d.V;
+    if constexpr (PE) env_params_marl(p, env_param_row(envp, min(e, E - 1)));
     const bool env_ok = e < E;
     const bool act = env_ok && v < V;
     const size_t ev = (size_t)e * V + v;
@@ -354,8 +357,10 @@ __device__ __noinline__ void phasor_f32(double x, float* re, float* im) {
 // k_sarl_scan below (several warps per env: the per-vehicle phase would be a serial section of
 // one warp per block and step).
 
-template <int VP, int MPL, int WPE>
-__global__ void __launch_bounds__(32 * WPE) k_sarl_rollout(Dims d, State s, risvec_params_t p, SarlArgs a) {
+// PE: per-env step parameters from the attached table `envp` (risvec_attach_env_params); unused without PE
+template <int VP, int MPL, int WPE, bool PE = false>
+__global__ void __launch_bounds__(32 * WPE) k_sarl_rollout(Dims d, State s, risvec_params_t p, SarlArgs a,
+                                                           const double* __restrict__ envp) {
     static_assert(MPL % 4 == 0, "elements are processed four at a time (LDS.128 + FFMA2 pairs)");
     constexpr int EPW = 32 / VP;  // envs per warp (= per block)
     constexpr int NT = 32 * WPE;
@@ -378,6 +383,7 @@ __global__ void __launch_bounds__(32 * WPE) k_sarl_rollout(Dims d, State s, risv
     const int slice = (((M + WPE - 1) / WPE) + 3) & ~3;  // multiples of 4 keep the float4 quads aligned
     const int m0 = w * slice;
     const int m1 = min(M, m0 + slice);
+    if constexpr (PE) env_params_sarl(p, env_param_row(envp, min(e, E - 1)));
 
     // ---- geometry phasor table -> registers (float64 argument reduction), as element pairs
     float2 WX[MPL / 2], WY[MPL / 2];
@@ -728,11 +734,14 @@ __global__ void __launch_bounds__(32 * WPE, (WPE <= 8 && MPL <= 32) ? 16 / WPE :
 // Second half of the split SARL step for large M: per-vehicle queue update and reward
 // (SARL:327-358) from the |S_v|^2 the cascade kernel left in a.g2.  An env owns VP lanes of a
 // warp (lane = vehicle); inputs of step t + 1 are prefetched while step t computes.
-template <int VP>
-__global__ void __launch_bounds__(128) k_sarl_scan(Dims d, State s, risvec_params_t p, SarlArgs a) {
+// PE: as k_sarl_rollout
+template <int VP, bool PE = false>
+__global__ void __launch_bounds__(128) k_sarl_scan(Dims d, State s, risvec_params_t p, SarlArgs a,
+                                                   const double* __restrict__ envp) {
     const int gtid = blockIdx.x * blockDim.x + threadIdx.x;
     const int e = gtid / VP, v = gtid % VP;
     const int E = d.E, V = d.V, T = a.T;
+    if constexpr (PE) env_params_sarl(p, env_param_row(envp, min(e, E - 1)));
     const bool env_ok = e < E;
     const bool act = env_ok && v < V;
     const size_t ev = (size_t)min(e, E - 1) * V + min(v, V - 1);
@@ -1139,10 +1148,13 @@ struct MarlHeavy {
 };
 
 // FUSED = the one-launch driver step (risvec_step_marl_fused): actions from the actors' raw outputs, observation out
-template <bool FULL, bool PACKED, bool FUSED = false>
-__global__ void __launch_bounds__(32) k_marl_v8(Dims d, State s, risvec_params_t p, MarlArgs a) {
+// PE: per-env step parameters from the attached table `envp` (risvec_attach_env_params); unused without PE
+template <bool FULL, bool PACKED, bool FUSED = false, bool PE = false>
+__global__ void __launch_bounds__(32) k_marl_v8(Dims d, State s, risvec_params_t p, MarlArgs a,
+                                                const double* __restrict__ envp) {
     static_assert(!FUSED || (!FULL && !PACKED), "the fused driver step is a variant of the generic form");
     static_assert(!PACKED || FULL, "the packed record layout carries every stream");
+    static_assert(!PE || !PACKED, "packed records take no per-env parameter table");
     constexpr int RIN = RISVEC_MARL_IN_WORDS, ROUT = RISVEC_MARL_OUT_WORDS;
     const int lane = threadIdx.x & 31, el = lane >> 3, v = lane & 7;
     const int E = d.E, V = d.V, T = a.T;
@@ -1151,6 +1163,7 @@ __global__ void __launch_bounds__(32) k_marl_v8(Dims d, State s, risvec_params_t
     const int e = min(e_raw, E - 1), vc = min(v, V - 1);
     const bool act = PACKED || (env_ok && v < V);
     const size_t ev = (size_t)e * V + vc;
+    if constexpr (PE) env_params_marl(p, env_param_row(envp, e));
 
     double buf = act ? s.databuf[ev] : 0.0;
     const double g = act ? s.gains[ev] : 0.0;
