@@ -142,7 +142,8 @@ __global__ void __launch_bounds__(128, 4)
             asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
             issue(k + STAGES);
         }
-        // ---- state-independent part of my four steps (MARL:555-578)
+        // ---- state-independent part of my four steps (MARL:555-578); this step and the delays / reward below are also
+        // written out in k_marl_v8: shared helpers changed that kernel's code
         float P0[4], P1[4], rate[4], dt[4], flf[4];
         double cap[4], cl[4], inc[4], dd[4];
         bool ok[4];
@@ -164,24 +165,17 @@ __global__ void __launch_bounds__(128, 4)
             cap[i] = __dmul_rn(f_local, c.tf);
             flf[i] = (float)f_local;
             // local capacity in kbit = cap / den, correctly rounded (same FMA division as the step itself)
-            const double q0 = __dmul_rn(cap[i], c.rden);
-            cl[i] = __fma_rn(__fma_rn(-q0, c.den, cap[i]), c.rden, q0);
+            cl[i] = div_rn_fma(cap[i], c.den, c.rden);
             inc[i] = ok[i] ? __dmul_rn(__dmul_rn((double)arr[i], c.tf), 1000.0) : 0.0;
             dd[i] = ok[i] ? cl[i] + (double)dt[i] : 0.0;  // a step removes min(DataBuf, cl + data_t)
         }
         // ---- DataBuf at my first step: scan of the four-step maps over tig (identity steps past T)
         double xin;
         {
-            MaxPlus f = mp_then(mp_then(MaxPlus{inc[0] - dd[0], inc[0]}, MaxPlus{inc[1] - dd[1], inc[1]}),
-                                mp_then(MaxPlus{inc[2] - dd[2], inc[2]}, MaxPlus{inc[3] - dd[3], inc[3]}));
-            MaxPlus q{__shfl_up_sync(kFull, f.a, 1, 4), __shfl_up_sync(kFull, f.b, 1, 4)};
-            const MaxPlus f1 = mp_then(q, f);
-            if (tig >= 1) f = f1;
-            q = MaxPlus{__shfl_up_sync(kFull, f.a, 2, 4), __shfl_up_sync(kFull, f.b, 2, 4)};
-            const MaxPlus f2m = mp_then(q, f);
-            if (tig >= 2) f = f2m;
-            const MaxPlus ex{__shfl_up_sync(kFull, f.a, 1, 4), __shfl_up_sync(kFull, f.b, 1, 4)};
-            const MaxPlus all{__shfl_sync(kFull, f.a, 3, 4), __shfl_sync(kFull, f.b, 3, 4)};
+            MaxPlus ex, all;
+            mp_scan<4>(mp_then(mp_then(MaxPlus{inc[0] - dd[0], inc[0]}, MaxPlus{inc[1] - dd[1], inc[1]}),
+                               mp_then(MaxPlus{inc[2] - dd[2], inc[2]}, MaxPlus{inc[3] - dd[3], inc[3]})),
+                       tig, ex, all);
             const double xi = mp_apply(ex, buf);
             xin = tig == 0 ? buf : xi;
             buf = mp_apply(all, buf);
@@ -196,8 +190,7 @@ __global__ void __launch_bounds__(128, 4)
                 backlog[i] = cur;
                 bcyc[i] = __dmul_rn(__dmul_rn(cur, 1000.0), c.Cpb);
                 used[i] = fmin(cap[i], bcyc[i]);
-                const double q0 = __dmul_rn(used[i], c.rden);
-                ldone[i] = __fma_rn(__fma_rn(-q0, c.den, used[i]), c.rden, q0);
+                ldone[i] = div_rn_fma(used[i], c.den, c.rden);
                 const double remaining = fmax(0.0, __dsub_rn(cur, ldone[i]));
                 off[i] = fmin((double)dt[i], remaining);                                   // MARL:595-596
                 edge_in[i] = __dmul_rn(__dmul_rn(off[i], 1000.0), c.Cpb);                  // MARL:604
@@ -219,16 +212,10 @@ __global__ void __launch_bounds__(128, 4)
             double sa[4];
 #pragma unroll
             for (int i = 0; i < 4; ++i) sa[i] = ok[i] ? S[i] - c.edge_cap : 0.0;
-            MaxPlus f = mp_then(mp_then(MaxPlus{sa[0], 0.0}, MaxPlus{sa[1], 0.0}),
-                                mp_then(MaxPlus{sa[2], 0.0}, MaxPlus{sa[3], 0.0}));
-            MaxPlus q{__shfl_up_sync(kFull, f.a, 1, 4), __shfl_up_sync(kFull, f.b, 1, 4)};
-            const MaxPlus f1 = mp_then(q, f);
-            if (tig >= 1) f = f1;
-            q = MaxPlus{__shfl_up_sync(kFull, f.a, 2, 4), __shfl_up_sync(kFull, f.b, 2, 4)};
-            const MaxPlus f2m = mp_then(q, f);
-            if (tig >= 2) f = f2m;
-            const MaxPlus ex{__shfl_up_sync(kFull, f.a, 1, 4), __shfl_up_sync(kFull, f.b, 1, 4)};
-            const MaxPlus all{__shfl_sync(kFull, f.a, 3, 4), __shfl_sync(kFull, f.b, 3, 4)};
+            MaxPlus ex, all;
+            mp_scan<4>(mp_then(mp_then(MaxPlus{sa[0], 0.0}, MaxPlus{sa[1], 0.0}),
+                               mp_then(MaxPlus{sa[2], 0.0}, MaxPlus{sa[3], 0.0})),
+                       tig, ex, all);
             const double qi = mp_apply(ex, Q);
             qin = tig == 0 ? Q : qi;
             Q = mp_apply(all, Q);

@@ -75,7 +75,8 @@ __global__ void __launch_bounds__(128, 4) k_sarl_mma(Dims d, State s, risvec_par
     const int vc = min(g, V - 1);
     const size_t ev = (size_t)e * V + vc;
 
-    // ---- A operand: phasors of vehicle g at the elements m = 8 j + 2 tig + {0, 1} of every k-tile
+    // ---- A operand: phasors of vehicle g at the elements m = 8 j + 2 tig + {0, 1} of every k-tile (written out, as in
+    // k_sarl_mma_tma: a shared builder with the mask as an argument changed this kernel's code)
     // (fragment columns 2 tig, 2 tig + 1 hold element 8 j + 2 tig, columns 2 tig + 8, + 9 element
     //  8 j + 2 tig + 1: the same element order the B fragments below use)
     uint32_t Ah[KT][4], Al[KT][4];
@@ -99,9 +100,7 @@ __global__ void __launch_bounds__(128, 4) k_sarl_mma(Dims d, State s, risvec_par
     double buf = s.databuf[ev];  // replicated over the 4 lanes of vehicle g
     const float coef = (float)(s.amp[ev] / (kSigma * kSigma));  // SARL:157-159
     const long long step0 = s.step_ctr[e];
-    const float c_dt = (float)(p.time_fast * p.bandwidth * 1000.0);
-    const float c_dp = (float)(cbrt(1.0 / p.k) * p.time_fast / p.L / 1000.0);  // SARL:331
-    const float c_rev = (float)(1000.0 * p.L / p.time_fast * cbrt(p.k));        // SARL:318-319
+    const SarlConsts sc = sarl_consts(p);  // SARL:160, 318-319, 331
     const float t1 = (float)p.t_factor1, t2 = (float)p.t_factor2, pen1 = (float)p.penalty1, pen2 = (float)p.penalty2;
     const float invV = 1.0f / (float)V;
     const float lam = (float)p.rate;
@@ -114,7 +113,7 @@ __global__ void __launch_bounds__(128, 4) k_sarl_mma(Dims d, State s, risvec_par
     };
     auto c_dt_e = [&]() -> float {
         if constexpr (PE) return (float)(p.time_fast * env_param_at_use(prow, RISVEC_ENVP_BANDWIDTH) * 1000.0);
-        else return c_dt;
+        else return sc.c_dt;
     };
 
     const size_t sM = (size_t)E * M, s2V = (size_t)E * 2 * V, sV = (size_t)E * V;
@@ -202,7 +201,7 @@ __global__ void __launch_bounds__(128, 4) k_sarl_mma(Dims d, State s, risvec_par
             const float g2 = __fmaf_rn(re, re, __fmul_rn(im, im));
             rate[i] = log1p_sfu(__fmul_rn(in.a0[i], __fmul_rn(coef, g2)));  // natural log, SARL:159
             dt[i] = __fmul_rn(rate[i], c_dt_e());
-            dp[i] = __fmul_rn(cbrt_sfu(in.a1[i]), c_dp);                    // SARL:331
+            dp[i] = __fmul_rn(cbrt_sfu(in.a1[i]), sc.c_dp);                    // SARL:331
             arr[i] = in.arr[i];
             if (ar_b == nullptr) arr[i] = (vact && ok[i]) ? draw_arrival(d, e, vc, step0 + t, at(lam, RISVEC_ENVP_RATE)) : 0;
             // steps past the end of the rollout are the identity of the recursion (DataBuf >= 0)
@@ -222,14 +221,15 @@ __global__ void __launch_bounds__(128, 4) k_sarl_mma(Dims d, State s, risvec_par
             if (q < 3 && tig == q + 1) xin = x;
         }
         buf = x;
-        // ---- my two steps again from their true start value: overflow terms, reward, traces
+        // ---- my two steps again from their true start value: overflow terms, reward, traces.  (Not sarl_step: the
+        // step starts from the tile's dd / inc and reads the per-env values at use, under the 128-register cap.)
         double cur = xin;
 #pragma unroll
         for (int i = 0; i < 2; ++i) {
             const int t = t0 + 2 * tig + i;
             const double raw = __dsub_rn(cur, dd[i]);  // SARL:334
             const bool neg = raw < 0.0;
-            const float b = __fmul_rn((float)fmax(0.0, raw + (double)dp[i]), c_rev);
+            const float b = __fmul_rn((float)fmax(0.0, raw + (double)dp[i]), sc.c_rev);
             const float overp = neg ? __fsub_rn(in.a1[i], __fmul_rn(__fmul_rn(b, b), b)) : 0.f;  // SARL:336-339
             const float overd = neg ? (float)(-raw) : 0.f;
             const double nb = neg ? 0.0 : raw;
@@ -386,47 +386,6 @@ __device__ __forceinline__ void tma_store_2d(const void* tmap, uint32_t src, int
                  ::"l"(tmap), "r"(src), "r"(c0), "r"(c1) : "memory");
 }
 
-// max-plus affine map x -> max(x + a, b): the DataBuf step x -> max(x - d, 0) + inc is (inc - d, inc)
-struct MaxPlus {
-    double a, b;
-};
-__device__ __forceinline__ MaxPlus mp_then(const MaxPlus& f, const MaxPlus& g) {  // g after f
-    MaxPlus r;
-    r.a = f.a + g.a;
-    const double fb = f.b + g.a;
-    r.b = fb > g.b ? fb : g.b;
-    return r;
-}
-__device__ __forceinline__ double mp_apply(const MaxPlus& f, double x) {
-    const double y = x + f.a;
-    return y > f.b ? y : f.b;
-}
-
-// scalar constants of the step, formed on the host in float64 and rounded once: as kernel parameters they
-// sit in the constant bank and are used as instruction operands (no registers, no in-kernel conversions)
-struct SarlConsts {
-    float c_dt;    // time_fast * bandwidth * 1000        (SARL:160, data_t = rate * c_dt)
-    float c_dp;    // cbrt(1 / k) * time_fast / L / 1000  (SARL:331)
-    float c_rev;   // 1000 * L / time_fast * cbrt(k)      (SARL:318-319)
-    float nt1, nt2;  // -t_factor1, -t_factor2            (SARL:341-352)
-    float pen1, pen2;
-    float lam;     // Poisson arrival rate (on-device draws)
-    double tf;     // time_fast
-};
-inline SarlConsts sarl_consts(const risvec_params_t& p) {
-    SarlConsts c;
-    c.c_dt = (float)(p.time_fast * p.bandwidth * 1000.0);
-    c.c_dp = (float)(cbrt(1.0 / p.k) * p.time_fast / p.L / 1000.0);
-    c.c_rev = (float)(1000.0 * p.L / p.time_fast * cbrt(p.k));
-    c.nt1 = -(float)p.t_factor1;
-    c.nt2 = -(float)p.t_factor2;
-    c.pen1 = (float)p.penalty1;
-    c.pen2 = (float)p.penalty2;
-    c.lam = (float)p.rate;
-    c.tf = p.time_fast;
-    return c;
-}
-
 constexpr int kSarlTmaRows = 16;    // steps per stage (two 8-step mma tiles)
 constexpr int kSarlTmaStages = 2;   // input stages per warp (one in use, one in flight)
 __host__ __device__ constexpr int sarl_tma_stage_bytes(int KT) { return kSarlTmaRows * (8 * KT + 16 + 8) * 4; }
@@ -569,11 +528,7 @@ __global__ void __launch_bounds__(128, RISVEC_TMA_MINB)
             arr[2 * h + 1] = ar[(2 * h + 1) * V];
             const float2 re = __fadd2_rn(make_float2(accM[0], accM[1]), make_float2(accX[0], accX[1]));
             const float2 im = __fadd2_rn(make_float2(accM[2], accM[3]), make_float2(accX[2], accX[3]));
-            const float2 g2 = __ffma2_rn(re, re, __fmul2_rn(im, im));
-            const float2 y = __fadd2_rn(f2(1.0f), __fmul2_rn(a0[h], __fmul2_rn(f2(coef), g2)));  // SARL:159
-            rate[h] = __fmul2_rn(make_float2(__log2f(y.x), __log2f(y.y)), f2(0.693147180559945309f));
-            dt[h] = __fmul2_rn(rate[h], f2(c.c_dt));
-            dp[h] = __fmul2_rn(make_float2(cbrt_sfu(a1[h].x), cbrt_sfu(a1[h].y)), f2(c.c_dp));  // SARL:331
+            sarl_rate2(re, im, a0[h], a1[h], coef, c, rate[h], dt[h], dp[h]);
         }
         // the inputs of this stage are in registers: its buffer can take the stage after next
         __syncwarp();
@@ -589,54 +544,35 @@ __global__ void __launch_bounds__(128, RISVEC_TMA_MINB)
             inc[i] = ok ? __dmul_rn(__dmul_rn((double)arr[i], c.tf), 1000.0) : 0.0;
         }
         // ---- DataBuf at my first step: inclusive scan of the lanes' four-step maps over tig = 0..3
-        MaxPlus f = mp_then(mp_then(MaxPlus{inc[0] - dd[0], inc[0]}, MaxPlus{inc[1] - dd[1], inc[1]}),
-                            mp_then(MaxPlus{inc[2] - dd[2], inc[2]}, MaxPlus{inc[3] - dd[3], inc[3]}));
-        {
-            MaxPlus q{__shfl_up_sync(kFull, f.a, 1, 4), __shfl_up_sync(kFull, f.b, 1, 4)};
-            const MaxPlus f1 = mp_then(q, f);
-            if (tig >= 1) f = f1;
-            q = MaxPlus{__shfl_up_sync(kFull, f.a, 2, 4), __shfl_up_sync(kFull, f.b, 2, 4)};
-            const MaxPlus f2m = mp_then(q, f);
-            if (tig >= 2) f = f2m;
-        }
-        const MaxPlus ex{__shfl_up_sync(kFull, f.a, 1, 4), __shfl_up_sync(kFull, f.b, 1, 4)};  // maps before mine
-        const MaxPlus all{__shfl_sync(kFull, f.a, 3, 4), __shfl_sync(kFull, f.b, 3, 4)};       // the whole stage
+        MaxPlus ex, all;  // the maps before mine, the whole stage
+        mp_scan<4>(mp_then(mp_then(MaxPlus{inc[0] - dd[0], inc[0]}, MaxPlus{inc[1] - dd[1], inc[1]}),
+                           mp_then(MaxPlus{inc[2] - dd[2], inc[2]}, MaxPlus{inc[3] - dd[3], inc[3]})),
+                   tig, ex, all);
         const double xin = mp_apply(ex, buf);
         double cur = tig == 0 ? buf : xin;
         buf = mp_apply(all, buf);
-        // ---- my four steps in the reference's order (SARL:333-358)
+        // ---- my four steps in the reference's order (SARL:333-358); past-the-end steps are identity steps
         float overd[4], nbf[4], barg[4], curf[4];
         bool pos[4];
 #pragma unroll
-        for (int i = 0; i < 4; ++i) {
-            const float dpi = (i & 1) ? dp[i >> 1].y : dp[i >> 1].x;
-            const double raw = __dsub_rn(cur, dd[i]);  // SARL:334
-            const bool neg = raw < 0.0;
-            pos[i] = raw > 0.0;
-            barg[i] = fmaxf(0.f, (float)(raw + (double)dpi));  // argument of localProcRev (SARL:337)
-            const float rawf = (float)raw;
-            overd[i] = fmaxf(0.f, -rawf);                      // over_data = -DataBuf where it went negative
-            nbf[i] = fmaxf(0.f, rawf);
-            cur = __dadd_rn(neg ? 0.0 : raw, inc[i]);          // SARL:354-356
-            curf[i] = (float)cur;
-        }
+        for (int i = 0; i < 4; ++i)
+            sarl_settle(cur, dd[i], (i & 1) ? dp[i >> 1].y : dp[i >> 1].x, inc[i], true, overd[i], nbf[i], barg[i],
+                        pos[i], curf[i]);
         // ---- the out tile is free again once the TMA stores of the previous stage have read it
         if (threadIdx.x == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
         __syncthreads();
         float rew[4];
 #pragma unroll
         for (int h = 0; h < 2; ++h) {
-            const float2 b = __fmul2_rn(make_float2(barg[2 * h], barg[2 * h + 1]), f2(c.c_rev));
-            const float2 b3 = __fmul2_rn(__fmul2_rn(b, b), b);
-            const float2 op = __fadd2_rn(a1[h], make_float2(-b3.x, -b3.y));  // SARL:336-339
-            const float2 base2 = __ffma2_rn(make_float2(nbf[2 * h], nbf[2 * h + 1]), f2(c.nt2),
-                                            __fmul2_rn(__fadd2_rn(a0[h], a1[h]), f2(c.nt1)));
+            float2 op, base2;
+            sarl_reward2(make_float2(barg[2 * h], barg[2 * h + 1]), make_float2(nbf[2 * h], nbf[2 * h + 1]), a0[h],
+                         a1[h], c, op, base2);
 #pragma unroll
             for (int u = 0; u < 2; ++u) {
                 const int i = 2 * h + u;
                 const float od = overd[i];
                 const float overp = od > 0.f ? (u ? op.y : op.x) : 0.f;  // only where the buffer went negative
-                const float pen = pos[i] ? c.pen1 : ((od > 2.0f) ? c.pen2 : 0.f);  // SARL:343-352
+                const float pen = pos[i] ? c.pen1 : ((od > 2.0f) ? c.pen2 : 0.f);  // SARL:343-352 (a helper changed the code)
                 rew[i] = __fsub_rn(u ? base2.y : base2.x, pen);
                 float* o = out_w + 32 * i;
                 o[0 * TRACE_WORDS] = curf[i];

@@ -252,16 +252,14 @@ __global__ void __launch_bounds__(kBigThreads, 1)
                 arr0 = ok0 ? draw_arrival_cold(d, e, vc, step0 + tb, c.lam) : 0;
                 arr1 = ok1 ? draw_arrival_cold(d, e, vc, step0 + tb + 1, c.lam) : 0;
             }
-            const float2 g2 = __ffma2_rn(re, re, __fmul2_rn(im, im));
-            const float2 y = __fadd2_rn(f2(1.0f), __fmul2_rn(a0, __fmul2_rn(f2(coef), g2)));  // SARL:159
-            const float2 rate = __fmul2_rn(make_float2(__log2f(y.x), __log2f(y.y)), f2(0.693147180559945309f));
-            const float2 dt = __fmul2_rn(rate, f2(c.c_dt));
-            const float2 dp = __fmul2_rn(make_float2(cbrt_sfu(a1.x), cbrt_sfu(a1.y)), f2(c.c_dp));  // SARL:331
+            float2 rate, dt, dp;
+            sarl_rate2(re, im, a0, a1, coef, c, rate, dt, dp);
             const double d0 = ok0 ? __dadd_rn((double)dt.x, (double)dp.x) : 0.0;  // identity step when not ok
             const double d1 = ok1 ? __dadd_rn((double)dt.y, (double)dp.y) : 0.0;
             const double i0 = ok0 ? __dmul_rn(__dmul_rn((double)arr0, c.tf), 1000.0) : 0.0;
             const double i1 = ok1 ? __dmul_rn(__dmul_rn((double)arr1, c.tf), 1000.0) : 0.0;
             // DataBuf at my first step: inclusive scan of the lanes' two-step maps over the vehicle's 8 lanes
+            // (the loop, not mp_scan<8>: the unrolled helper compiles to different code for this kernel)
             MaxPlus f = mp_then(MaxPlus{i0 - d0, i0}, MaxPlus{i1 - d1, i1});
 #pragma unroll
             for (int o = 1; o < 8; o <<= 1) {
@@ -278,23 +276,11 @@ __global__ void __launch_bounds__(kBigThreads, 1)
             float overd[2], nbf[2], barg[2], curf[2];
             bool pos[2];
 #pragma unroll
-            for (int i = 0; i < 2; ++i) {
-                const double dd = i ? d1 : d0, inc = i ? i1 : i0;
-                const float dpi = i ? dp.y : dp.x;
-                const double raw = __dsub_rn(cur, dd);  // SARL:334
-                const bool neg = raw < 0.0;
-                pos[i] = raw > 0.0;
-                barg[i] = fmaxf(0.f, (float)(raw + (double)dpi));  // argument of localProcRev (SARL:337)
-                const float rawf = (float)raw;
-                overd[i] = fmaxf(0.f, -rawf);                      // over_data = -DataBuf where it went negative
-                nbf[i] = fmaxf(0.f, rawf);
-                if (i ? ok1 : ok0) cur = __dadd_rn(neg ? 0.0 : raw, inc);  // SARL:354-356
-                curf[i] = (float)cur;
-            }
-            const float2 b = __fmul2_rn(make_float2(barg[0], barg[1]), f2(c.c_rev));
-            const float2 b3 = __fmul2_rn(__fmul2_rn(b, b), b);
-            const float2 op = __fadd2_rn(a1, make_float2(-b3.x, -b3.y));  // SARL:336-339
-            const float2 base2 = __ffma2_rn(make_float2(nbf[0], nbf[1]), f2(c.nt2), __fmul2_rn(__fadd2_rn(a0, a1), f2(c.nt1)));
+            for (int i = 0; i < 2; ++i)
+                sarl_settle(cur, i ? d1 : d0, i ? dp.y : dp.x, i ? i1 : i0, i ? ok1 : ok0, overd[i], nbf[i], barg[i],
+                            pos[i], curf[i]);
+            float2 op, base2;
+            sarl_reward2(make_float2(barg[0], barg[1]), make_float2(nbf[0], nbf[1]), a0, a1, c, op, base2);
             // the out tile is free again once the TMA stores of the previous stage have read it
             if (leader) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
             named_bar_sync(2, STEP_THREADS);
@@ -303,7 +289,7 @@ __global__ void __launch_bounds__(kBigThreads, 1)
             for (int i = 0; i < 2; ++i) {
                 const float od = overd[i];
                 const float overp = od > 0.f ? (i ? op.y : op.x) : 0.f;  // only where the buffer went negative
-                const float pen = pos[i] ? c.pen1 : ((od > 2.0f) ? c.pen2 : 0.f);  // SARL:343-352
+                const float pen = pos[i] ? c.pen1 : ((od > 2.0f) ? c.pen2 : 0.f);  // SARL:343-352 (a helper changed the code)
                 rew[i] = (i ? ok1 : ok0) ? __fsub_rn(i ? base2.y : base2.x, pen) : 0.f;
                 if (vact) {
                     float* o = out_w + i * V;

@@ -312,11 +312,7 @@ __global__ void __launch_bounds__(kUmmaThreads, 1)
             for (int h = 0; h < 2; ++h) {
                 const float2 re = __fadd2_rn(make_float2(dm[4 * h], dm[4 * h + 1]), make_float2(dx[4 * h], dx[4 * h + 1]));
                 const float2 im = __fadd2_rn(make_float2(dm[4 * h + 2], dm[4 * h + 3]), make_float2(dx[4 * h + 2], dx[4 * h + 3]));
-                const float2 g2 = __ffma2_rn(re, re, __fmul2_rn(im, im));
-                const float2 y = __fadd2_rn(f2(1.0f), __fmul2_rn(a0[h], __fmul2_rn(f2(coef), g2)));  // SARL:159
-                rate[h] = __fmul2_rn(make_float2(__log2f(y.x), __log2f(y.y)), f2(0.693147180559945309f));
-                dt[h] = __fmul2_rn(rate[h], f2(c.c_dt));
-                dp[h] = __fmul2_rn(make_float2(cbrt_sfu(a1[h].x), cbrt_sfu(a1[h].y)), f2(c.c_dp));  // SARL:331
+                sarl_rate2(re, im, a0[h], a1[h], coef, c, rate[h], dt[h], dp[h]);
             }
             double dd[4], inc[4];
 #pragma unroll
@@ -326,18 +322,10 @@ __global__ void __launch_bounds__(kUmmaThreads, 1)
                 inc[i] = ok[i] ? __dmul_rn(__dmul_rn((double)arr[i], c.tf), 1000.0) : 0.0;
             }
             // ---- composed map of my four steps, inclusive scan over tig (state independent)
-            MaxPlus f = mp_then(mp_then(MaxPlus{inc[0] - dd[0], inc[0]}, MaxPlus{inc[1] - dd[1], inc[1]}),
-                                mp_then(MaxPlus{inc[2] - dd[2], inc[2]}, MaxPlus{inc[3] - dd[3], inc[3]}));
-            {
-                MaxPlus q{__shfl_up_sync(kFull, f.a, 1, 4), __shfl_up_sync(kFull, f.b, 1, 4)};
-                const MaxPlus f1 = mp_then(q, f);
-                if (tig >= 1) f = f1;
-                q = MaxPlus{__shfl_up_sync(kFull, f.a, 2, 4), __shfl_up_sync(kFull, f.b, 2, 4)};
-                const MaxPlus f2m = mp_then(q, f);
-                if (tig >= 2) f = f2m;
-            }
-            const MaxPlus ex{__shfl_up_sync(kFull, f.a, 1, 4), __shfl_up_sync(kFull, f.b, 1, 4)};  // maps before mine
-            const MaxPlus all{__shfl_sync(kFull, f.a, 3, 4), __shfl_sync(kFull, f.b, 3, 4)};       // the whole stage
+            MaxPlus ex, all;  // the maps before mine, the whole stage
+            mp_scan<4>(mp_then(mp_then(MaxPlus{inc[0] - dd[0], inc[0]}, MaxPlus{inc[1] - dd[1], inc[1]}),
+                               mp_then(MaxPlus{inc[2] - dd[2], inc[2]}, MaxPlus{inc[3] - dd[3], inc[3]})),
+                       tig, ex, all);
             // ---- the serial link: DataBuf after stage k - 1 from the other set, DataBuf after stage k to it
             if (k > 0) {
                 mbar_wait(bar_h_other, (uint32_t)((k - 1) >> 1) & 1u);
@@ -355,18 +343,9 @@ __global__ void __launch_bounds__(kUmmaThreads, 1)
             float overd[4], nbf[4], barg[4], curf[4];
             bool pos[4];
 #pragma unroll
-            for (int i = 0; i < 4; ++i) {
-                const float dpi = (i & 1) ? dp[i >> 1].y : dp[i >> 1].x;
-                const double raw = __dsub_rn(cur, dd[i]);  // SARL:334
-                const bool neg = raw < 0.0;
-                pos[i] = raw > 0.0;
-                barg[i] = fmaxf(0.f, (float)(raw + (double)dpi));  // argument of localProcRev (SARL:337)
-                const float rawf = (float)raw;
-                overd[i] = fmaxf(0.f, -rawf);                      // over_data = -DataBuf where it went negative
-                nbf[i] = fmaxf(0.f, rawf);
-                if (ok[i]) cur = __dadd_rn(neg ? 0.0 : raw, inc[i]);  // SARL:354-356
-                curf[i] = (float)cur;
-            }
+            for (int i = 0; i < 4; ++i)
+                sarl_settle(cur, dd[i], (i & 1) ? dp[i >> 1].y : dp[i >> 1].x, inc[i], ok[i], overd[i], nbf[i], barg[i],
+                            pos[i], curf[i]);
             // ---- my set's out tile is free again once the TMA stores of its previous stage have read it
             if (leader) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
             named_bar_sync(bar_id, 128);
@@ -377,17 +356,15 @@ __global__ void __launch_bounds__(kUmmaThreads, 1)
             float rew[4];
 #pragma unroll
             for (int h = 0; h < 2; ++h) {
-                const float2 b = __fmul2_rn(make_float2(barg[2 * h], barg[2 * h + 1]), f2(c.c_rev));
-                const float2 b3 = __fmul2_rn(__fmul2_rn(b, b), b);
-                const float2 op = __fadd2_rn(a1[h], make_float2(-b3.x, -b3.y));  // SARL:336-339
-                const float2 base2 = __ffma2_rn(make_float2(nbf[2 * h], nbf[2 * h + 1]), f2(c.nt2),
-                                                __fmul2_rn(__fadd2_rn(a0[h], a1[h]), f2(c.nt1)));
+                float2 op, base2;
+                sarl_reward2(make_float2(barg[2 * h], barg[2 * h + 1]), make_float2(nbf[2 * h], nbf[2 * h + 1]), a0[h],
+                             a1[h], c, op, base2);
 #pragma unroll
                 for (int u = 0; u < 2; ++u) {
                     const int i = 2 * h + u;
                     const float od = overd[i];
                     const float overp = od > 0.f ? (u ? op.y : op.x) : 0.f;  // only where the buffer went negative
-                    const float pen = pos[i] ? c.pen1 : ((od > 2.0f) ? c.pen2 : 0.f);  // SARL:343-352
+                    const float pen = pos[i] ? c.pen1 : ((od > 2.0f) ? c.pen2 : 0.f);  // SARL:343-352 (a helper changed the code)
                     rew[i] = ok[i] ? __fsub_rn(u ? base2.y : base2.x, pen) : 0.f;
                     if (vact) {
                         float* o = out_w + i * V;

@@ -11,6 +11,7 @@
 #include <type_traits>
 
 #include "common.cuh"
+#include "step_math.cuh"
 
 namespace risvec {
 
@@ -272,9 +273,6 @@ __global__ void __launch_bounds__(128) k_marl_rollout(Dims d, State s, risvec_pa
     }
 }
 
-// ---- packed-fp32x2 math helpers shared by the SARL kernels
-__device__ __forceinline__ float2 f2(float a) { return make_float2(a, a); }
-
 // sin/cos of two float32 angles (radians, |x| < ~1e4; RIS phases live in [0, 2*pi]) in packed
 // fp32x2 arithmetic: Cody-Waite reduction to [-pi/4, pi/4] by quadrants, Cephes minimax
 // polynomials (<= 1 ulp there), quadrant fix-up with integer sign flips.
@@ -298,40 +296,6 @@ __device__ __forceinline__ void sincos_fast2(float2 x, float2* sn, float2* cs) {
     cs->x = __int_as_float(__float_as_int(ca) ^ (((qa + 1) << 30) & 0x80000000));
     sn->y = __int_as_float(__float_as_int(sb) ^ ((qb << 30) & 0x80000000));
     cs->y = __int_as_float(__float_as_int(cb) ^ (((qb + 1) << 30) & 0x80000000));
-}
-
-// ln(1 + x) for x >= 0 through the SFU: MUFU.LG2 of the rounded sum.  Absolute error <= 6e-8 near
-// zero (the rounding of 1 + x) and ~2^-22 relative elsewhere -- inside the SARL rate tolerance
-// (tests/parity.py), and SARL has no threshold on the rate itself.
-__device__ __forceinline__ float log1p_sfu(float x) { return __fmul_rn(__log2f(__fadd_rn(1.0f, x)), 0.693147180559945309f); }
-
-// cbrt(x) for x >= 0: SFU seed exp2(log2(x) / 3) (rel. error ~5e-7) + one Newton step
-// y <- y - (y^3 - x) / (3 y^2), which brings it to ~1 ulp; cbrt(0) = 0.
-__device__ __forceinline__ float cbrt_sfu(float x) {
-    const float y = exp2f(__fmul_rn(__log2f(x), 0.333333343f));
-    const float y2 = __fmul_rn(y, y);
-    const float r = __fdividef(__fmaf_rn(-y2, y, x), __fmul_rn(3.0f, y2));
-    return (x > 0.f) ? __fadd_rn(y, r) : 0.f;
-}
-
-// ln(1 + x) for x >= 0 with relative error < 1e-6 everywhere: far-user NOMA SINRs are << 1, where
-// 1 + x would lose x, so below 1/4 a degree-11 series in x is used (truncation < 2e-8 relative) and
-// above it MUFU.LG2 of (1 + x) (there |log2| >= 0.32 and the unit's absolute error 2^-22 is < 6e-7
-// relative).  Both branches are evaluated, one select; about a third of the library's log1pf.
-__device__ __forceinline__ float log1p_pos(float x) {
-    const float big = __fmul_rn(__log2f(__fadd_rn(1.0f, x)), 0.693147180559945309f);
-    float p = 0.0909090909f;                       // 1/11
-    p = __fmaf_rn(p, x, -0.1f);
-    p = __fmaf_rn(p, x, 0.111111111f);
-    p = __fmaf_rn(p, x, -0.125f);
-    p = __fmaf_rn(p, x, 0.142857143f);
-    p = __fmaf_rn(p, x, -0.166666667f);
-    p = __fmaf_rn(p, x, 0.2f);
-    p = __fmaf_rn(p, x, -0.25f);
-    p = __fmaf_rn(p, x, 0.333333333f);
-    p = __fmaf_rn(p, x, -0.5f);
-    p = __fmaf_rn(p, x, 1.0f);
-    return x < 0.25f ? __fmul_rn(p, x) : big;
 }
 
 __device__ __forceinline__ float2 shfl_xor2(float2 x, int o) {
@@ -387,19 +351,7 @@ __global__ void __launch_bounds__(32 * WPE) k_sarl_rollout(Dims d, State s, risv
 
     // ---- geometry phasor table -> registers (float64 argument reduction), as element pairs
     float2 WX[MPL / 2], WY[MPL / 2];
-    {
-        // w(v, m0 + i) = z^m0 * z^i in float64 from one sincospi per lane
-        const double2 z = unit_phasor64(act ? d.angle_BR - s.angle[ev] : 0.0);
-        double2 wv = cpow64(z, (unsigned)m0);
-#pragma unroll
-        for (int i = 0; i < MPL; ++i) {
-            const bool on = act && (m0 + i < m1);
-            const float re = on ? (float)wv.x : 0.f, im = on ? (float)wv.y : 0.f;
-            if (i & 1) { WX[i >> 1].y = re; WY[i >> 1].y = im; }
-            else       { WX[i >> 1].x = re; WY[i >> 1].x = im; }
-            wv = cmul64(wv, z);
-        }
-    }
+    phasor_pairs<MPL>(d, s, ev, act, m0, m1, WX, WY);
     for (int i = threadIdx.x; i < 6 * plane; i += NT) th[i] = 0.f;  // pad elements must stay finite
     const bool cphase = (w == 0);
     const int t_begin = 0, t_end = T;
@@ -407,17 +359,15 @@ __global__ void __launch_bounds__(32 * WPE) k_sarl_rollout(Dims d, State s, risv
     const float coef = act ? (float)(s.amp[ev] / (kSigma * kSigma)) : 0.f;  // SARL:157-159
     const long long step0 = env_ok ? s.step_ctr[e] : 0;
 
-    const float c_dt = (float)(p.time_fast * p.bandwidth * 1000.0);
-    const float c_dp = (float)(cbrt(1.0 / p.k) * p.time_fast / p.L / 1000.0);       // SARL:331
-    const float c_rev = (float)(1000.0 * p.L / p.time_fast * cbrt(p.k));             // SARL:318-319
+    const SarlConsts sc = sarl_consts(p);  // SARL:160, 318-319, 331
     const float t1 = (float)p.t_factor1, t2 = (float)p.t_factor2, pen1 = (float)p.penalty1, pen2 = (float)p.penalty2;
     const float invV = 1.0f / (float)V;
     const float lam = (float)p.rate;
     const int n_env_here = min(EPW, E - e0);
     const int n_ph = n_env_here * M;  // the EPW rows of phase[t] are contiguous in HBM
 
-    float o_rate = 0.f, o_dt = 0.f, o_dp = 0.f, o_overp = 0.f, o_overd = 0.f, o_rew = 0.f;
-    int o_arr = 0;
+    SarlLast last{};
+    float o_rew = 0.f;
 
     // theta(t) -> smem buffer t & 1: thread k handles elements k, k + NT, ... in packed pairs.
     // The first pair of every step is prefetched one step ahead into (pf0, pf1).  All stream
@@ -549,41 +499,22 @@ __global__ void __launch_bounds__(32 * WPE) k_sarl_rollout(Dims d, State s, risv
 
             const float g2 = __fmaf_rn(sr, sr, __fmul_rn(si, si));
             const float rate = log1p_sfu(__fmul_rn(a0, __fmul_rn(coef, g2)));  // natural log, SARL:159
-            const float data_t = __fmul_rn(rate, c_dt);
-            const float data_p = __fmul_rn(cbrt_sfu(a1), c_dp);
-            const double raw = __dsub_rn(buf, __dadd_rn((double)data_t, (double)data_p));  // SARL:334
-            const bool neg = raw < 0.0;
-            const float b = __fmul_rn((float)fmax(0.0, raw + (double)data_p), c_rev);
-            const float overp = neg ? __fsub_rn(a1, __fmul_rn(__fmul_rn(b, b), b)) : 0.f;  // SARL:336-339
-            const float overd = neg ? (float)(-raw) : 0.f;
-            const double nb = neg ? 0.0 : raw;
-            const float base = __fsub_rn(-__fmul_rn(t1, __fadd_rn(a0, a1)), __fmul_rn(t2, (float)nb));
-            const float pen = (nb > 0.0) ? pen1 : ((overd > 2.0f) ? pen2 : 0.f);  // SARL:343-352
-            const float rew = __fmul_rn(seg_sum<VP>(act ? __fsub_rn(base, pen) : 0.f), invV);
-            buf = __dadd_rn(nb, __dmul_rn(__dmul_rn((double)arr, p.time_fast), 1000.0));  // SARL:354-356
-
+            const float data_p = __fmul_rn(cbrt_sfu(a1), sc.c_dp);
+            const SarlStep st = sarl_step(buf, rate, data_p, a0, a1, arr, sc.c_dt, sc.c_rev, t1, t2, pen1, pen2, p.time_fast);
+            const float rew = __fmul_rn(seg_sum<VP>(act ? st.ru : 0.f), invV);
+            last = SarlLast{rate, st.data_t, data_p, st.overp, st.overd, arr};
             if (act) {
-                if (a.out.DataBuf != nullptr) a.out.DataBuf[tev] = (float)buf;
-                if (a.out.data_t != nullptr) a.out.data_t[tev] = data_t;
-                if (a.out.data_p != nullptr) a.out.data_p[tev] = data_p;
-                if (a.out.over_power != nullptr) a.out.over_power[tev] = overp;
-                if (a.out.over_data != nullptr) a.out.over_data[tev] = overd;
-                if (a.out.rate != nullptr) a.out.rate[tev] = rate;
+                sarl_store_traces(a.out, tev, (float)buf, last);
                 if (v == 0 && a.out.reward != nullptr) a.out.reward[(size_t)t * E + e] = rew;
             }
-            o_rate = rate; o_dt = data_t; o_dp = data_p; o_overp = overp; o_overd = overd; o_rew = rew; o_arr = arr;
+            o_rew = rew;
         }
         if (WPE == 1) __syncwarp();  // theta(t + 1) of this warp is complete before the next MACs
     }
 
     if (cphase && act && T > 0) {
         s.databuf[ev] = buf;
-        s.rate[ev] = o_rate;
-        s.data_t[ev] = o_dt;
-        s.data_p[ev] = o_dp;
-        s.over_power[ev] = o_overp;
-        s.over_data[ev] = o_overd;
-        s.data_r[ev] = o_arr;
+        sarl_store_last(s, ev, last);
         if (v == 0) {
             s.reward[e] = o_rew;
             s.step_ctr[e] = step0 + T;
@@ -619,18 +550,7 @@ __global__ void __launch_bounds__(32 * WPE, (WPE <= 8 && MPL <= 32) ? 16 / WPE :
     const int m0 = w * slice, m1 = min(M, m0 + slice);
 
     float2 WX[MPL / 2], WY[MPL / 2];
-    {
-        const double2 z = unit_phasor64(act ? d.angle_BR - s.angle[ev] : 0.0);
-        double2 wv = cpow64(z, (unsigned)m0);
-#pragma unroll
-        for (int i = 0; i < MPL; ++i) {
-            const bool on = act && (m0 + i < m1);
-            const float re = on ? (float)wv.x : 0.f, im = on ? (float)wv.y : 0.f;
-            if (i & 1) { WX[i >> 1].y = re; WY[i >> 1].y = im; }
-            else       { WX[i >> 1].x = re; WY[i >> 1].x = im; }
-            wv = cmul64(wv, z);
-        }
-    }
+    phasor_pairs<MPL>(d, s, ev, act, m0, m1, WX, WY);
     for (int i = threadIdx.x; i < 8 * plane; i += NT) th[i] = 0.f;  // pad elements must stay finite
     const int t_begin = (int)blockIdx.y * a.t_chunk, t_end = min(T, t_begin + a.t_chunk);
     const int n_ph = min(EPW, E - e0) * M;
@@ -748,9 +668,7 @@ __global__ void __launch_bounds__(128) k_sarl_scan(Dims d, State s, risvec_param
     double buf = s.databuf[ev];
     const float coef = (float)(s.amp[ev] / (kSigma * kSigma));  // SARL:157-159
     const long long step0 = s.step_ctr[min(e, E - 1)];
-    const float c_dt = (float)(p.time_fast * p.bandwidth * 1000.0);
-    const float c_dp = (float)(cbrt(1.0 / p.k) * p.time_fast / p.L / 1000.0);
-    const float c_rev = (float)(1000.0 * p.L / p.time_fast * cbrt(p.k));
+    const SarlConsts sc = sarl_consts(p);  // SARL:160, 318-319, 331
     const float t1 = (float)p.t_factor1, t2 = (float)p.t_factor2, pen1 = (float)p.penalty1, pen2 = (float)p.penalty2;
     const float invV = 1.0f / (float)V;
     const float lam = (float)p.rate;
@@ -770,8 +688,8 @@ __global__ void __launch_bounds__(128) k_sarl_scan(Dims d, State s, risvec_param
     };
 #pragma unroll
     for (int k = 0; k < D; ++k) fetch(k, k);
-    float o_rate = 0.f, o_dt = 0.f, o_dp = 0.f, o_overp = 0.f, o_overd = 0.f, o_rew = 0.f;
-    int o_arr = 0;
+    SarlLast last{};
+    float o_rew = 0.f;
     for (int tb = 0; tb < T; tb += D) {
         float ca0[D], ca1[D], cg2[D];
         int carr[D];
@@ -791,39 +709,20 @@ __global__ void __launch_bounds__(128) k_sarl_scan(Dims d, State s, risvec_param
         int arr = carr[k];
         if (act && a.arrivals == nullptr) arr = draw_arrival(d, e, v, step0 + t, lam);
         const float rate = log1p_sfu(__fmul_rn(a0, __fmul_rn(coef, g2)));  // natural log, SARL:159
-        const float data_t = __fmul_rn(rate, c_dt);
-        const float data_p = __fmul_rn(cbrt_sfu(a1), c_dp);
-        const double raw = __dsub_rn(buf, __dadd_rn((double)data_t, (double)data_p));  // SARL:334
-        const bool neg = raw < 0.0;
-        const float b = __fmul_rn((float)fmax(0.0, raw + (double)data_p), c_rev);
-        const float overp = neg ? __fsub_rn(a1, __fmul_rn(__fmul_rn(b, b), b)) : 0.f;  // SARL:336-339
-        const float overd = neg ? (float)(-raw) : 0.f;
-        const double nb = neg ? 0.0 : raw;
-        const float base = __fsub_rn(-__fmul_rn(t1, __fadd_rn(a0, a1)), __fmul_rn(t2, (float)nb));
-        const float pen = (nb > 0.0) ? pen1 : ((overd > 2.0f) ? pen2 : 0.f);  // SARL:343-352
-        const float rew = __fmul_rn(seg_sum<VP>(act ? __fsub_rn(base, pen) : 0.f), invV);
-        buf = __dadd_rn(nb, __dmul_rn(__dmul_rn((double)arr, p.time_fast), 1000.0));  // SARL:354-356
+        const float data_p = __fmul_rn(cbrt_sfu(a1), sc.c_dp);
+        const SarlStep st = sarl_step(buf, rate, data_p, a0, a1, arr, sc.c_dt, sc.c_rev, t1, t2, pen1, pen2, p.time_fast);
+        const float rew = __fmul_rn(seg_sum<VP>(act ? st.ru : 0.f), invV);
+        last = SarlLast{rate, st.data_t, data_p, st.overp, st.overd, arr};
         if (act) {
-            const size_t tev = (size_t)t * sV + ev;
-            if (a.out.DataBuf != nullptr) a.out.DataBuf[tev] = (float)buf;
-            if (a.out.data_t != nullptr) a.out.data_t[tev] = data_t;
-            if (a.out.data_p != nullptr) a.out.data_p[tev] = data_p;
-            if (a.out.over_power != nullptr) a.out.over_power[tev] = overp;
-            if (a.out.over_data != nullptr) a.out.over_data[tev] = overd;
-            if (a.out.rate != nullptr) a.out.rate[tev] = rate;
+            sarl_store_traces(a.out, (size_t)t * sV + ev, (float)buf, last);
             if (v == 0 && a.out.reward != nullptr) a.out.reward[(size_t)t * E + e] = rew;
         }
-        o_rate = rate; o_dt = data_t; o_dp = data_p; o_overp = overp; o_overd = overd; o_rew = rew; o_arr = arr;
+        o_rew = rew;
         }
     }
     if (act && T > 0) {
         s.databuf[ev] = buf;
-        s.rate[ev] = o_rate;
-        s.data_t[ev] = o_dt;
-        s.data_p[ev] = o_dp;
-        s.over_power[ev] = o_overp;
-        s.over_data[ev] = o_overd;
-        s.data_r[ev] = o_arr;
+        sarl_store_last(s, ev, last);
         if (v == 0) {
             s.reward[e] = o_rew;
             s.step_ctr[e] = step0 + T;
@@ -924,9 +823,7 @@ __global__ void __launch_bounds__(32) k_sarl_v8(Dims d, State s, risvec_params_t
     double buf = s.databuf[ev];
     const float coef = (float)(s.amp[ev] / (kSigma * kSigma));  // SARL:157-159
     const long long step0 = s.step_ctr[e];
-    const float c_dt = (float)(p.time_fast * p.bandwidth * 1000.0);
-    const float c_dp = (float)(cbrt(1.0 / p.k) * p.time_fast / p.L / 1000.0);  // SARL:331
-    const float c_rev = (float)(1000.0 * p.L / p.time_fast * cbrt(p.k));        // SARL:318-319
+    const SarlConsts sc = sarl_consts(p);  // SARL:160, 318-319, 331
     const float t1 = (float)p.t_factor1, t2 = (float)p.t_factor2, pen1 = (float)p.penalty1, pen2 = (float)p.penalty2;
     const float invV = 1.0f / (float)V;
     const float lam = (float)p.rate;
@@ -1028,24 +925,24 @@ __global__ void __launch_bounds__(32) k_sarl_v8(Dims d, State s, risvec_params_t
         const float g0 = sarl_reduce_abs2(RE0, IM0), g1 = sarl_reduce_abs2(RE1, IM1);
         h0.rate = log1p_sfu(__fmul_rn(i0.a0, __fmul_rn(coef, g0)));
         h1.rate = log1p_sfu(__fmul_rn(i1.a0, __fmul_rn(coef, g1)));
-        h0.data_p = __fmul_rn(cbrt_sfu(i0.a1), c_dp);
-        h1.data_p = __fmul_rn(cbrt_sfu(i1.a1), c_dp);
+        h0.data_p = __fmul_rn(cbrt_sfu(i0.a1), sc.c_dp);
+        h1.data_p = __fmul_rn(cbrt_sfu(i1.a1), sc.c_dp);
     };
 
     float l_rate = 0.f, l_dt = 0.f, l_dp = 0.f, l_overp = 0.f, l_overd = 0.f, l_rew = 0.f;
     int l_arr = 0;
 
     // sequential part of one step (SARL:333-358), branch-free so that it can be interleaved
-    // with the next pair's heavy part
+    // with the next pair's heavy part (written out, not sarl_step: the helper compiles to different code here)
     auto scan_step = [&](const SarlScalarIn& in, const SarlHeavyOut& h, unsigned t) {
         int arr = in.arr;
         if (!FULL && ar_b == nullptr) arr = act ? draw_arrival(d, e, v, step0 + t, lam) : 0;
-        const float data_t = __fmul_rn(h.rate, c_dt);
+        const float data_t = __fmul_rn(h.rate, sc.c_dt);
         const double raw = __dsub_rn(buf, __dadd_rn((double)data_t, (double)h.data_p));  // SARL:334
         const bool neg = raw < 0.0;
         // (explicit _rn intrinsics: no FMA contraction, so the loop copy and the tail copy of this
         //  code -- and therefore T = 1 launches and fused rollouts -- round identically)
-        const float b = __fmul_rn((float)fmax(0.0, raw + (double)h.data_p), c_rev);
+        const float b = __fmul_rn((float)fmax(0.0, raw + (double)h.data_p), sc.c_rev);
         const float overp = neg ? __fsub_rn(in.a1, __fmul_rn(__fmul_rn(b, b), b)) : 0.f;  // SARL:337
         const float overd = neg ? (float)(-raw) : 0.f;
         const double nb = neg ? 0.0 : raw;
@@ -1195,7 +1092,7 @@ __global__ void __launch_bounds__(32) k_marl_v8(Dims d, State s, risvec_params_t
     floor_d = fmax(0.0, fmin(floor_d, 0.95));
     const float floor_f = (float)floor_d;
     const double Cpb = p.cycles_per_bit, den = Cpb * 1000.0, tf = p.time_fast, flm = p.f_local_max;
-    const double rden = 1.0 / den;  // correctly rounded reciprocal for the FMA division below
+    const double rden = 1.0 / den;  // correctly rounded reciprocal for div_rn_fma
     const double edge_cap = p.f_edge_max * p.time_fast;
     const float inv_fedge = (float)(1.0 / (p.f_edge_max + 1e-12));
     const float kf = (float)p.k;
@@ -1266,17 +1163,15 @@ __global__ void __launch_bounds__(32) k_marl_v8(Dims d, State s, risvec_params_t
     using No = std::false_type;   // steps before the last: no `last_*` statistics
     using Yes = std::true_type;   // the final step also produces the `last_*` state
 
-    // sequential part of a step: local CPU, offload, MEC queue, delays, energy, reward
+    // sequential part of a step: local CPU, offload, MEC queue, delays, energy, reward (written out, as k_marl_tma's
+    // copy: shared helpers for the power / rate, delay / reward and last_* parts changed this kernel's code)
     auto scan_step = [&](const MarlIn& in, const MarlHeavy& h, unsigned t, auto with_stats) {
         int arr = in.arr;
         if (!FULL && ar_b == nullptr) arr = act ? draw_arrival(d, e, v, step0 + t, lam) : 0;
         const double backlog_kbit = buf;
         const double backlog_cyc = __dmul_rn(__dmul_rn(backlog_kbit, 1000.0), Cpb);  // MARL:585-592
         const double used = fmin(h.cap, backlog_cyc);
-        // used / den, correctly rounded, without the library's special-case branches (Markstein:
-        // q0 = RN(a*r), rem = a - q0*b exactly by FMA, q = RN(q0 + rem*r) with r = RN(1/b))
-        const double q0 = __dmul_rn(used, rden);
-        const double local_done = __fma_rn(__fma_rn(-q0, den, used), rden, q0);
+        const double local_done = div_rn_fma(used, den, rden);
         const double remaining = fmax(0.0, __dsub_rn(backlog_kbit, local_done));
         const double off = fmin((double)h.data_t, remaining);                       // MARL:595-596
         const double edge_in = __dmul_rn(__dmul_rn(off, 1000.0), Cpb);               // MARL:604
