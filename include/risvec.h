@@ -494,6 +494,28 @@ enum risvec_env_param {
 };
 int risvec_attach_env_params(risvec_env_t* env, const double* table);
 
+/* Per-env RIS size: env e has the RIS elements 0 .. n_elem[e] - 1 of the handle's M-element array, so one handle can
+ * sweep the number of elements (one launch and one CUDA graph for the whole sweep) or draw a new size for the next
+ * episode of one env.  An env with n elements is exactly an env of a handle with M = n: the geometry phasors depend on
+ * m only, and every quantity that depends on M is a sum over the elements.  `n_elem` [E] int32, a device pointer on
+ * the handle's device, owned by the caller; NULL detaches.  Each value is clamped to [1, M] before it is used as a
+ * bound (0 would leave all-zero gains for the pairing's dB arithmetic), and rows are not otherwise validated.  The
+ * array is read at each launch and never copied: rewrite it between launches, also inside a captured CUDA graph.
+ * The elements m >= n of an env are absent: no sum includes them and the BCD neither scores nor writes their theta.
+ * Their theta_re / theta_im / phase_real entries and their phase / raw-action columns keep the handle's width M (the
+ * observation and action widths do not change) and affect nothing.
+ * Entry points that read it:
+ *   MARL: risvec_optimize_phase_shift, risvec_update_channel_gains (free channel), the CHANNEL stage of
+ *         risvec_begin_episode and risvec_episode_tick -- a new count takes effect at the env's next CHANNEL stage;
+ *         the step reads the gains only, so the rollouts and the fused step are unchanged.  The 3GPP channel branch
+ *         has no RIS term and ignores the array.
+ *   SARL: risvec_rollout_sarl, its _host form and risvec_step_sarl_fused -- a new count takes effect at the next step.
+ * While it is attached the SARL kernels k_sarl_mma_tma, k_sarl_umma, k_sarl_mma_big and k_sarl_v8 are not chosen
+ * (k_sarl_mma and the generic kernels take the array, as with a per-env parameter table, and both can be attached
+ * together), and risvec_rollout_sarl_packed / _packed_host return RISVEC_ERR_UNSUPPORTED.  The MARL kernel choice,
+ * packed records included, does not change. */
+int risvec_attach_ris_elements(risvec_env_t* env, const int32_t* n_elem);
+
 /* Per-episode statistics of staggered episodes: per-env running sums on the device and a log of completed episodes.
  * n_user = V for MARL, 0 for SARL.  All memory is owned by the caller.
  * running [E, RISVEC_EPLOG_RUN_COLS(n_user)] f64, zero-filled by the caller, one row per env:

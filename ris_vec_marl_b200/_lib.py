@@ -202,6 +202,7 @@ EXPORTS = {
                                             C.c_void_p, C.c_void_p]),
     "risvec_attach_stats_accumulator": (C.c_int, [C.c_void_p, C.c_void_p]),
     "risvec_attach_env_params": (C.c_int, [C.c_void_p, C.c_void_p]),
+    "risvec_attach_ris_elements": (C.c_int, [C.c_void_p, C.c_void_p]),
     "risvec_collect_stats": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     "risvec_shared_buffer_create": (C.c_int, [C.c_int, C.c_uint64, C.POINTER(C.c_void_p), C.c_char_p]),
     "risvec_shared_buffer_open": (C.c_int, [C.c_int, C.c_char_p, C.POINTER(C.c_void_p)]),

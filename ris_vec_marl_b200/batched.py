@@ -114,6 +114,7 @@ class BatchedEnviron:
             self._views[name] = self._views[name].view(self.E, self.V, self.V)
         self.pairing = default_pairing(self.V)
         self.env_params = None  # the attached per-env parameter table (attach_env_params)
+        self._ris_elements = None  # the attached per-env RIS size (attach_ris_elements)
 
     # ------------------------------------------------------------------ params
     def _set_lanes(self, name, vals):
@@ -189,6 +190,50 @@ class BatchedEnviron:
                 col.copy_(v)
             else:
                 col.fill_(float(v))
+
+    def attach_ris_elements(self, attach=True, counts=None):
+        """Per-env RIS size (`risvec_attach_ris_elements`): env e uses the RIS elements 0 .. counts[e] - 1 of the
+        handle's M, exactly as a handle created with M = counts[e] would (a sweep over the number of elements in one
+        handle, or a new size for the next episode of one env).  Values are clamped to [1, M] on the device.
+
+        Allocates an int32 [E] device tensor filled with M, attaches it and returns it.  `counts` attaches the
+        caller's tensor instead; anything but a contiguous int32 [E] tensor on this device is refused, not converted.
+        The library reads it at every launch and never copies it: rewrite it with `set_ris_elements` or torch ops
+        between steps, also inside a captured CUDA graph.  MARL takes a new count at the env's next CHANNEL stage
+        (`optimize_phase_shift` / `update_channel_gains`, or an episode start), SARL at its next step.  The widths of
+        phases, actions and observations stay M; the columns m >= counts[e] are ignored.  `attach=False` detaches it.
+        Attaching while one is attached raises: a CUDA graph captured earlier holds the attached tensor's address."""
+        if not attach:
+            check(self._lib.risvec_attach_ris_elements(self._h, self._p(None)))
+            self._ris_elements = None
+            return None
+        if self._ris_elements is not None:
+            raise RuntimeError("a per-env RIS size is already attached: attach_ris_elements(False) first, or write it "
+                               "in place with set_ris_elements")
+        if counts is None:
+            counts = torch.full((self.E,), self.M, dtype=torch.int32, device=self.device)
+        else:
+            self._check("counts", counts, torch.int32, (self.E,), self.device)
+        check(self._lib.risvec_attach_ris_elements(self._h, self._p(counts)))
+        self._ris_elements = counts
+        return counts
+
+    def set_ris_elements(self, counts):
+        """Write the attached per-env RIS size in place: a Python int (every env) or an int32 [E] tensor on this
+        device (anything else is refused).  No host synchronisation, so the call can be captured in a CUDA graph."""
+        if self._ris_elements is None:
+            raise RuntimeError("attach_ris_elements() first")
+        if isinstance(counts, torch.Tensor):
+            if tuple(counts.shape) != (self.E,) or counts.device != self.device or counts.dtype != torch.int32:
+                raise ValueError(f"counts must be an int32 [{self.E}] tensor on {self.device}")
+            self._ris_elements.copy_(counts)
+        else:
+            self._ris_elements.fill_(int(counts))
+
+    @property
+    def ris_elements(self):
+        """The attached per-env RIS size (int32 [E] device tensor), or None."""
+        return self._ris_elements
 
     def get_param(self, name):
         return getattr(self.params, name)
@@ -680,7 +725,8 @@ class BatchedEnviron:
     def state_dict(self):
         """Everything a resumed run needs to CONTINUE this one: the state arena, the host-side call counters
         that key the on-device Philox draws, the scalar parameters, the pairing knobs and, when one is attached, the
-        per-env parameter table (`"_env_params"`).  `load_state_dict` of a state without a table detaches one."""
+        per-env parameter table (`"_env_params"`) and RIS size (`"_ris_elements"`).  `load_state_dict` of a state
+        without one detaches an attached one."""
         ctr = (C.c_uint64 * 3)()
         check(self._lib.risvec_get_rng_counters(self._h, ctr))
         sd = {k: v.clone() for k, v in self._views.items()}
@@ -689,6 +735,8 @@ class BatchedEnviron:
         sd["_pairing"] = bytes(self.pairing)
         if self.env_params is not None:
             sd["_env_params"] = self.env_params.clone()
+        if self._ris_elements is not None:
+            sd["_ris_elements"] = self._ris_elements.clone()
         return sd
 
     def load_state_dict(self, sd):
@@ -711,3 +759,12 @@ class BatchedEnviron:
             self.env_params.copy_(t.to(self.device))
         elif self.env_params is not None:  # saved without a table: every env follows the saved params again
             self.attach_env_params(False)
+        if "_ris_elements" in sd:  # copied into the attached one, as the table
+            t = sd["_ris_elements"]
+            if tuple(t.shape) != (self.E,) or t.dtype != torch.int32:
+                raise ValueError(f"_ris_elements must be int32 [{self.E}]")
+            if self._ris_elements is None:
+                self.attach_ris_elements()
+            self._ris_elements.copy_(t.to(self.device))
+        elif self._ris_elements is not None:  # saved without one: every env has M elements again
+            self.attach_ris_elements(False)

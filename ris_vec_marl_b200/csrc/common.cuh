@@ -111,6 +111,15 @@ __device__ __forceinline__ void env_params_sarl(risvec_params_t& p, const double
     p.penalty2 = __ldg(row + RISVEC_ENVP_PENALTY2);
 }
 
+// Per-env RIS size (risvec_attach_ris_elements): env e has the elements 0 .. n - 1 of the handle's M.  The count is
+// clamped to [1, M] before it bounds a loop or an index (0 would leave all-zero gains, which the pairing's dB
+// arithmetic does not take).  A kernel instantiated with NE = false gets n = M, the bound it had without an array.
+template <bool NE>
+__device__ __forceinline__ int ris_count(const int* __restrict__ n_elem, long long e, int M) {
+    if constexpr (NE) return min(max(__ldg(n_elem + e), 1), M);
+    else return M;
+}
+
 __device__ inline uint4 rng_draw(const Dims& d, long long env_local, unsigned long long call, unsigned slot,
                                  unsigned kind) {
     unsigned long long ge = (unsigned long long)(d.env_base + env_local);

@@ -62,8 +62,10 @@ __global__ void k_episode_clock(Dims d, EpisodeArgs a) {
 // shared memory, where lanes (env, vehicle) read it for the channel gains; the pairing reset comes last.  Envs
 // without CHANNEL in a warp that runs the BCD take part in its shuffles and write nothing.  CLOCK: the bits come
 // from the episode clock (advanced here) and the draws are keyed by the episode index (RNG kinds 5-7).
-template <bool CLOCK>
-__global__ void __launch_bounds__(128) k_begin_episode(Dims d, State s, risvec_params_t p, PairArgs pa, EpisodeArgs a) {
+// NE: per-env RIS size `n_elem` (risvec_attach_ris_elements), read by the channel stage; unused without NE
+template <bool CLOCK, bool NE = false>
+__global__ void __launch_bounds__(128) k_begin_episode(Dims d, State s, risvec_params_t p, PairArgs pa, EpisodeArgs a,
+                                                       const int* __restrict__ n_elem) {
     extern __shared__ double2 bcd_smem[];
     const int wpb = blockDim.x >> 5;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, el = lane >> 3, k = lane & 7;
@@ -114,9 +116,11 @@ __global__ void __launch_bounds__(128) k_begin_episode(Dims d, State s, risvec_p
         const bool ch = env_ok && (bits & RISVEC_EP_CHANNEL) != 0;
         double2* c = bcd_smem + (size_t)(warp * 4 + el) * 2 * M;
         double2* th = c + M;
-        bcd_v8_warp(d, s, e, ch, angle, c, th);
+        const int n = ris_count<NE>(n_elem, e, M);
+        if constexpr (NE) bcd_v8_warp_n(d, s, e, ch, angle, c, th, n);
+        else bcd_v8_warp(d, s, e, ch, angle, c, th);
         __syncwarp();
-        if (ch && k < V) s.gains[ev] = gains_free_lane(d, angle, amp, &th[0].x, &th[0].y, 2);
+        if (ch && k < V) s.gains[ev] = gains_free_lane(d, angle, amp, &th[0].x, &th[0].y, 2, n);
     }
     if (env_ok && (bits & RISVEC_EP_PAIRING)) pair_reset_env(pa, V, e, k, 8);
 }

@@ -81,17 +81,19 @@ __device__ inline void geom_phasor(double delta, int m, double* re, double* im) 
 // K > 0 independent of theta.  The coordinate search therefore keeps S incrementally:
 // for each m the candidate maximising |S - theta_m c_m + e_k c_m|^2 wins, first maximum on
 // ties, accepted only if strictly positive (best starts at 0, MARL:210-218).
-__global__ void k_bcd(Dims d, State s, EnvGate g) {
+// NE: per-env RIS size `n_elem` (risvec_attach_ris_elements): the env's elements m < n only; unused without NE
+template <bool NE = false>
+__global__ void k_bcd(Dims d, State s, EnvGate g, const int* __restrict__ n_elem) {
     extern __shared__ double2 bcd_smem[];
     const int wpb = blockDim.x >> 5;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int e = blockIdx.x * wpb + warp;
     if (e >= d.E || !g.on(e)) return;  // whole warp leaves together
-    const int V = d.V, M = d.M;
+    const int V = d.V, M = d.M, n = ris_count<NE>(n_elem, e, M);
     double2* c = bcd_smem + (size_t)warp * 2 * M;
     double2* th = c + M;
     double sr = 0.0, si = 0.0;
-    for (int m = lane; m < M; m += 32) {
+    for (int m = lane; m < n; m += 32) {
         double cr = 0.0, ci = 0.0;
         for (int v = 0; v < V; ++v) {
             double re, im;
@@ -117,7 +119,7 @@ __global__ void k_bcd(Dims d, State s, EnvGate g) {
     if (one && lane < d.ncand) sincospi(2.0 * (double)lane / (double)d.ncand, &ei0, &er0);
     int width = 32;
     if (one) { width = 1; while (width < d.ncand) width <<= 1; }
-    for (int m = 0; m < M; ++m) {
+    for (int m = 0; m < n; ++m) {
         const double2 cm = c[m], tm = th[m];
         const double rr = sr - (tm.x * cm.x - tm.y * cm.y);
         const double ri = si - (tm.x * cm.y + tm.y * cm.x);
@@ -160,7 +162,7 @@ __global__ void k_bcd(Dims d, State s, EnvGate g) {
         }
         __syncwarp();
     }
-    for (int m = lane; m < M; m += 32) {
+    for (int m = lane; m < n; m += 32) {
         s.theta_re[(size_t)e * M + m] = th[m].x;
         s.theta_im[(size_t)e * M + m] = th[m].y;
     }
@@ -245,7 +247,86 @@ __device__ __forceinline__ void bcd_v8_warp(const Dims& d, const State& s, int e
         }
 }
 
-__global__ void k_bcd_v8(Dims d, State s, EnvGate g) {
+// bcd_v8_warp for a per-env RIS size: env e's lanes score and write the elements m < n only (n = its own count).  The
+// element loop runs to the largest count of the warp's four envs, because its shuffles need every lane; an env past
+// its count takes part in them and keeps its state.  For m < n the operations are those of bcd_v8_warp on a handle
+// with M = n.  A separate copy: a count argument in bcd_v8_warp changed the machine code of k_begin_episode.
+__device__ __forceinline__ void bcd_v8_warp_n(const Dims& d, const State& s, int e, bool write, double angle,
+                                              double2* c, double2* th, int n) {
+    const int lane = threadIdx.x & 31, k = lane & 7;
+    const int V = d.V, M = d.M, base = lane & ~7;
+    const int nw = max(max(__shfl_sync(kFull, n, 0), __shfl_sync(kFull, n, 8)),
+                       max(__shfl_sync(kFull, n, 16), __shfl_sync(kFull, n, 24)));
+    const double2 my_z = unit_phasor64(d.angle_BR - angle);
+    for (int m = k; m < n; m += 8) c[m] = make_double2(0.0, 0.0);
+    for (int v = 0; v < V; ++v) {
+        const double2 z = make_double2(__shfl_sync(kFull, my_z.x, base + v), __shfl_sync(kFull, my_z.y, base + v));
+        double2 w = cpow64(z, (unsigned)k);
+        const double2 z2 = cmul64(z, z), z4 = cmul64(z2, z2), z8 = cmul64(z4, z4);
+        for (int m = k; m < n; m += 8) {
+            c[m].x += w.x;
+            c[m].y += w.y;
+            w = cmul64(w, z8);
+        }
+    }
+    double sr = 0.0, si = 0.0;
+    for (int m = k; m < n; m += 8) {
+        const double tr = s.theta_re[(size_t)e * M + m], ti = s.theta_im[(size_t)e * M + m];
+        const double2 cm = c[m];
+        th[m] = make_double2(tr, ti);
+        sr += tr * cm.x - ti * cm.y;
+        si += tr * cm.y + ti * cm.x;
+    }
+    sr = seg_sum<8>(sr);
+    si = seg_sum<8>(si);
+    __syncwarp();
+    double er0 = 0.0, ei0 = 0.0;
+    if (k < d.ncand) sincospi(2.0 * (double)k / (double)d.ncand, &ei0, &er0);
+    for (int m = 0; m < nw; ++m) {
+        const bool own = m < n;  // uniform over the env's 8 lanes
+        const double2 cm = own ? c[m] : make_double2(0.0, 0.0), tm = own ? th[m] : make_double2(0.0, 0.0);
+        const double rr = sr - (tm.x * cm.x - tm.y * cm.y);
+        const double ri = si - (tm.x * cm.y + tm.y * cm.x);
+        double best = -1.0, bsr = rr, bsi = ri;
+        int bk = 0x7fffffff;
+        if (k < d.ncand) {
+            const double cr = rr + (er0 * cm.x - ei0 * cm.y);
+            const double ci = ri + (er0 * cm.y + ei0 * cm.x);
+            const double val = cr * cr + ci * ci;
+            if (val > best) { best = val; bk = k; bsr = cr; bsi = ci; }
+        }
+        double wv = best;
+        int wk = bk;
+#pragma unroll
+        for (int o = 4; o > 0; o >>= 1) {
+            const double ov = __shfl_xor_sync(kFull, wv, o);
+            const int ok = __shfl_xor_sync(kFull, wk, o);
+            if (ov > wv || (ov == wv && ok < wk)) { wv = ov; wk = ok; }
+        }
+        const bool acc = wv > 0.0;
+        const int src = base + (acc ? (wk & 7) : 0);
+        const double nsr = __shfl_sync(kFull, bsr, src), nsi = __shfl_sync(kFull, bsi, src);
+        if (own) {
+            sr = acc ? nsr : rr;
+            si = acc ? nsi : ri;
+            if (acc) {
+                if (lane == src) th[m] = make_double2(er0, ei0);
+            } else if (k == 0) {  // never improved on best = 0: the reference stores the integer 0
+                th[m] = make_double2(0.0, 0.0);
+            }
+        }
+        __syncwarp();
+    }
+    if (write)
+        for (int m = k; m < n; m += 8) {
+            s.theta_re[(size_t)e * M + m] = th[m].x;
+            s.theta_im[(size_t)e * M + m] = th[m].y;
+        }
+}
+
+// NE: as k_bcd; the four envs of a warp may have different counts (the element loop is per env's lane group)
+template <bool NE = false>
+__global__ void k_bcd_v8(Dims d, State s, EnvGate g, const int* __restrict__ n_elem) {
     extern __shared__ double2 bcd_smem[];
     const int wpb = blockDim.x >> 5;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, el = lane >> 3, k = lane & 7;
@@ -253,22 +334,24 @@ __global__ void k_bcd_v8(Dims d, State s, EnvGate g) {
     const int e = min(e_raw, d.E - 1);
     const bool env_ok = e_raw < d.E && g.on(e);
     double2* c = bcd_smem + (size_t)(warp * 4 + el) * 2 * d.M;
-    bcd_v8_warp(d, s, e, env_ok, s.angle[(size_t)e * d.V + min(k, d.V - 1)], c, c + d.M);
+    const double angle = s.angle[(size_t)e * d.V + min(k, d.V - 1)];
+    if constexpr (NE) bcd_v8_warp_n(d, s, e, env_ok, angle, c, c + d.M, ris_count<NE>(n_elem, e, d.M));
+    else bcd_v8_warp(d, s, e, env_ok, angle, c, c + d.M);
 }
 
 // update_channel_gains, "free" model, lane = (env, vehicle): the vehicle's phasor z_v^m is stepped
 // by one float64 complex multiplication per element (re-anchored by an exact sincospi every 32
 // elements), the M products theta_m z_v^m are summed in order -- no shuffles at all.
 // gains_free_lane is the per-vehicle body: theta_m = (tr[m * ts], ti[m * ts]) (ts = 1: the state arrays; ts = 2: an
-// interleaved double2 copy in shared memory).  Shared by k_gains_free_v and the fused episode start.
+// interleaved double2 copy in shared memory), summed over the elements m < n (d.M, or the env's per-env RIS size).
+// Shared by k_gains_free_v and the fused episode start.
 __device__ __forceinline__ double gains_free_lane(const Dims& d, double angle, double amp, const double* tr,
-                                                  const double* ti, int ts) {
-    const int M = d.M;
+                                                  const double* ti, int ts, int n) {
     const double delta = d.angle_BR - angle;
     const double2 z = unit_phasor64(delta);
     double sr = 0.0, si = 0.0;
     double2 w = make_double2(1.0, 0.0);
-    for (int m = 0; m < M; ++m) {
+    for (int m = 0; m < n; ++m) {
         if ((m & 31) == 0 && m) w = unit_phasor64((double)m * delta);
         const double a = tr[(size_t)m * ts], b = ti[(size_t)m * ts];
         sr += a * w.x - b * w.y;
@@ -278,31 +361,33 @@ __device__ __forceinline__ double gains_free_lane(const Dims& d, double angle, d
     return amp * (sr * sr + si * si);
 }
 
-template <int VP>
-__global__ void k_gains_free_v(Dims d, State s, EnvGate g) {
+// NE: as k_bcd
+template <int VP, bool NE = false>
+__global__ void k_gains_free_v(Dims d, State s, EnvGate g, const int* __restrict__ n_elem) {
     const long long gtid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     const int e_raw = (int)(gtid / VP), v = (int)(gtid % VP);
     const int e = min(e_raw, d.E - 1), M = d.M;
     const bool act = e_raw < d.E && v < d.V && g.on(e);
     const size_t ev = (size_t)e * d.V + min(v, d.V - 1);
     const double gain = gains_free_lane(d, s.angle[ev], s.amp[ev], s.theta_re + (size_t)e * M,
-                                        s.theta_im + (size_t)e * M, 1);
+                                        s.theta_im + (size_t)e * M, 1, ris_count<NE>(n_elem, e, M));
     if (act) s.gains[ev] = gain;
 }
 
 // update_channel_gains, "free" model (MARL:263-273): the cascaded RIS reduction
 //   gain_v = amp_v * | sum_m theta_m * phasor(v, m) |^2
-// one warp per env, lanes stride over the M elements, complex warp-shuffle reduction.
-__global__ void k_gains_free(Dims d, State s, EnvGate g) {
+// one warp per env, lanes stride over the M elements, complex warp-shuffle reduction.  NE: as k_bcd
+template <bool NE = false>
+__global__ void k_gains_free(Dims d, State s, EnvGate g, const int* __restrict__ n_elem) {
     const int wpb = blockDim.x >> 5;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int e = blockIdx.x * wpb + warp;
     if (e >= d.E || !g.on(e)) return;
-    const int V = d.V, M = d.M;
+    const int V = d.V, M = d.M, n = ris_count<NE>(n_elem, e, M);
     for (int v = 0; v < V; ++v) {
         const double delta = d.angle_BR - s.angle[(size_t)e * V + v];
         double sr = 0.0, si = 0.0;
-        for (int m = lane; m < M; m += 32) {
+        for (int m = lane; m < n; m += 32) {
             double re, im;
             geom_phasor(delta, m, &re, &im);
             const double tr = s.theta_re[(size_t)e * M + m], ti = s.theta_im[(size_t)e * M + m];
@@ -316,7 +401,8 @@ __global__ void k_gains_free(Dims d, State s, EnvGate g) {
 }
 
 // update_channel_gains, simplified 3GPP TR 38.901 UMi / UMa branch (MARL:275-327): direct
-// vehicle<->BS link with LOS draw, log-normal shadowing and Rayleigh / Rice small-scale power.
+// vehicle<->BS link with LOS draw, log-normal shadowing and Rayleigh / Rice small-scale power.  No RIS term, so it
+// takes no per-env RIS size.
 // One thread per (env, vehicle).  Draw order per vehicle in the reference: rand, normal,
 // then exponential (K = 0) or two normals.
 __global__ void k_gains_3gpp(Dims d, State s, risvec_params_t p, const double* __restrict__ c_rand,

@@ -1,5 +1,6 @@
 // C ABI of the risvec library (include/risvec.h): handle, state arena, launches.
 #include <algorithm>
+#include <array>
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
@@ -114,6 +115,7 @@ struct risvec_env {
     unsigned char* ep_bits;   // [E] in the arena: stage bits of the current tick (episode clock, unfused shapes)
     int* ep_keys;             // [E] in the arena: episode index that keys the tick's draws (same)
     const double* env_params; // attached per-env parameter table [E, RISVEC_ENVP_COLS] (risvec_attach_env_params) or null
+    const int32_t* ris_elem;  // attached per-env RIS size [E] (risvec_attach_ris_elements) or null
 };
 
 struct risvec_replay {
@@ -192,6 +194,11 @@ int ensure_scratch(risvec_env* env, size_t bytes) {
 template <typename F>
 int dispatch_pe(const risvec_env* env, F&& f) {
     return env->env_params ? f(std::true_type{}) : f(std::false_type{});
+}
+// the same for an attached per-env RIS size (the NE instantiations)
+template <typename F>
+int dispatch_re(const risvec_env* env, F&& f) {
+    return env->ris_elem ? f(std::true_type{}) : f(std::false_type{});
 }
 
 // f(std::integral_constant<int, VP>{}) for the least power of two VP >= V (V <= 32); dispatch_vp<8> starts at 8
@@ -272,8 +279,9 @@ SarlKernel choose_sarl(const risvec_env* env, const SarlArgs& a, int from = kSar
     const Dims& d = env->dims;
     const SarlPath p = env->ovr.sarl;
     if (a.in_rec) return kSarlV8;  // the caller checked the packed shape
-    // an attached per-env parameter table: only k_sarl_mma and the generic kernels have PE instantiations
-    const bool pe = env->env_params != nullptr;
+    // an attached per-env parameter table or RIS size: only k_sarl_mma and the generic kernels have PE / NE
+    // instantiations
+    const bool pe = env->env_params != nullptr || env->ris_elem != nullptr;
     const bool mma = p == kPathAuto || p == kPathMmaLdg || p == kPathMmaSync;
     // tensor cores, one warp per env: V <= 8, M even, M <= 64
     const bool mma_fits = mma && d.V <= 8 && d.M % 2 == 0 && d.M <= 64 && (!a.raw || aligned8(a.raw));
@@ -312,19 +320,22 @@ int launch_sarl_mma_tma(risvec_env* env, const SarlArgs& a, cudaStream_t st, boo
 }
 
 // tensor cores, LDG (sarl_mma.cuh): one warp per env, 4 envs per block; KT k-tiles of 8 elements, M <= 8 KT
-// [per-env table][fused][KT]
+// [per-env RIS size][per-env table][fused][KT]
+using SarlMmaRow = std::array<decltype(&k_sarl_mma<1>), 5>;  // over KT
+template <bool FUSED, bool PE, bool NE>
+SarlMmaRow sarl_mma_row() {
+    return {k_sarl_mma<1, FUSED, PE, NE>, k_sarl_mma<2, FUSED, PE, NE>, k_sarl_mma<3, FUSED, PE, NE>,
+            k_sarl_mma<5, FUSED, PE, NE>, k_sarl_mma<8, FUSED, PE, NE>};
+}
 int launch_sarl_mma(risvec_env* env, const SarlArgs& a, cudaStream_t st) {
-    using Kern = decltype(&k_sarl_mma<1>);
-    static const Kern kerns[2][2][5] = {
-        {{k_sarl_mma<1>, k_sarl_mma<2>, k_sarl_mma<3>, k_sarl_mma<5>, k_sarl_mma<8>},
-         {k_sarl_mma<1, true>, k_sarl_mma<2, true>, k_sarl_mma<3, true>, k_sarl_mma<5, true>, k_sarl_mma<8, true>}},
-        {{k_sarl_mma<1, false, true>, k_sarl_mma<2, false, true>, k_sarl_mma<3, false, true>,
-          k_sarl_mma<5, false, true>, k_sarl_mma<8, false, true>},
-         {k_sarl_mma<1, true, true>, k_sarl_mma<2, true, true>, k_sarl_mma<3, true, true>, k_sarl_mma<5, true, true>,
-          k_sarl_mma<8, true, true>}}};
+    static const SarlMmaRow kerns[2][2][2] = {
+        {{sarl_mma_row<false, false, false>(), sarl_mma_row<true, false, false>()},
+         {sarl_mma_row<false, true, false>(), sarl_mma_row<true, true, false>()}},
+        {{sarl_mma_row<false, false, true>(), sarl_mma_row<true, false, true>()},
+         {sarl_mma_row<false, true, true>(), sarl_mma_row<true, true, true>()}}};
     const int M = env->dims.M, kt = M <= 8 ? 0 : M <= 16 ? 1 : M <= 24 ? 2 : M <= 40 ? 3 : 4;
-    kerns[env->env_params != nullptr][a.raw != nullptr][kt]<<<(env->dims.E + 3) / 4, 128, 0, st>>>(
-        env->dims, env->st, env->params, a, env->env_params);
+    const auto kern = kerns[env->ris_elem != nullptr][env->env_params != nullptr][a.raw != nullptr][kt];
+    kern<<<(env->dims.E + 3) / 4, 128, 0, st>>>(env->dims, env->st, env->params, a, env->env_params, env->ris_elem);
     return check_step_launch(env, "k_sarl_mma");
 }
 
@@ -392,11 +403,14 @@ int launch_sarl_cfg(risvec_env* env, const SarlArgs& a_in, cudaStream_t st) {
     if constexpr (WPE == 1) {  // one warp per env group: fused step kernel
         const size_t smem = 6 * EPW * MS * sizeof(float);
         return dispatch_pe(env, [&](auto pe) {
-            auto kern = k_sarl_rollout<VP, MPL, WPE, decltype(pe)::value>;
-            if (smem > 48 * 1024)
-                CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            kern<<<blocks, 32 * WPE, smem, st>>>(env->dims, env->st, env->params, a, env->env_params);
-            return check_step_launch(env, "k_sarl_rollout");
+            return dispatch_re(env, [&](auto re) {
+                auto kern = k_sarl_rollout<VP, MPL, WPE, decltype(pe)::value, decltype(re)::value>;
+                if (smem > 48 * 1024)
+                    CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+                kern<<<blocks, 32 * WPE, smem, st>>>(env->dims, env->st, env->params, a, env->env_params,
+                                                     env->ris_elem);
+                return check_step_launch(env, "k_sarl_rollout");
+            });
         });
     } else {
         // several warps per env (large M): cascade kernel over (env group, time chunk) -> |S|^2 scratch,
@@ -407,11 +421,15 @@ int launch_sarl_cfg(risvec_env* env, const SarlArgs& a_in, cudaStream_t st) {
         while (chunk > 2 && (long long)blocks * ((a.T + chunk - 1) / chunk) < 4 * 148) chunk >>= 1;  // fill the SMs
         a.t_chunk = chunk;
         const size_t smem2 = 8 * EPW * MS * sizeof(float) + 4 * WPE * 32 * sizeof(float2);
-        auto kern = k_sarl_cascade2<VP, MPL, WPE>;
-        if (smem2 > 48 * 1024)
-            CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2));
-        kern<<<dim3(blocks, (a.T + chunk - 1) / chunk), 32 * WPE, smem2, st>>>(env->dims, env->st, a);
-        if (int rc = check_launch(env, "k_sarl_cascade2")) return rc;
+        if (int rc = dispatch_re(env, [&](auto re) {
+                auto kern = k_sarl_cascade2<VP, MPL, WPE, decltype(re)::value>;
+                if (smem2 > 48 * 1024)
+                    CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2));
+                kern<<<dim3(blocks, (a.T + chunk - 1) / chunk), 32 * WPE, smem2, st>>>(env->dims, env->st, a,
+                                                                                         env->ris_elem);
+                return check_launch(env, "k_sarl_cascade2");
+            }))
+            return rc;
         const long long total = (long long)E * VP;
         // the scan reads the step parameters: the cascade only forms |S|^2
         if (int rc = dispatch_pe(env, [&](auto pe) {
@@ -841,38 +859,45 @@ int launch_compute_parms(risvec_env* env, EnvGate g, void* stream) {
     return check_launch(env, "k_compute_parms");
 }
 int launch_bcd(risvec_env* env, EnvGate g, void* stream) {
-    if (env->dims.ncand <= 8 && env->dims.V <= 8 && env->dims.M <= 256 && !env->ovr.force_generic) {
-        // 4 envs per warp, lane = (env, candidate)
-        const int wpb = env->dims.M <= 64 ? 4 : 1;
-        const int blocks = (env->dims.E + 4 * wpb - 1) / (4 * wpb);
-        const size_t smem = (size_t)wpb * 4 * 2 * env->dims.M * sizeof(double2);
+    return dispatch_re(env, [&](auto re) {
+        constexpr bool NE = decltype(re)::value;
+        if (env->dims.ncand <= 8 && env->dims.V <= 8 && env->dims.M <= 256 && !env->ovr.force_generic) {
+            // 4 envs per warp, lane = (env, candidate)
+            const int wpb = env->dims.M <= 64 ? 4 : 1;
+            const int blocks = (env->dims.E + 4 * wpb - 1) / (4 * wpb);
+            const size_t smem = (size_t)wpb * 4 * 2 * env->dims.M * sizeof(double2);
+            if (smem > 48 * 1024)
+                CUDA_TRY(cudaFuncSetAttribute(k_bcd_v8<NE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            k_bcd_v8<NE><<<blocks, 32 * wpb, smem, (cudaStream_t)stream>>>(env->dims, env->st, g, env->ris_elem);
+            return check_launch(env, "k_bcd_v8");
+        }
+        const int wpb = 4, threads = 32 * wpb, blocks = (env->dims.E + wpb - 1) / wpb;
+        const size_t smem = (size_t)wpb * 2 * env->dims.M * sizeof(double2);
         if (smem > 48 * 1024)
-            CUDA_TRY(cudaFuncSetAttribute(k_bcd_v8, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        k_bcd_v8<<<blocks, 32 * wpb, smem, (cudaStream_t)stream>>>(env->dims, env->st, g);
-        return check_launch(env, "k_bcd_v8");
-    }
-    const int wpb = 4, threads = 32 * wpb, blocks = (env->dims.E + wpb - 1) / wpb;
-    const size_t smem = (size_t)wpb * 2 * env->dims.M * sizeof(double2);
-    if (smem > 48 * 1024)
-        CUDA_TRY(cudaFuncSetAttribute(k_bcd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    k_bcd<<<blocks, threads, smem, (cudaStream_t)stream>>>(env->dims, env->st, g);
-    return check_launch(env, "k_bcd");
+            CUDA_TRY(cudaFuncSetAttribute(k_bcd<NE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        k_bcd<NE><<<blocks, threads, smem, (cudaStream_t)stream>>>(env->dims, env->st, g, env->ris_elem);
+        return check_launch(env, "k_bcd");
+    });
 }
 int launch_gains(risvec_env* env, const double* chan_rand, const double* chan_normal, const double* chan_exp, EnvGate g,
                  void* stream) {
-    if (env->params.channel_model == RISVEC_CHANNEL_FREE) {
-        if (!env->ovr.force_generic)  // lane = (env, vehicle), sequential over the elements
-            return dispatch_vp(env->dims.V, [&](auto vp) {
-                constexpr int VP = decltype(vp)::value;
-                const long long n = (long long)env->dims.E * VP;
-                const int threads = 128, blocks = (int)((n + threads - 1) / threads);
-                k_gains_free_v<VP><<<blocks, threads, 0, (cudaStream_t)stream>>>(env->dims, env->st, g);
-                return check_launch(env, "k_gains_free_v");
-            });
-        const int wpb = 4, threads = 32 * wpb, blocks = (env->dims.E + wpb - 1) / wpb;
-        k_gains_free<<<blocks, threads, 0, (cudaStream_t)stream>>>(env->dims, env->st, g);
-        return check_launch(env, "k_gains_free");
-    }
+    if (env->params.channel_model == RISVEC_CHANNEL_FREE)
+        return dispatch_re(env, [&](auto re) {
+            constexpr bool NE = decltype(re)::value;
+            if (!env->ovr.force_generic)  // lane = (env, vehicle), sequential over the elements
+                return dispatch_vp(env->dims.V, [&](auto vp) {
+                    constexpr int VP = decltype(vp)::value;
+                    const long long n = (long long)env->dims.E * VP;
+                    const int threads = 128, blocks = (int)((n + threads - 1) / threads);
+                    k_gains_free_v<VP, NE><<<blocks, threads, 0, (cudaStream_t)stream>>>(env->dims, env->st, g,
+                                                                                          env->ris_elem);
+                    return check_launch(env, "k_gains_free_v");
+                });
+            const int wpb = 4, threads = 32 * wpb, blocks = (env->dims.E + wpb - 1) / wpb;
+            k_gains_free<NE><<<blocks, threads, 0, (cudaStream_t)stream>>>(env->dims, env->st, g, env->ris_elem);
+            return check_launch(env, "k_gains_free");
+        });
+    // the 3GPP branch has no RIS term: it takes no per-env RIS size
     const long long n = (long long)env->dims.E * env->dims.V;
     const int threads = 128, blocks = (int)((n + threads - 1) / threads);
     const unsigned long long call = g.call ? 0 : env->chan_calls++;
@@ -909,6 +934,9 @@ int check_sarl_packed_args(const risvec_env* env, int T, const void* in_rec, con
         return fail(RISVEC_ERR_UNSUPPORTED, "packed SARL records need V == 8, E %% 4 == 0 and M in {16, 40} "
                     "(got V = %d, E = %d, M = %d)", env->dims.V, env->dims.E, env->dims.M);
     if (env->env_params) return fail(RISVEC_ERR_UNSUPPORTED, "%s", kPackedEnvParamsMsg);
+    if (env->ris_elem)
+        return fail(RISVEC_ERR_UNSUPPORTED, "packed SARL records take no per-env RIS size: one is attached "
+                    "(risvec_attach_ris_elements); detach it or use the per-array entry points");
     return RISVEC_OK;
 }
 int check_marl_packed_args(const risvec_env* env, int T, const void* in_rec, const void* partner, const void* ngroups,
@@ -1419,11 +1447,14 @@ int launch_begin_episode(risvec_env* env, const EpisodeArgs& a, void* stream) {
     const int wpb = env->dims.M <= 64 ? 4 : 1;  // as k_bcd_v8: 4 envs per warp, 2 M double2 of shared memory per env
     const int blocks = (env->dims.E + 4 * wpb - 1) / (4 * wpb);
     const size_t smem = (size_t)wpb * 4 * 2 * env->dims.M * sizeof(double2);
-    if (smem > 48 * 1024)
-        CUDA_TRY(cudaFuncSetAttribute(k_begin_episode<CLOCK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    k_begin_episode<CLOCK><<<blocks, 32 * wpb, smem, (cudaStream_t)stream>>>(env->dims, env->st, env->params,
-                                                                              pair_state_args(env), a);
-    return check_launch(env, "k_begin_episode");
+    return dispatch_re(env, [&](auto re) {
+        auto kern = k_begin_episode<CLOCK, decltype(re)::value>;
+        if (smem > 48 * 1024)
+            CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        kern<<<blocks, 32 * wpb, smem, (cudaStream_t)stream>>>(env->dims, env->st, env->params, pair_state_args(env), a,
+                                                               env->ris_elem);
+        return check_launch(env, "k_begin_episode");
+    });
 }
 
 // the stages `stages` as separate kernels restricted by `g` (g.bits null = every env), in the fixed order
@@ -1793,6 +1824,25 @@ int risvec_attach_env_params(risvec_env_t* env, const double* table) {
                         at.device, env->device);
     }
     env->env_params = table;
+    return RISVEC_OK;
+}
+
+int risvec_attach_ris_elements(risvec_env_t* env, const int32_t* n_elem) {
+    if (!env) return fail(RISVEC_ERR_INVALID, "NULL handle");
+    if (n_elem != nullptr) {
+        if (((uintptr_t)n_elem) & 3u) return fail(RISVEC_ERR_INVALID, "the per-env RIS size must be 4-byte aligned");
+        cudaPointerAttributes at;
+        if (cudaPointerGetAttributes(&at, n_elem) != cudaSuccess) {
+            cudaGetLastError();
+            return fail(RISVEC_ERR_INVALID, "the per-env RIS size is not a CUDA pointer");
+        }
+        if (at.type != cudaMemoryTypeDevice && at.type != cudaMemoryTypeManaged)
+            return fail(RISVEC_ERR_INVALID, "the per-env RIS size must be device memory");
+        if (at.device != env->device)
+            return fail(RISVEC_ERR_INVALID, "the per-env RIS size is on device %d, the handle on device %d", at.device,
+                        env->device);
+    }
+    env->ris_elem = n_elem;
     return RISVEC_OK;
 }
 

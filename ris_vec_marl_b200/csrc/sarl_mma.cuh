@@ -64,9 +64,11 @@ struct SarlMmaIn {     // inputs of one 8-step tile, as one lane needs them
 // KT = k-tiles of 8 RIS elements (M <= 8 KT, M even).  Block = 4 warps = 4 adjacent envs.
 // FUSED = the one-launch driver step (risvec_step_sarl_fused): inputs from the actor's raw row, observation out
 // PE: per-env step parameters from the attached table `envp` (risvec_attach_env_params); unused without PE
-template <int KT, bool FUSED = false, bool PE = false>
+// NE: per-env RIS size `n_elem` (risvec_attach_ris_elements): the A operand is zero at the elements m >= n; unused
+// without NE
+template <int KT, bool FUSED = false, bool PE = false, bool NE = false>
 __global__ void __launch_bounds__(128, 4) k_sarl_mma(Dims d, State s, risvec_params_t p, SarlArgs a,
-                                                     const double* __restrict__ envp) {
+                                                     const double* __restrict__ envp, const int* __restrict__ n_elem) {
     const int lane = threadIdx.x & 31, g = lane >> 2, tig = lane & 3;
     const int E = d.E, V = d.V, M = d.M, T = a.T;
     const int e = blockIdx.x * 4 + (threadIdx.x >> 5);
@@ -81,6 +83,7 @@ __global__ void __launch_bounds__(128, 4) k_sarl_mma(Dims d, State s, risvec_par
     //  8 j + 2 tig + 1: the same element order the B fragments below use)
     uint32_t Ah[KT][4], Al[KT][4];
     {
+        const int n = ris_count<NE>(n_elem, e, M);
         const double2 z = unit_phasor64(d.angle_BR - s.angle[ev]);  // w(v, m) = z^m, float64 (SARL:134-145)
         const double2 z2 = cmul64(z, z), z4 = cmul64(z2, z2), z8 = cmul64(z4, z4);
         double2 w = cpow64(z, 2u * (unsigned)tig);
@@ -88,8 +91,8 @@ __global__ void __launch_bounds__(128, 4) k_sarl_mma(Dims d, State s, risvec_par
         for (int j = 0; j < KT; ++j) {
             const int ma = 8 * j + 2 * tig;
             double2 wa = w, wb = cmul64(w, z);
-            if (!(vact && ma < M)) wa = make_double2(0.0, 0.0);
-            if (!(vact && ma + 1 < M)) wb = make_double2(0.0, 0.0);
+            if (!(vact && ma < n)) wa = make_double2(0.0, 0.0);
+            if (!(vact && ma + 1 < n)) wb = make_double2(0.0, 0.0);
             split_h2(wa.x, -wa.y, Ah[j][0], Al[j][0]);  // row g     (Re S_g): ( Re w, -Im w)
             split_h2(wa.y, wa.x, Ah[j][1], Al[j][1]);   // row g + 8 (Im S_g): ( Im w,  Re w)
             split_h2(wb.x, -wb.y, Ah[j][2], Al[j][2]);

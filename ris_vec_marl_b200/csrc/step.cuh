@@ -322,9 +322,12 @@ __device__ __noinline__ void phasor_f32(double x, float* re, float* im) {
 // one warp per block and step).
 
 // PE: per-env step parameters from the attached table `envp` (risvec_attach_env_params); unused without PE
-template <int VP, int MPL, int WPE, bool PE = false>
+// NE: per-env RIS size `n_elem` (risvec_attach_ris_elements): the phasor pairs of the elements m >= n are zero, so the
+// step loop is unchanged; unused without NE
+template <int VP, int MPL, int WPE, bool PE = false, bool NE = false>
 __global__ void __launch_bounds__(32 * WPE) k_sarl_rollout(Dims d, State s, risvec_params_t p, SarlArgs a,
-                                                           const double* __restrict__ envp) {
+                                                           const double* __restrict__ envp,
+                                                           const int* __restrict__ n_elem) {
     static_assert(MPL % 4 == 0, "elements are processed four at a time (LDS.128 + FFMA2 pairs)");
     constexpr int EPW = 32 / VP;  // envs per warp (= per block)
     constexpr int NT = 32 * WPE;
@@ -351,7 +354,7 @@ __global__ void __launch_bounds__(32 * WPE) k_sarl_rollout(Dims d, State s, risv
 
     // ---- geometry phasor table -> registers (float64 argument reduction), as element pairs
     float2 WX[MPL / 2], WY[MPL / 2];
-    phasor_pairs<MPL>(d, s, ev, act, m0, m1, WX, WY);
+    phasor_pairs<MPL>(d, s, ev, act, m0, NE ? min(m1, ris_count<NE>(n_elem, min(e, E - 1), M)) : m1, WX, WY);
     for (int i = threadIdx.x; i < 6 * plane; i += NT) th[i] = 0.f;  // pad elements must stay finite
     const bool cphase = (w == 0);
     const int t_begin = 0, t_end = T;
@@ -528,10 +531,10 @@ __global__ void __launch_bounds__(32 * WPE) k_sarl_rollout(Dims d, State s, risv
 // every warp runs its element slice against both steps' theta planes (the phasor table in
 // registers is read once per pair), and one __syncthreads per pair publishes the partial sums
 // that the first warp folds over the WPE warps.  theta planes and partial sums are
-// double-buffered over pairs.
-template <int VP, int MPL, int WPE>
+// double-buffered over pairs.  NE: as k_sarl_rollout
+template <int VP, int MPL, int WPE, bool NE = false>
 __global__ void __launch_bounds__(32 * WPE, (WPE <= 8 && MPL <= 32) ? 16 / WPE : 1)
-    k_sarl_cascade2(Dims d, State s, SarlArgs a) {
+    k_sarl_cascade2(Dims d, State s, SarlArgs a, const int* __restrict__ n_elem) {
     static_assert(MPL % 4 == 0 && WPE > 1, "");
     constexpr int EPW = 32 / VP;
     constexpr int NT = 32 * WPE;
@@ -550,7 +553,7 @@ __global__ void __launch_bounds__(32 * WPE, (WPE <= 8 && MPL <= 32) ? 16 / WPE :
     const int m0 = w * slice, m1 = min(M, m0 + slice);
 
     float2 WX[MPL / 2], WY[MPL / 2];
-    phasor_pairs<MPL>(d, s, ev, act, m0, m1, WX, WY);
+    phasor_pairs<MPL>(d, s, ev, act, m0, NE ? min(m1, ris_count<NE>(n_elem, min(e, E - 1), M)) : m1, WX, WY);
     for (int i = threadIdx.x; i < 8 * plane; i += NT) th[i] = 0.f;  // pad elements must stay finite
     const int t_begin = (int)blockIdx.y * a.t_chunk, t_end = min(T, t_begin + a.t_chunk);
     const int n_ph = min(EPW, E - e0) * M;
