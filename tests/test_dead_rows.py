@@ -82,6 +82,47 @@ def test_gpu_dead_rows_vs_oracle():
 
 
 @pytest.mark.gpu
+@pytest.mark.parametrize("control_bit", [0, 1, 4, 10])
+def test_gpu_random_phase_every_resolution(control_bit):
+    """`Random_phase` at the other phase resolutions (1 ... 1024 candidates; control_bit 3 is the test above):
+    injected choices give the oracle's theta, and the gains on it; on-device draws land on the grid of 2 pi / ncand
+    and, with ncand <= 8, take every value."""
+    from ris_vec_marl_b200 import BatchedEnviron
+
+    E, V, M = 64, 8, 40
+    ncand = 2 ** control_bit
+    rng = np.random.default_rng(2)
+    env = BatchedEnviron("marl", n_envs=E, n_veh=V, M=M, control_bit=control_bit, device=0, seed=3)
+    env.make_new_game(); env.renew_positions(); env.compute_parms()
+    o = EnvOracle("marl", V, M, control_bit, E=E)
+    pos = np.stack([env.pos_x.cpu().numpy(), env.pos_y.cpu().numpy()], axis=-1)
+    o.set_vehicles(pos, env.state("dir").cpu().numpy(), env.vel.cpu().numpy())
+    o.compute_parms()
+    idx = rng.integers(0, ncand, (E, M)).astype(np.int32)
+    idx[0, :min(M, ncand)] = np.arange(min(M, ncand))  # the first candidates, 0 included, at least once
+    idx[1, :] = ncand - 1                              # and the last one
+    env.Random_phase(idx)
+    o.random_phase(idx)
+    th = env.theta_re.cpu().numpy() + 1j * env.theta_im.cpu().numpy()
+    # the same angle k * (2 pi / ncand) on both sides; CUDA sincos and numpy exp are each within an ulp of its phasor
+    np.testing.assert_allclose(th, o.elements_phase_shift_complex, rtol=0, atol=2.5e-16)
+    np.testing.assert_allclose(env.phase_real.cpu().numpy(), o.elements_phase_shift_real, rtol=1e-7)
+    env.update_channel_gains(); o.update_channel_gains()
+    np.testing.assert_allclose(env.gains.cpu().numpy(), o.channel_gains, rtol=1e-9)
+    env.Random_phase()                               # on-device draws: every angle a multiple of 2 pi / ncand
+    th = env.theta_re.cpu().numpy() + 1j * env.theta_im.cpu().numpy()
+    k = np.mod(np.angle(th), 2 * np.pi) / (2 * np.pi / ncand)
+    k = np.where(np.abs(k - ncand) < 1e-9, 0.0, k)   # angle 0 may read as 2 pi - ulp
+    kr = np.round(k).astype(int)
+    assert np.allclose(k, kr, rtol=0, atol=1e-9) and kr.min() >= 0 and kr.max() <= ncand - 1
+    np.testing.assert_allclose(th, np.exp(1j * o.possible_angles[kr]), rtol=0, atol=2.5e-16)
+    np.testing.assert_allclose(env.phase_real.cpu().numpy(), o.possible_angles[kr], rtol=1e-7)
+    if ncand <= 8:
+        assert len(np.unique(kr)) == ncand
+    env.close()
+
+
+@pytest.mark.gpu
 def test_gpu_compat_random_phase_follows_python_random():
     import random
 
